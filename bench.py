@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py -- sites/sec of the fused window scan on 1..8 B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload C4|C5] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload C4|C5] [--impl reference] [--dump-outputs DIR]
     torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
 
 A step is one pass of the hot path (level-1 unit reduction + level-2 window combine) over the whole synthetic
@@ -25,6 +25,9 @@ core and all cores -- SURVEY 8d's second CPU figure: the reference itself cannot
 
 --impl reference runs only that CPU arm (the reference's own implementation of the path); it never imports the
 product package or loads libpgtscan.so.
+
+--dump-outputs DIR writes the window table of the last timed step as .npy files (dump_outputs): the inputs come from
+the seeded generator, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -61,7 +64,14 @@ def parse_args():
     ap.add_argument("--configs", default="", help="comma-separated subset of the per-config legs")
     ap.add_argument("--config-steps", type=int, default=5)
     ap.add_argument("--cpu-sample-sites", type=float, default=4.8e7)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the window table of the last one to DIR/<field>.npy (float64)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the tables of the B200 scan (--impl b200)")
+    return args
 
 
 # ------------------------------------------------------------------------------ reference arm
@@ -515,6 +525,47 @@ def run_config(cfg, R, pgt, steps, peak):
         torch.cuda.empty_cache()
 
 
+DUMP_BYTES = 64_000_000  # --dump-outputs writes at most this many bytes
+
+
+def dump_outputs(out_dir, tab, R, glob=None, budget=DUMP_BYTES):
+    """--dump-outputs: the window table the last timed step left, i.e. the arrays scan() hands its caller, one
+    DIR/<field>.npy per field in float64 (exact for the uint32 fields too), DIR/window_index.npy with the global
+    window index of each row and, for the fused scan, DIR/dxy_global.npy.  A table above `budget` bytes is written at
+    a sample of rows drawn with a fixed seed: the same rows for the same arguments, so that two builds of the project
+    can be compared output for output.  Collective when the table is sharded over the ranks."""
+    import numpy as np
+    torch = R.torch
+    nwin = tab.nwin
+    nrows = min(nwin, (budget - 4096) // (8 * (len(tab.fields) + 1)))  # 4 KB: .npy headers and dxy_global
+    rows = np.arange(nwin) if nrows == nwin else np.sort(np.random.default_rng(0).choice(nwin, nrows, replace=False))
+    lo, hi = (0, nwin) if tab.placement == "rank0" else (tab.w_lo, tab.w_hi)
+    part = None
+    if R.rank == 0 or tab.placement != "rank0":
+        mine = rows[(rows >= lo) & (rows < hi)]
+        idx = torch.as_tensor(mine - lo, device=R.dev)
+        part = {"window_index": mine.astype(np.float64)}
+        for k, a in tab.rows(lo, hi).items():
+            if k == "dxy_global":
+                continue
+            t = torch.as_tensor(a, device=R.dev)
+            if t.dtype == torch.float64:
+                part[k] = t[idx].cpu().numpy()
+            else:  # uint32: gathered through an int32 view of the same bits
+                part[k] = t.view(torch.int32)[idx].cpu().numpy().view(np.uint32).astype(np.float64)
+    if tab.placement != "rank0":
+        parts = [None] * R.world if R.rank == 0 else None
+        R.dist.gather_object(part, parts, dst=0)
+        if R.rank == 0:
+            part = {k: np.concatenate([p[k] for p in parts]) for k in part}
+    if R.rank == 0:
+        os.makedirs(out_dir, exist_ok=True)
+        for k, v in part.items():
+            np.save(os.path.join(out_dir, k + ".npy"), v)
+        if glob is not None:
+            np.save(os.path.join(out_dir, "dxy_global.npy"), np.asarray(glob, np.float64))
+
+
 class PinnedColumns:
     """Host columns of the WHOLE genome in page-locked memory of exactly their size (pgt_host_alloc; torch's pinned
     allocator rounds every tensor up to a power of two, 64 GB for the 48 GB of C4)."""
@@ -633,6 +684,8 @@ def run_b200(args):
     value = n_total / (ms_step * 1e-3)
     result_checksum = tab.checksum()
     glob = tab.global_line() if fused else None
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, tab, R, glob)
 
     # ---- roofline of the dominant kernel (level 1) on this rank
     peak, peak_src = hbm_peak()

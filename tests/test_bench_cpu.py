@@ -39,3 +39,49 @@ def test_reference_arm_line_on_a_tiny_sample():
     assert d["impl"] == "reference" and d["unit"] == "sites/s" and d["value"] > 0 and d["gpu_launches"] == 0
     assert d["cpu_baseline"]["kind"] in ("reference", "port") and d["cpu_baseline"]["cores"] >= 1
     assert d["e2e"] == {"value": d["value"], "unit": "sites/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
+
+
+def test_steps_and_dump_arguments_are_checked():
+    for argv in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", "out"]):
+        r = subprocess.run([sys.executable, "bench.py", *argv], cwd=ROOT, capture_output=True, text=True, timeout=120)
+        assert r.returncode == 2 and "error:" in r.stderr, (argv, r.stderr[-500:])
+
+
+def test_dump_outputs_writes_the_whole_table_or_a_fixed_sample(tmp_path):
+    """--dump-outputs on a window table (the /dev/shm layout of SharedTable, the same code path as in HBM): every field
+    as float64, bit-exact; above the byte budget the same seeded rows on every call, and never more than the budget."""
+    import types
+    import numpy as np
+    import torch
+    import bench
+    from popgenomicstools_b200.sharding import SharedTable
+    nwin = 1000
+    R = types.SimpleNamespace(rank=0, world=1, dev=torch.device("cpu"), torch=torch, dist=None)
+    tab = SharedTable(("label", "start_pos", "nsites", "sum_a", "fst", "dxy_global"), nwin, 0, 1, None, torch=torch,
+                      backend="shm", tag=f"pgt_dump_test_{os.getpid()}")
+    try:
+        rng = np.random.default_rng(1)
+        want = {k: rng.random(nwin) if k in ("sum_a", "fst") else rng.integers(0, 1 << 32, nwin, dtype=np.uint32)
+                for k in tab.fields}
+        rows = tab.rows()
+        for k, v in want.items():
+            rows[k][:] = v
+        full = tmp_path / "full"
+        bench.dump_outputs(str(full), tab, R, glob=np.array([1.5, 7.0, 2.0]))
+        assert sorted(os.listdir(full)) == sorted([k + ".npy" for k in want] + ["window_index.npy", "dxy_global.npy"])
+        assert np.array_equal(np.load(full / "window_index.npy"), np.arange(nwin))
+        assert np.array_equal(np.load(full / "dxy_global.npy"), [1.5, 7.0, 2.0])
+        for k, v in want.items():
+            got = np.load(full / f"{k}.npy")
+            assert got.dtype == np.float64 and np.array_equal(got, v.astype(np.float64)), k
+        budget = 4096 + 8 * (len(want) + 1) * 100  # 100 rows
+        dirs = [tmp_path / "s1", tmp_path / "s2"]
+        for d in dirs:
+            bench.dump_outputs(str(d), tab, R, budget=budget)
+            assert sum(os.path.getsize(d / f) for f in os.listdir(d)) <= budget
+        idx = np.load(dirs[0] / "window_index.npy")
+        assert len(idx) == 100 and np.all(np.diff(idx) > 0) and np.array_equal(idx, np.load(dirs[1] / "window_index.npy"))
+        for k, v in want.items():
+            assert np.array_equal(np.load(dirs[0] / f"{k}.npy"), v[idx.astype(np.int64)].astype(np.float64)), k
+    finally:
+        tab.close()

@@ -17,9 +17,10 @@ ROOT = U.ROOT
 
 def binding(tool):
     p = os.path.join(ROOT, "oracle", "_ref", tool + "_pgt")
-    if os.path.isdir("/root/reference"):
+    reference = os.environ.get("PGT_REFERENCE")  # directory of the original PopGenomicsTools sources
+    if reference and os.path.isdir(reference):
         U.ours(tool)  # libpgtscan.so must exist to link against
-        subprocess.run(["make", "-s", "-C", os.path.join(ROOT, "oracle"), "binding"], check=True)
+        subprocess.run(["make", "-s", "-C", os.path.join(ROOT, "oracle"), "binding", f"REFERENCE={reference}"], check=True)
     return p if os.access(p, os.X_OK) else None
 
 

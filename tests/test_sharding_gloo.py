@@ -161,3 +161,53 @@ def test_shared_table_in_place_rows_gloo(tmp_path):
         assert status == "ok"
         sums.append(checksum)
     assert sums[0] == sums[1] == sums[2], sums  # the table's checksum does not depend on how many ranks wrote it
+
+
+def _dworker(rank, world, port, nwin, budget, out_dir):
+    """bench.dump_outputs on a window table sharded over the ranks: every rank sends its sampled rows to rank 0."""
+    os.environ["MASTER_ADDR"] = "127.0.0.1"
+    os.environ["MASTER_PORT"] = str(port)
+    dist.init_process_group("gloo", rank=rank, world_size=world)
+    import types
+    import bench
+    from popgenomicstools_b200.sharding import SharedTable
+    bounds = np.linspace(0, nwin, world + 1).astype(int)
+    w_lo, w_hi = int(bounds[rank]), int(bounds[rank + 1])
+    tab = SharedTable(("label", "sum_a", "fst"), nwin, rank, world, dist, torch=torch, backend="shm", tag="pgt_dump_gloo_test",
+                      w_lo=w_lo, w_hi=w_hi)
+    # the /dev/shm layout indexes rows globally, so every rank's rows stay valid; only the dump's gather path changes
+    tab.placement = "sharded"
+    want = _dump_table(nwin)
+    rows = tab.rows()
+    for k, v in want.items():
+        rows[k][:] = v[w_lo:w_hi]
+    dist.barrier()
+    bench.dump_outputs(out_dir, tab, types.SimpleNamespace(rank=rank, world=world, dev=torch.device("cpu"), torch=torch, dist=dist),
+                       budget=budget)
+    dist.barrier()
+    tab.close()
+    dist.destroy_process_group()
+
+
+def _dump_table(nwin):
+    rng = np.random.default_rng(5)
+    return dict(label=rng.integers(0, 1 << 32, nwin, dtype=np.uint32), sum_a=rng.random(nwin), fst=rng.random(nwin))
+
+
+def test_bench_dump_gathers_a_sharded_table_gloo(tmp_path):
+    nwin = 1000
+    want = _dump_table(nwin)
+    sampled = []
+    for world, budget in ((2, 1 << 20), (2, 4096 + 8 * 4 * 300), (3, 4096 + 8 * 4 * 300)):
+        d = tmp_path / f"dump_{world}_{budget}"
+        mp.spawn(_dworker, args=(world, _free_port(), nwin, budget, str(d)), nprocs=world, join=True)
+        idx = np.load(d / "window_index.npy")
+        if budget == 1 << 20:
+            assert np.array_equal(idx, np.arange(nwin))
+        else:
+            assert len(idx) == 300 and np.all(np.diff(idx) > 0)
+            sampled.append(idx)
+        for k, v in want.items():
+            got = np.load(d / f"{k}.npy")
+            assert got.dtype == np.float64 and np.array_equal(got, v[idx.astype(np.int64)].astype(np.float64)), (world, k)
+    assert np.array_equal(sampled[0], sampled[1])  # the same rows whatever the number of ranks
