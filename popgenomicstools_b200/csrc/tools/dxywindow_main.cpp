@@ -72,14 +72,6 @@ struct Maf {
 	}
 };
 
-struct MafChunk {
-	size_t begin, end;    // byte range
-	uint64_t nlines = 0;  // lines in the chunk
-	uint64_t row0 = 0;    // first site index
-	std::vector<ContigRun> runs;
-	long bad_line = -1;
-};
-
 // tokenizeStr, dxyWindow.cpp:141-153: chr, unsigned pos, three single chars, double, int
 static bool parse_maf_line(const char* p, const char* le, const char** name_b, const char** name_e, uint32_t* pos, double* f, int32_t* n) {
 	const char* s = skip_ws(p, le);
@@ -165,11 +157,7 @@ static int report_maf(int rc, const char* path, const char* which) {
 static int parse_maf(const Input& in, Maf* m, const char* path) {
 	if (pgtcol::is_colfile(in.data, in.size)) {  // cached columns of one population
 		pgtcol::View v;
-		std::string err;
-		if (pgtcol::open_view(in.data, in.size, &v, &err) != 0 || v.kind != pgtcol::KIND_MAF) {
-			fprintf(stderr, "dxyWindow: %s: %s\n", path, err.empty() ? "columnar file of another tool" : err.c_str());
-			return -1;
-		}
+		if (pgtcol::open_view_of(in.data, in.size, pgtcol::KIND_MAF, &v, "dxyWindow", path) != 0) return -1;
 		m->n = v.nsites;  // the columns are the file mapping itself (`in` outlives the Maf)
 		m->pos = (const uint32_t*)v.col[0];
 		m->freq = (const double*)v.col[1];
@@ -182,36 +170,8 @@ static int parse_maf(const Input& in, Maf* m, const char* path) {
 	size_t begin = nl ? (size_t)(nl + 1 - in.data) : in.size;
 	size_t n_eff = begin + effective_size(in.data + begin, in.size - begin);
 	const unsigned nt = (n_eff - begin) < parallel_min_bytes() ? 1 : parse_threads();
-	std::vector<size_t> starts = chunk_starts(in.data, begin, n_eff, nt);
-	std::vector<MafChunk> chunks(starts.size() - 1);
-	for (size_t i = 0; i + 1 < starts.size(); ++i) {
-		chunks[i].begin = starts[i];
-		chunks[i].end = starts[i + 1];
-	}
-	auto for_chunks = [&](auto fn) {
-		std::vector<std::thread> th;
-		for (MafChunk& c : chunks) th.emplace_back(fn, std::ref(c));
-		for (auto& x : th) x.join();
-	};
-	// pass 1: lines per chunk, so that pass 2 writes straight into the final columns (no per-chunk
-	// vectors and no serial concatenation: that was 100 of 170 ms per 3 M-line file on 8 threads)
-	for_chunks([&](MafChunk& c) {
-		const char* p = in.data + c.begin;
-		const char* e = in.data + c.end;
-		uint64_t k = 0;
-		while (p < e) {
-			const char* q = (const char*)memchr(p, '\n', (size_t)(e - p));
-			++k;
-			if (!q) break;
-			p = q + 1;
-		}
-		c.nlines = k;
-	});
 	uint64_t n = 0;
-	for (MafChunk& c : chunks) {
-		c.row0 = n;
-		n += c.nlines;
-	}
+	std::vector<TextChunk> chunks = split_lines(in.data, begin, n_eff, nt, nt, &n);
 	uint32_t* pos = (uint32_t*)malloc(std::max<uint64_t>(n, 1) * sizeof(uint32_t));
 	double* freq = (double*)malloc(std::max<uint64_t>(n, 1) * sizeof(double));
 	int32_t* nind = (int32_t*)malloc(std::max<uint64_t>(n, 1) * sizeof(int32_t));
@@ -222,11 +182,9 @@ static int parse_maf(const Input& in, Maf* m, const char* path) {
 		fprintf(stderr, "dxyWindow: out of memory for %llu sites of %s\n", (unsigned long long)n, path);
 		return -1;
 	}
-	for_chunks([&](MafChunk& c) {
+	for_chunks(chunks, nt, [&](TextChunk& c, size_t) {
 		const char* p = in.data + c.begin;
 		const char* e = in.data + c.end;
-		const char* prev = nullptr;
-		size_t prev_len = 0;
 		uint64_t row = c.row0;
 		long li = 0;
 		while (p < e) {
@@ -240,12 +198,7 @@ static int parse_maf(const Input& in, Maf* m, const char* path) {
 				if (c.bad_line < 0) c.bad_line = li;
 				nb = ne = p;
 			}
-			if (!prev || (size_t)(ne - nb) != prev_len || memcmp(prev, nb, prev_len) != 0) {
-				c.runs.push_back(ContigRun{std::string(nb, ne), 0});
-				prev = nb;
-				prev_len = (size_t)(ne - nb);
-			}
-			c.runs.back().count++;
+			c.add_row(nb, ne);
 			pos[row] = ps;
 			freq[row] = f;
 			nind[row] = ni;
@@ -255,12 +208,10 @@ static int parse_maf(const Input& in, Maf* m, const char* path) {
 			p = q + 1;
 		}
 	});
-	for (MafChunk& c : chunks) {
-		if (c.bad_line >= 0) {
-			fprintf(stderr, "dxyWindow: cannot parse line %llu of %s\n", (unsigned long long)(2 + c.row0 + c.bad_line), path);
-			return -1;
-		}
-		append_runs(m->runs, c.runs);
+	const int64_t bad = merge_chunks(chunks, &m->runs);
+	if (bad >= 0) {
+		fprintf(stderr, "dxyWindow: cannot parse line %llu of %s\n", (unsigned long long)(2 + bad), path);
+		return -1;
 	}
 	m->n = n;
 	m->pos = pos;

@@ -92,13 +92,7 @@ static bool stream_f64(const char*& p, const char* e, double* v) {
 
 enum : uint8_t { ROW_OK = 0, ROW_STALE_SCORE = 1, ROW_BLANK = 2 };
 
-struct Chunk {
-	size_t begin, end;
-	uint64_t nlines = 0, row0 = 0;
-	std::vector<ContigRun> runs;             // a run named kSame continues the previous chunk's last run
-	std::vector<std::pair<uint64_t, uint8_t>> head_fix;  // rows at the chunk head that depend on the previous chunk
-};
-static const char* kSame = "\x01";
+static const char* kSame = "\x01";  // name of a chunk's first run when it continues the previous chunk's last run
 
 int main(int argc, char** argv) {
 	unsigned winsize = 100000;  // ihsWindow.cpp:194, xpehhWindow.cpp:199
@@ -203,13 +197,7 @@ int main(int argc, char** argv) {
 	if (!pack_path) warm.start();
 	pgtcol::View view;
 	const bool columnar = pgtcol::is_colfile(in.data, in.size);
-	if (columnar) {
-		std::string err;
-		if (pgtcol::open_view(in.data, in.size, &view, &err) != 0 || view.kind != pgtcol::KIND_SCORE) {
-			fprintf(stderr, "%s: %s: %s\n", kTool, argv[1], err.empty() ? "columnar file of another tool" : err.c_str());
-			return -1;
-		}
-	}
+	if (columnar && pgtcol::open_view_of(in.data, in.size, pgtcol::KIND_SCORE, &view, kTool, argv[1]) != 0) return -1;
 	size_t begin = 0;
 #if defined(PGT_TOOL_XPEHH)
 	if (!columnar) {  // skip header (xpehhWindow.cpp:110-115)
@@ -224,34 +212,8 @@ int main(int argc, char** argv) {
 	const size_t text_end = columnar ? begin : in.size;  // columnar input: nothing to parse
 	const unsigned nt = (text_end - begin) < parallel_min_bytes() ? 1 : parse_threads();
 	tm.threads = nt;
-	std::vector<size_t> starts = chunk_starts(in.data, begin, text_end, nt);
-	std::vector<Chunk> chunks(starts.size() - 1);
-	for (size_t i = 0; i + 1 < starts.size(); ++i) {
-		chunks[i].begin = starts[i];
-		chunks[i].end = starts[i + 1];
-	}
-	auto count_lines = [&](Chunk& c) {
-		const char* p = in.data + c.begin;
-		const char* e = in.data + c.end;
-		uint64_t k = 0;
-		while (p < e) {
-			const char* q = (const char*)memchr(p, '\n', (size_t)(e - p));
-			++k;
-			if (!q) break;
-			p = q + 1;
-		}
-		c.nlines = k;
-	};
-	{
-		std::vector<std::thread> th;
-		for (Chunk& c : chunks) th.emplace_back(count_lines, std::ref(c));
-		for (auto& x : th) x.join();
-	}
 	uint64_t n = 0;
-	for (Chunk& c : chunks) {
-		c.row0 = n;
-		n += c.nlines;
-	}
+	std::vector<TextChunk> chunks = split_lines(in.data, begin, text_end, nt, nt, &n);
 	if (columnar) n = view.nsites;
 	uint32_t* pos = columnar ? (uint32_t*)view.col[0] : (uint32_t*)malloc(std::max<uint64_t>(n, 1) * sizeof(uint32_t));
 	double* score = columnar ? (double*)view.col[1] : (double*)malloc(std::max<uint64_t>(n, 1) * sizeof(double));
@@ -259,15 +221,14 @@ int main(int argc, char** argv) {
 		fprintf(stderr, "%s: out of memory for %llu sites\n", kTool, (unsigned long long)n);
 		return -1;
 	}
-	auto parse_chunk = [&](Chunk& c) {
+	// Values a row inherits from the row before it (stream semantics above) are copied on the spot, unless that
+	// row is itself still waiting for the previous CHUNK's last row: the dependency is then recorded in the
+	// chunk's head_fix and resolved in row order after all chunks are parsed.
+	std::vector<std::vector<std::pair<uint64_t, uint8_t>>> head_fix(chunks.size());
+	for_chunks(chunks, nt, [&](TextChunk& c, size_t ci) {
 		const char* p = in.data + c.begin;
 		const char* e = in.data + c.end;
 		uint64_t row = c.row0;
-		const char* prev_name = nullptr;
-		size_t prev_len = 0;
-		// Values a row inherits from the row before it (stream semantics above) are copied on the spot,
-		// unless that row is itself still waiting for the previous CHUNK's last row: the dependency is
-		// then recorded in head_fix and resolved in row order after all chunks are parsed.
 		bool pend_pos = true, pend_score = true;  // "row - 1 is unresolved": true at the chunk head
 		while (p < e) {
 			const char* q = (const char*)memchr(p, '\n', (size_t)(e - p));
@@ -280,16 +241,11 @@ int main(int argc, char** argv) {
 					pos[row] = pos[row - 1];
 					score[row] = score[row - 1];
 				} else {
-					c.head_fix.emplace_back(row, ROW_BLANK);
+					head_fix[ci].emplace_back(row, ROW_BLANK);
 					pend_pos = pend_score = true;
 				}
-				if (have_prev) {
-					c.runs.back().count++;
-				} else {
-					c.runs.push_back(ContigRun{kSame, 1});
-					prev_name = kSame;
-					prev_len = 1;
-				}
+				if (have_prev) c.runs.back().count++;
+				else c.runs.push_back(ContigRun{kSame, 1});
 			} else {
 				const char* us = (const char*)memchr(s, '_', (size_t)(t - s));
 				const char* ne = us ? us : t;  // extractChr
@@ -303,7 +259,7 @@ int main(int argc, char** argv) {
 						pos[row] = pos[row - 1];
 					} else {
 						pos[row] = 0;
-						c.head_fix.emplace_back(row, ROW_BLANK);  // takes pos and score of the previous row
+						head_fix[ci].emplace_back(row, ROW_BLANK);  // takes pos and score of the previous row
 						deferred = true;
 						pend_pos = pend_score = true;
 					}
@@ -337,37 +293,27 @@ int main(int argc, char** argv) {
 					if (!pend_score) {
 						score[row] = score[row - 1];
 					} else {
-						c.head_fix.emplace_back(row, ROW_STALE_SCORE);
+						head_fix[ci].emplace_back(row, ROW_STALE_SCORE);
 						pend_score = true;
 					}
 				}
-				if (!prev_name || (size_t)(ne - s) != prev_len || memcmp(prev_name, s, prev_len) != 0) {
-					c.runs.push_back(ContigRun{std::string(s, ne), 0});
-					prev_name = s;
-					prev_len = (size_t)(ne - s);
-				}
-				c.runs.back().count++;
+				c.add_row(s, ne);
 			}
 			++row;
 			if (!q) break;
 			p = q + 1;
 		}
-	};
-	{
-		std::vector<std::thread> th;
-		for (Chunk& c : chunks) th.emplace_back(parse_chunk, std::ref(c));
-		for (auto& x : th) x.join();
-	}
+	});
 	// rows at a chunk head that repeat the previous chunk's last row (sequential, rare)
 	std::vector<ContigRun> runs;
 	if (columnar) runs = view.runs;
-	for (Chunk& c : chunks) {
-		for (auto& fx : c.head_fix) {
+	for (size_t ci = 0; ci < chunks.size(); ++ci) {
+		for (auto& fx : head_fix[ci]) {
 			const uint64_t r = fx.first;
 			if (fx.second == ROW_BLANK) pos[r] = r ? pos[r - 1] : 0u;
 			score[r] = r ? score[r - 1] : 0.0;
 		}
-		for (const ContigRun& r : c.runs) {
+		for (const ContigRun& r : chunks[ci].runs) {
 			if (r.name == kSame) {
 				if (runs.empty()) runs.push_back(ContigRun{std::string(), r.count});
 				else runs.back().count += r.count;

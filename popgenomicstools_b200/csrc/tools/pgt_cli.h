@@ -441,26 +441,82 @@ inline size_t effective_size(const char* d, size_t n) {
 	return q < n ? q + 1 : n;
 }
 
-inline std::vector<size_t> chunk_starts(const char* d, size_t begin, size_t n, unsigned nthreads) {
-	std::vector<size_t> st;
-	st.push_back(begin);
-	for (unsigned t = 1; t < nthreads; ++t) {
-		size_t guess = begin + (n - begin) / nthreads * t;
-		if (guess <= st.back()) continue;
-		const char* q = (const char*)memchr(d + guess, '\n', n - guess);
-		if (!q) break;
-		size_t s = (size_t)(q + 1 - d);
-		if (s > st.back() && s < n) st.push_back(s);
+// A line-aligned byte range of the text.  Its lines are counted first, so that its parser thread writes rows
+// [row0, row0 + nlines) straight into the final columns: no per-chunk vectors and no serial concatenation (that
+// was 100 of 170 ms per 3 M-line MAF on 8 threads).
+struct TextChunk {
+	size_t begin = 0, end = 0;  // byte range
+	uint64_t nlines = 0;        // lines in the range (a last line without '\n' counts)
+	uint64_t row0 = 0;          // first output row
+	std::vector<ContigRun> runs;
+	long bad_line = -1;         // chunk-local index of the first malformed line
+
+	// the next row's contig name is [s, e): it extends the last run or starts a new one
+	void add_row(const char* s, const char* e) {
+		const size_t len = (size_t)(e - s);
+		if (runs.empty() || runs.back().name.size() != len || memcmp(runs.back().name.data(), s, len) != 0)
+			runs.push_back(ContigRun{std::string(s, e), 0});
+		runs.back().count++;
 	}
-	st.push_back(n);
-	return st;
+};
+
+// run `fn(chunk, index)` over all chunks on nt threads (the calling thread is one of them), chunks taken in file order
+template <class Fn>
+inline void for_chunks(std::vector<TextChunk>& chunks, unsigned nt, Fn fn) {
+	std::atomic<size_t> next{0};
+	auto worker = [&]() {
+		for (size_t i = next++; i < chunks.size(); i = next++) fn(chunks[i], i);
+	};
+	std::vector<std::thread> th;
+	for (unsigned t = 1; t < nt && t < chunks.size(); ++t) th.emplace_back(worker);
+	worker();
+	for (auto& x : th) x.join();
 }
 
-inline void append_runs(std::vector<ContigRun>& dst, const std::vector<ContigRun>& src) {
-	for (const ContigRun& r : src) {
-		if (!dst.empty() && dst.back().name == r.name) dst.back().count += r.count;
-		else dst.push_back(r);
+// [begin, end) of d cut at line starts into at most nchunks chunks (at least one), their lines counted on nt threads
+// and row0 set; *nrows = the lines of all chunks
+inline std::vector<TextChunk> split_lines(const char* d, size_t begin, size_t end, unsigned nchunks, unsigned nt, uint64_t* nrows) {
+	std::vector<TextChunk> chunks(1);
+	chunks[0].begin = begin;
+	for (unsigned t = 1; t < nchunks; ++t) {
+		const size_t guess = begin + (end - begin) / nchunks * t;
+		if (guess <= chunks.back().begin) continue;
+		const char* q = (const char*)memchr(d + guess, '\n', end - guess);
+		if (!q) break;
+		const size_t s = (size_t)(q + 1 - d);
+		if (s > chunks.back().begin && s < end) {
+			chunks.back().end = s;
+			chunks.emplace_back();
+			chunks.back().begin = s;
+		}
 	}
+	chunks.back().end = end;
+	for_chunks(chunks, nt, [d](TextChunk& c, size_t) {
+		for (const char *p = d + c.begin, *e = d + c.end; p < e; ++c.nlines) {
+			const char* q = (const char*)memchr(p, '\n', (size_t)(e - p));
+			p = q ? q + 1 : e;
+		}
+	});
+	uint64_t n = 0;
+	for (TextChunk& c : chunks) {
+		c.row0 = n;
+		n += c.nlines;
+	}
+	*nrows = n;
+	return chunks;
+}
+
+// Appends the chunks' runs to *runs in file order (a run cut by a chunk boundary becomes one again).  Returns the row
+// of the first malformed line in file order, or -1 when there is none.
+inline int64_t merge_chunks(const std::vector<TextChunk>& chunks, std::vector<ContigRun>* runs) {
+	for (const TextChunk& c : chunks) {
+		if (c.bad_line >= 0) return (int64_t)c.row0 + c.bad_line;
+		for (const ContigRun& r : c.runs) {
+			if (!runs->empty() && runs->back().name == r.name) runs->back().count += r.count;
+			else runs->push_back(r);
+		}
+	}
+	return -1;
 }
 
 // ---- output ----------------------------------------------------------------------------
@@ -720,7 +776,7 @@ struct Timing {
 // ---- streaming upload of the tools' columns (pgt_uploader, include/pgt_scan.h) -----------------------------
 //
 // One GPU, an input of some size: the columns become device-resident while the producer is still running.
-// Text: the parser threads finish chunks in file order and a feeder queues the rows of the finished prefix;
+// Text: the parser thread that finishes a chunk queues that chunk's rows (rows_ready only enqueues, any order);
 // the uploader's copy threads stage them through the pinned ring, so the wall time is max(parse, upload), not
 // their sum.  Columnar cache: the file's column blocks are read with pread straight into the ring (no
 // page-cache mapping handed to the driver).  Afterwards the scan runs in PGT_MEM_DEVICE and only the window rows
@@ -817,7 +873,7 @@ struct ColumnStreamer {
 		});
 	}
 
-	// rows [lo, hi) of every column are final in host memory (called by the tools' feeder thread)
+	// rows [lo, hi) of every column are final in host memory (called by the parser threads, one range per chunk)
 	void rows_ready(uint64_t lo, uint64_t hi) {
 		if (!on || failed.load()) return;
 		std::lock_guard<std::mutex> lk(mu);
@@ -830,9 +886,13 @@ struct ColumnStreamer {
 		if (!on) return -1;
 		const double t0 = now_ms();
 		if (th.joinable()) th.join();
-		uint64_t sent = 0;
+		uint64_t sent = 0, want = 0;
+		for (int c = 0; c < ncol; ++c) want += n * cols[c].elem;
 		if (!failed.load() && pgt_uploader_drain(up, &sent) != PGT_OK) {
 			why = pgt_last_error();
+			failed.store(true);
+		} else if (!failed.load() && sent != want) {  // rows never queued: the scan would read unwritten device memory
+			why = "uploaded " + std::to_string(sent) + " of " + std::to_string(want) + " column bytes";
 			failed.store(true);
 		}
 		if (failed.load()) {

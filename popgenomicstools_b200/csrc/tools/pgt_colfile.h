@@ -181,5 +181,13 @@ inline int open_view(const char* d, size_t n, View* v, std::string* err) {
 	return 0;
 }
 
+// open_view for a tool that reads `kind`: 0 ok; otherwise prints "<tool>: <path>: <why>" and returns -1
+inline int open_view_of(const char* d, size_t n, uint32_t kind, View* v, const char* tool, const char* path) {
+	std::string err;
+	if (open_view(d, n, v, &err) == 0 && v->kind == kind) return 0;
+	fprintf(stderr, "%s: %s: %s\n", tool, path, err.empty() ? "columnar file of another tool" : err.c_str());
+	return -1;
+}
+
 }  // namespace pgtcol
 #endif

@@ -16,8 +16,6 @@
 // exits without touching the GPU; a `.pgtc` file given as the input (magic sniff) skips the parsing.
 // Set PGT_TIMING=1 for a JSON timing line on stderr (parse / scan / format, opt-in so stderr
 // stays byte-identical by default); PGT_DEVICE selects the GPU, PGT_THREADS the parser threads.
-#include <atomic>
-
 #include "pgt_cli.h"
 #include "pgt_colfile.h"
 
@@ -43,14 +41,6 @@ static void info(unsigned winsize, unsigned stepsize) {
 	       "(4) window midpoint position\n%s(6) Number sites in window\n\n",
 	       kUsageLine, winsize, stepsize, kStatName);
 }
-
-struct Chunk {
-	size_t begin, end;      // byte range
-	uint64_t nlines = 0;    // lines in the chunk
-	uint64_t row0 = 0;      // first output row
-	std::vector<ContigRun> runs;
-	long bad_line = -1;     // chunk-local index of the first malformed line
-};
 
 int main(int argc, char** argv) {
 	unsigned winsize = 1, stepsize = 1;  // fstWindow.cpp:161-162
@@ -97,54 +87,15 @@ int main(int argc, char** argv) {
 #endif
 	pgtcol::View view;
 	const bool columnar = pgtcol::is_colfile(in.data, in.size);
-	if (columnar) {
-		std::string err;
-		if (pgtcol::open_view(in.data, in.size, &view, &err) != 0 || view.kind != want_kind) {
-			fprintf(stderr, "%s: %s: %s\n", kTool, argv[1], err.empty() ? "columnar file of another tool" : err.c_str());
-			return -1;
-		}
-	}
+	if (columnar && pgtcol::open_view_of(in.data, in.size, want_kind, &view, kTool, argv[1]) != 0) return -1;
 	const size_t n_eff = columnar ? 0 : effective_size(in.data, in.size);
 	const unsigned nt = n_eff < parallel_min_bytes() ? 1 : parse_threads();
 	tm.threads = nt;
-	// Many more chunks than threads, handed out in file order: the prefix of finished rows advances steadily,
-	// and the uploader below sends it to the device while the rest is still being parsed.
+	// Many more chunks than threads, handed out in file order: rows reach the uploader below chunk by chunk
+	// while the rest is still being parsed.
 	const unsigned nchunk_want = (nt > 1 && n_eff >= ((size_t)64 << 20)) ? nt * 8 : nt;
-	std::vector<size_t> starts = chunk_starts(in.data, 0, n_eff, nchunk_want);
-	std::vector<Chunk> chunks(starts.size() - 1);
-	for (size_t i = 0; i + 1 < starts.size(); ++i) {
-		chunks[i].begin = starts[i];
-		chunks[i].end = starts[i + 1];
-	}
-	auto count_lines = [&](Chunk& c) {
-		const char* p = in.data + c.begin;
-		const char* e = in.data + c.end;
-		uint64_t k = 0;
-		while (p < e) {
-			const char* q = (const char*)memchr(p, '\n', (size_t)(e - p));
-			++k;
-			if (!q) break;
-			p = q + 1;
-		}
-		c.nlines = k;
-	};
-	// run `fn(chunk)` over all chunks on nt threads, chunks taken in file order
-	auto for_chunks = [&](auto fn) {
-		std::atomic<size_t> next{0};
-		auto worker = [&]() {
-			for (size_t i = next++; i < chunks.size(); i = next++) fn(chunks[i]);
-		};
-		std::vector<std::thread> th;
-		for (unsigned t = 1; t < nt && t < chunks.size(); ++t) th.emplace_back(worker);
-		worker();
-		for (auto& x : th) x.join();
-	};
-	for_chunks(count_lines);
 	uint64_t n = 0;
-	for (Chunk& c : chunks) {
-		c.row0 = n;
-		n += c.nlines;
-	}
+	std::vector<TextChunk> chunks = split_lines(in.data, 0, n_eff, nchunk_want, nt, &n);
 	if (columnar) n = view.nsites;
 	// columnar input: the columns are the file mapping itself (read-only from here on)
 	uint32_t* pos = columnar ? (uint32_t*)view.col[0] : (uint32_t*)malloc(std::max<uint64_t>(n, 1) * sizeof(uint32_t));
@@ -173,14 +124,10 @@ int main(int argc, char** argv) {
 	// straight from the cache file (pread into the pinned ring); the scan then reads HBM, not host memory.
 	ColumnStreamer streamer;
 	if (!pack_path && n > 0) streamer.start(&warm, scol, nscol, n, (uint64_t)n / stepsize + 65536, 28, columnar ? argv[1] : nullptr);
-	std::vector<std::atomic<unsigned char>> chunk_done(chunks.size());
-	for (auto& f : chunk_done) f.store(0);
-	auto parse_chunk = [&](Chunk& c) {
+	for_chunks(chunks, nt, [&](TextChunk& c, size_t) {
 		const char* p = in.data + c.begin;
 		const char* e = in.data + c.end;
 		uint64_t row = c.row0;
-		const char* prev_name = nullptr;
-		size_t prev_len = 0;
 		long li = 0;
 		while (p < e) {
 			const char* s;
@@ -222,58 +169,20 @@ int main(int argc, char** argv) {
 			// hetWindow.cpp:78-80 only distinguishes g < 0, g == 1, other
 			geno[row] = (int8_t)(g < 0 ? -1 : (g > 127 ? 127 : g));
 #endif
-			if (!prev_name || (size_t)(t - s) != prev_len || memcmp(prev_name, s, prev_len) != 0) {
-				c.runs.push_back(ContigRun{std::string(s, t), 0});
-				prev_name = s;
-				prev_len = (size_t)(t - s);
-			}
-			c.runs.back().count++;
+			c.add_row(s, t);
 			++row;
 			++li;
 			if (!q) break;
 			p = q + 1;
 		}
-	};
-	{
-		// the feeder follows the prefix of finished chunks and queues its rows for upload
-		std::atomic<bool> parse_over{false};
-		std::thread feeder;
-		if (streamer.active() && !columnar) {
-			feeder = std::thread([&]() {
-				size_t ci = 0;
-				uint64_t sent = 0;
-				while (ci < chunks.size()) {
-					if (!chunk_done[ci].load(std::memory_order_acquire)) {
-						if (parse_over.load()) break;  // a chunk failed: nothing more will arrive
-						std::this_thread::sleep_for(std::chrono::microseconds(200));
-						continue;
-					}
-					uint64_t upto = chunks[ci].row0 + chunks[ci].nlines;
-					while (ci + 1 < chunks.size() && chunk_done[ci + 1].load(std::memory_order_acquire)) {
-						++ci;
-						upto = chunks[ci].row0 + chunks[ci].nlines;
-					}
-					++ci;
-					streamer.rows_ready(sent, upto);
-					sent = upto;
-				}
-			});
-		}
-		for_chunks([&](Chunk& c) {
-			parse_chunk(c);
-			chunk_done[&c - chunks.data()].store(1, std::memory_order_release);
-		});
-		parse_over.store(true);
-		if (feeder.joinable()) feeder.join();
-	}
+		if (!columnar) streamer.rows_ready(c.row0, c.row0 + c.nlines);
+	});
 	std::vector<ContigRun> runs;
 	if (columnar) runs = view.runs;
-	for (Chunk& c : chunks) {
-		if (c.bad_line >= 0) {
-			fprintf(stderr, "%s: cannot parse line %llu of %s\n", kTool, (unsigned long long)(c.row0 + c.bad_line + 1), argv[1]);
-			return -1;
-		}
-		append_runs(runs, c.runs);
+	const int64_t bad = merge_chunks(chunks, &runs);
+	if (bad >= 0) {
+		fprintf(stderr, "%s: cannot parse line %llu of %s\n", kTool, (unsigned long long)(bad + 1), argv[1]);
+		return -1;
 	}
 	tm.sites = n;
 	tm.parse_ms = now_ms() - t_start;
