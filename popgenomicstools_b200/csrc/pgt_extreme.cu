@@ -37,18 +37,8 @@
 #include <thread>
 #include <vector>
 
-#include "../../include/pgt_extreme.h"
 #include "../../include/pgt_synth.h"
-#include "pgt_internal.h"
-
-static int xcuda_fail(cudaError_t e, const char* what) {
-	return pgt_set_error(PGT_ERR_CUDA, std::string(what) + ": " + cudaGetErrorName(e) + " (" + cudaGetErrorString(e) + ")");
-}
-#define PGT_CUDA(call)                                         \
-	do {                                                       \
-		cudaError_t e__ = (call);                              \
-		if (e__ != cudaSuccess) return xcuda_fail(e__, #call); \
-	} while (0)
+#include "pgt_cuda.h"
 
 static const uint32_t kDefaultUnit = 2048;
 
@@ -567,26 +557,6 @@ extern "C" int pgt_synth_score(uint64_t seed, uint64_t site0, uint64_t n, double
 
 namespace {
 
-struct XProf {
-	cudaEvent_t a = nullptr, b = nullptr;
-	cudaStream_t st;
-	int kind;
-	bool on;
-	XProf(int k, cudaStream_t s) : st(s), kind(k), on(pgt_profile_enabled()) {
-		if (!on) return;
-		if (cudaEventCreate(&a) != cudaSuccess || cudaEventCreate(&b) != cudaSuccess) {
-			on = false;
-			return;
-		}
-		cudaEventRecord(a, st);
-	}
-	~XProf() {
-		if (!on) return;
-		cudaEventRecord(b, st);
-		pgt_profile_push(kind, a, b);
-	}
-};
-
 size_t xalign(size_t x) { return (x + 255) / 256 * 256; }
 
 struct XLayout {
@@ -680,7 +650,7 @@ int x_run(const XDev& P, uint64_t nsite, uint64_t nunit, const double* score, co
 		int per_sm = 0;
 		if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_xsmall<MODE>, 256, smem) != cudaSuccess || per_sm < 1) per_sm = 1;
 		const uint64_t cap = (uint64_t)x_num_sms() * per_sm;
-		XProf prof(2, st);
+		ProfScope prof(2, st);
 		uint64_t* bw = part.idx;  // the partials are not used on this path: >= nw entries, and nw >= nbatches + 1 (checked by the caller)
 		k_xbatches<<<(unsigned)((nbatches + 256) / 256), 256, 0, st>>>(P, nbatches, bw);
 		pgt_count_launch();
@@ -690,7 +660,7 @@ int x_run(const XDev& P, uint64_t nsite, uint64_t nunit, const double* score, co
 		return PGT_OK;
 	}
 	if (nsite) {
-		XProf prof(2, st);
+		ProfScope prof(2, st);
 		// lanes per unit from the mean unit length: short windows get narrow groups, so that every
 		// lane still streams several rounds of 8 loads per unit
 		const uint64_t mean = nunit ? nsite / nunit : 0;
@@ -706,7 +676,7 @@ int x_run(const XDev& P, uint64_t nsite, uint64_t nunit, const double* score, co
 		PGT_CUDA(cudaGetLastError());
 	}
 	if (P.nw) {
-		XProf prof(3, st);
+		ProfScope prof(3, st);
 		k_xwindows<MODE><<<(unsigned)((P.nw + 255) / 256), 256, 0, st>>>(P, pos, part, out);
 		pgt_count_launch();
 		PGT_CUDA(cudaGetLastError());
@@ -761,7 +731,7 @@ extern "C" int pgt_scan_extreme(const pgt_xplan* plan, const pgt_range* range, p
 	int ndev = 0;
 	{
 		cudaError_t e = cudaGetDeviceCount(&ndev);
-		if (e != cudaSuccess || ndev == 0) return xcuda_fail(e != cudaSuccess ? e : cudaErrorNoDevice, "pgt_scan_extreme: no usable CUDA device");
+		if (e != cudaSuccess || ndev == 0) return cuda_fail(e != cudaSuccess ? e : cudaErrorNoDevice, "pgt_scan_extreme: no usable CUDA device");
 	}
 	cudaStream_t st = (cudaStream_t)stream;
 	unsigned char* ws = (unsigned char*)(((uintptr_t)workspace + 255) / 256 * 256);
@@ -831,11 +801,15 @@ extern "C" int pgt_scan_extreme(const pgt_xplan* plan, const pgt_range* range, p
 			site_tmp.resize(L.nw);
 			h_site = site_tmp.data();
 		}
-		if (out->ext_value) PGT_CUDA(cudaMemcpyAsync(out->ext_value, dout.ext_value, L.nw * sizeof(double), cudaMemcpyDeviceToHost, st));
-		if (h_site) PGT_CUDA(cudaMemcpyAsync(h_site, dout.ext_site, L.nw * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
-		if (out->prop) PGT_CUDA(cudaMemcpyAsync(out->prop, dout.prop, L.nw * sizeof(double), cudaMemcpyDeviceToHost, st));
-		if (out->nbig) PGT_CUDA(cudaMemcpyAsync(out->nbig, dout.nbig, L.nw * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
-		if (out->nsites) PGT_CUDA(cudaMemcpyAsync(out->nsites, dout.nsites, L.nw * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+		pgt_xwindows host = *out;  // (ext_pos: gathered below)
+		host.ext_site = h_site;
+		host.ext_pos = nullptr;
+		cudaError_t e = cudaSuccess;
+		auto back = [&](auto* h, auto* d) {
+			if (e == cudaSuccess && h) e = cudaMemcpyAsync(h, d, L.nw * sizeof(*h), cudaMemcpyDeviceToHost, st);
+		};
+		for_each_xfield(back, host, dout);
+		if (e != cudaSuccess) return cuda_fail(e, "cudaMemcpyAsync(window table -> host)");
 		PGT_CUDA(cudaStreamSynchronize(st));
 		if (out->ext_pos) {
 			for (uint64_t w = 0; w < L.nw; ++w) out->ext_pos[w] = h_site[w] == ~0ull ? 0u : pos[h_site[w] - origin];

@@ -5,6 +5,7 @@
 #include <string>
 #include <vector>
 
+#include "../../include/pgt_extreme.h"
 #include "../../include/pgt_scan.h"
 #include "pgt_geom.h"
 
@@ -41,5 +42,25 @@ uint64_t pgt_plan_unit_start(const pgt_plan* p, uint64_t j);
 uint64_t pgt_plan_windows_within(const pgt_plan* p, uint64_t w, uint64_t w_hi, uint64_t limit);
 // contig c with off[c] <= x < off[c+1]
 uint32_t pgt_plan_contig_of(const pgt_plan* p, uint64_t x);
+
+// The per-window arrays of one or more result tables, member by member: fn(a.sum_a, b.sum_a), fn(a.sum_b, b.sum_b), ...
+// for_each_value visits the nine values the window kernels write, in the order of the slots of a host-mode output
+// table; for_each_field visits all fourteen arrays.  (dxy_global is one triple per scan, not a per-window array.)
+template <class F, class... T>
+void for_each_value(F&& fn, T&... t) {
+	fn(t.sum_a...), fn(t.sum_b...), fn(t.fst...), fn(t.nhet...), fn(t.nonmissing...), fn(t.het...), fn(t.dxy...), fn(t.neffective...),
+	    fn(t.nskip...);
+}
+template <class F, class... T>
+void for_each_field(F&& fn, T&... t) {
+	fn(t.label...), fn(t.start_pos...), fn(t.end_pos...), fn(t.mid_pos...), fn(t.nsites...);
+	for_each_value(fn, t...);
+}
+// the same for extreme-score tables, in the order of the host-mode staging blocks; ext_pos last (host-memory scans
+// gather it on the host)
+template <class F, class... T>
+void for_each_xfield(F&& fn, T&... t) {
+	fn(t.ext_value...), fn(t.ext_site...), fn(t.prop...), fn(t.nbig...), fn(t.nsites...), fn(t.ext_pos...);
+}
 
 #endif

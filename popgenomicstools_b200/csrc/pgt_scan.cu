@@ -38,28 +38,13 @@
 #include <type_traits>
 #include <vector>
 
-#include "../../include/pgt_extreme.h"
-#include "pgt_internal.h"
+#include "pgt_cuda.h"
 
 // ----------------------------------------------------------------------------- utilities
 
 static std::atomic<uint64_t> g_launches{0};
 extern "C" uint64_t pgt_kernel_launch_count(void) { return g_launches.load(); }
 void pgt_count_launch() { g_launches++; }
-
-static int cuda_fail(cudaError_t e, const char* what) {
-	return pgt_set_error(PGT_ERR_CUDA, std::string(what) + ": " + cudaGetErrorName(e) + " (" + cudaGetErrorString(e) + ")");
-}
-#define PGT_CUDA(call)                                         \
-	do {                                                       \
-		cudaError_t e__ = (call);                              \
-		if (e__ != cudaSuccess) return cuda_fail(e__, #call);  \
-	} while (0)
-#define PGT_TRY(call)                    \
-	do {                                 \
-		int rc__ = (call);               \
-		if (rc__ != PGT_OK) return rc__; \
-	} while (0)
 
 extern "C" int pgt_device_count(void) {
 	int n = 0;
@@ -119,8 +104,7 @@ extern "C" int pgt_host_unregister(void* p) {
 	return PGT_OK;
 }
 
-// ---- optional per-kernel timing (bench.py roofline): CUDA events on the launching stream
-// kinds: 0 = level 1 (k_units*), 1 = level 2 (k_windows*), 2 / 3 = level 1 / 2 of the extreme scan
+// ---- optional per-kernel timing (bench.py roofline): CUDA events on the launching stream (ProfScope, pgt_cuda.h)
 struct ProfEvent {
 	cudaEvent_t a, b;
 	int kind;
@@ -136,27 +120,6 @@ void pgt_profile_push(int kind, void* ev_a, void* ev_b) {
 	std::lock_guard<std::mutex> lk(g_prof_mutex);
 	g_prof_events.push_back(ProfEvent{(cudaEvent_t)ev_a, (cudaEvent_t)ev_b, kind});
 }
-
-struct ProfScope {
-	cudaStream_t st;
-	ProfEvent ev;
-	bool on;
-	ProfScope(int kind, cudaStream_t s) : st(s), on(g_profile) {
-		if (!on) return;
-		ev.kind = kind;
-		if (cudaEventCreate(&ev.a) != cudaSuccess || cudaEventCreate(&ev.b) != cudaSuccess) {
-			on = false;
-			return;
-		}
-		cudaEventRecord(ev.a, st);
-	}
-	~ProfScope() {
-		if (!on) return;
-		cudaEventRecord(ev.b, st);
-		std::lock_guard<std::mutex> lk(g_prof_mutex);
-		g_prof_events.push_back(ev);
-	}
-};
 
 extern "C" int pgt_profile(int enable) {
 	g_profile = enable != 0;
@@ -229,6 +192,12 @@ static int num_sms() {
 
 static size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
 
+// Grid of a grid-stride kernel that wants `want` blocks: at most 8 per SM.
+static unsigned capped_grid(uint64_t want) {
+	const uint64_t cap = (uint64_t)num_sms() * 8;
+	return (unsigned)(want < cap ? want : cap);
+}
+
 // Grid of a grid-stride kernel: the blocks that are resident at once (one wave), or fewer when the work is small.
 // (A fixed cap of 8 blocks per SM launched the per-site kernel -- 6 resident blocks at 40 registers -- as one full wave
 // plus a third of one: ncu "waves per SM 1.33", profiles/r02h_persite_ncu_details.txt.)
@@ -250,30 +219,44 @@ static unsigned one_wave_grid(K kern, int threads, uint64_t want_blocks) {
 static const uint64_t kSlabSites = 1ull << 22;  // PGT_MEM_HOST: sites (entries) staged per slab
 static const uint64_t kSlabSlack = 8192;         // >= 2 units
 
+// One input column: where its pointer lives inside Cols, and its bytes per site.
 struct ColDesc {
-	const void* ptr;        // host pointer (PGT_MEM_HOST) or device pointer
-	size_t elem;            // bytes per site
-	size_t offset_in_cols;  // byte offset of the pointer member inside Cols
+	size_t member;  // offsetof(Cols, ...)
+	uint32_t elem;
 };
 
-// the columns a statistic reads, in staging order; `c` may be NULL (sizing only)
-static int stat_columns(pgt_stat stat, pgt_mode mode, const pgt_columns* c, ColDesc* d) {
+// The columns a statistic reads, in staging order -- pos first in bp mode, then a b f1 f2 n1 n2 g.  The tiled and
+// sliding-tile kernels read their staged columns in this order.
+static int stat_columns(pgt_stat stat, pgt_mode mode, ColDesc* d) {
 	int n = 0;
-	auto put = [&](const void* p, size_t e, size_t off) { d[n++] = ColDesc{p, e, off}; };
-	if (mode == PGT_MODE_BP) put(c ? c->pos : nullptr, 4, offsetof(Cols, pos));
+	if (mode == PGT_MODE_BP) d[n++] = {offsetof(Cols, pos), 4};
 	if (stat == PGT_STAT_FST || stat == PGT_STAT_FUSED) {
-		put(c ? c->a : nullptr, 8, offsetof(Cols, a));
-		put(c ? c->b : nullptr, 8, offsetof(Cols, b));
+		d[n++] = {offsetof(Cols, a), 8};
+		d[n++] = {offsetof(Cols, b), 8};
 	}
 	if (stat == PGT_STAT_DXY || stat == PGT_STAT_FUSED) {
-		put(c ? c->f1 : nullptr, 8, offsetof(Cols, f1));
-		put(c ? c->f2 : nullptr, 8, offsetof(Cols, f2));
-		put(c ? c->n1 : nullptr, 4, offsetof(Cols, n1));
-		put(c ? c->n2 : nullptr, 4, offsetof(Cols, n2));
+		d[n++] = {offsetof(Cols, f1), 8};
+		d[n++] = {offsetof(Cols, f2), 8};
+		d[n++] = {offsetof(Cols, n1), 4};
+		d[n++] = {offsetof(Cols, n2), 4};
 	}
-	if (stat == PGT_STAT_HET || stat == PGT_STAT_FUSED) put(c ? c->geno : nullptr, 1, offsetof(Cols, g));
+	if (stat == PGT_STAT_HET || stat == PGT_STAT_FUSED) d[n++] = {offsetof(Cols, g), 1};
 	return n;
 }
+static const void* col_ptr(const Cols& c, const ColDesc& d) {
+	const void* p;
+	memcpy(&p, (const char*)&c + d.member, sizeof(p));
+	return p;
+}
+static void set_col_ptr(Cols* c, const ColDesc& d, const void* p) { memcpy((char*)c + d.member, &p, sizeof(p)); }
+
+static Cols cols_from(const pgt_columns& c, int minind) { return Cols{c.pos, c.a, c.b, c.geno, c.f1, c.f2, c.n1, c.n2, minind}; }
+
+template <class Stat>
+static constexpr pgt_stat kStatOf = std::is_same<Stat, FstStat>::value   ? PGT_STAT_FST
+                                    : std::is_same<Stat, HetStat>::value ? PGT_STAT_HET
+                                    : std::is_same<Stat, DxyStat>::value ? PGT_STAT_DXY
+                                                                         : PGT_STAT_FUSED;
 
 static size_t acc_bytes(pgt_stat stat) {
 	switch (stat) {
@@ -284,28 +267,7 @@ static size_t acc_bytes(pgt_stat stat) {
 	}
 }
 
-struct Layout {
-	uint64_t w_lo, w_hi, u_lo, u_hi, g_hi, origin;
-	size_t segs_off, off_off, siteoff_off, gpart_off, units_off, pre_off, bounds_off, stage_off, outs_off, tileseg_off, total;
-	uint64_t tileseg_cap;   // entries of the tile -> segment table (0 = not used: few segments)
-	bool hgw;               // level 2 in scan mode
-	bool unit_table;        // very many segments: level 1 reads unit starts from a table (k_unit_starts) instead of the segment records
-	bool slide;             // fine steps: windows straight from the sites (k_slide), no unit array
-	bool persite;           // W = S = 1: elementwise (k_windows_persite), no unit array
-	uint32_t slide_stages;
-	size_t slide_smem;
-	uint64_t gsite_lo, gsite_hi;  // global sites this scan owns for dxyWindow's global line
-	size_t gslab_off;             // host mode without units: one global-line triple per slab
-	uint64_t out_slab_rows;       // host mode without units: rows of each of the two slab-sized output tables
-	uint64_t gslab_cap;
-	uint64_t blk_lo, blk_hi;  // scan blocks covering [u_lo, u_hi)
-	size_t stage_col_bytes[8];
-	uint64_t slab_sites;
-};
-
 // Sliding-tile scan (k_slide): shared-memory shape, and whether the geometry takes that path at all.
-// The choice fixes the summation order, so it is a pure function of (W, S, unit, statistic) and the
-// tuning knob -- never of the input size, the window range or the shard.
 struct SlideShape {
 	uint32_t E, wpb, G, wp, nstages, stage_bytes, sf_off, pr_off, pos_off, stage_off, ncol;
 	uint32_t col_off[kMaxStageCols], col_cap[kMaxStageCols];
@@ -320,7 +282,7 @@ static void slide_footprint(const pgt_geom& g, pgt_stat stat, SlideShape* sh) {
 	sh->G = tm.G;
 	sh->wp = (uint32_t)align_up(g.W, 32);
 	ColDesc d[8];
-	const int nc = stat_columns(stat, PGT_MODE_SITES, nullptr, d);
+	const int nc = stat_columns(stat, PGT_MODE_SITES, d);
 	uint32_t o = 0;
 	for (int c = 0; c <= nc; ++c) {  // column nc = pos (uint32); a stage holds the G blocks of a step
 		sh->col_off[c] = o;
@@ -368,6 +330,34 @@ static bool slide_shape(const pgt_geom& g, pgt_mode mode, pgt_stat stat, SlideSh
 	return false;
 }
 
+// The kernel path of a scan of `stat` over `plan` (PGT_PATH_*), and for the sliding tile its shape.  The path fixes
+// the summation order, so it is a function of (W, S, unit, statistic) and the tuning knobs only -- never of the input
+// size, the window range or the shard.
+static int scan_path(const pgt_plan* plan, pgt_stat stat, SlideShape* sh) {
+	if (slide_shape(plan->g, plan->mode, stat, sh)) return PGT_PATH_SLIDE;
+	if (plan->mode == PGT_MODE_SITES && plan->g.W == 1 && plan->g.S == 1 && g_tune_level2 != 1) return PGT_PATH_PERSITE;
+	return PGT_PATH_UNITS;
+}
+
+struct Layout {
+	uint64_t w_lo, w_hi, u_lo, u_hi, g_hi, origin;
+	size_t segs_off, off_off, siteoff_off, gpart_off, units_off, pre_off, bounds_off, stage_off, outs_off, tileseg_off, total;
+	uint64_t tileseg_cap;  // entries of the tile -> segment table (0 = not used: few segments)
+	bool hgw;              // level 2 in scan mode
+	bool unit_table;       // very many segments: level 1 reads unit starts from a table (k_unit_starts) instead of the segment records
+	// PGT_PATH_UNITS: level 1 (unit partials) + level 2.  PGT_PATH_SLIDE (fine steps: k_slide) and PGT_PATH_PERSITE
+	// (W = S = 1: k_windows_persite) form the windows straight from the sites: no unit array, no level 2.
+	int path;
+	SlideShape slide;             // PGT_PATH_SLIDE
+	uint64_t gsite_lo, gsite_hi;  // global sites this scan owns for dxyWindow's global line
+	size_t gslab_off;             // host mode without units: one global-line triple per slab
+	uint64_t out_slab_rows;       // host mode without units: rows of each of the two slab-sized output tables
+	uint64_t gslab_cap;
+	uint64_t blk_lo, blk_hi;  // scan blocks covering [u_lo, u_hi)
+	size_t stage_col_bytes[8];
+	uint64_t slab_sites;
+};
+
 static int make_layout(const pgt_plan* plan, const pgt_range* range, pgt_stat stat, pgt_mem mem, Layout* L) {
 	if (!plan) return pgt_set_error(PGT_ERR_ARGS, "plan is NULL");
 	if ((int)stat < 0 || (int)stat > (int)PGT_STAT_FUSED) return pgt_set_error(PGT_ERR_ARGS, "unknown statistic");
@@ -407,16 +397,8 @@ static int make_layout(const pgt_plan* plan, const pgt_range* range, pgt_stat st
 	// sites owned for the global line (same boundaries as the units [u_lo, g_hi))
 	L->gsite_lo = pgt_plan_unit_start(plan, L->u_lo);
 	L->gsite_hi = pgt_plan_unit_start(plan, L->g_hi);
-	{
-		SlideShape sh;
-		L->slide = slide_shape(plan->g, plan->mode, stat, &sh);
-		if (L->slide) {
-			L->slide_stages = sh.nstages;
-			L->slide_smem = sh.smem;
-		}
-		L->persite = !L->slide && plan->mode == PGT_MODE_SITES && plan->g.W == 1 && plan->g.S == 1 && g_tune_level2 != 1;
-	}
-	const bool nounits = L->slide || L->persite;  // windows come straight from the sites: no unit array, no level 2
+	L->path = scan_path(plan, stat, &L->slide);
+	const bool nounits = L->path != PGT_PATH_UNITS;
 	const uint64_t nunits = nounits ? 0 : L->u_hi - L->u_lo;
 	size_t o = 0;
 	L->segs_off = o;
@@ -462,7 +444,7 @@ static int make_layout(const pgt_plan* plan, const pgt_range* range, pgt_stat st
 	if (mem == PGT_MEM_HOST) {
 		L->slab_sites = std::min<uint64_t>(kSlabSites, std::max<uint64_t>(plan->nsites, 1)) + kSlabSlack;
 		ColDesc d[8];
-		const int nc = stat_columns(stat, plan->mode, nullptr, d);
+		const int nc = stat_columns(stat, plan->mode, d);
 		for (int i = 0; i < nc; ++i) L->stage_col_bytes[i] = align_up((size_t)L->slab_sites * d[i].elem, 256);
 		for (int s = 0; s < 2; ++s)
 			for (int i = 0; i < nc; ++i) o += L->stage_col_bytes[i];
@@ -488,9 +470,7 @@ extern "C" int pgt_plan_scan_path(const pgt_plan* plan, pgt_stat stat) {
 	if (!plan) return pgt_set_error(PGT_ERR_ARGS, "pgt_plan_scan_path: plan is NULL");
 	if ((int)stat < 0 || (int)stat > (int)PGT_STAT_FUSED) return pgt_set_error(PGT_ERR_ARGS, "unknown statistic");
 	SlideShape sh;
-	if (slide_shape(plan->g, plan->mode, stat, &sh)) return PGT_PATH_SLIDE;
-	if (plan->mode == PGT_MODE_SITES && plan->g.W == 1 && plan->g.S == 1 && g_tune_level2 != 1) return PGT_PATH_PERSITE;
-	return PGT_PATH_UNITS;
+	return scan_path(plan, stat, &sh);
 }
 
 extern "C" size_t pgt_plan_device_bytes(const pgt_plan* plan) {
@@ -537,36 +517,44 @@ extern "C" int pgt_tune(const char* key, int value) {
 	return PGT_OK;
 }
 
+// the statistic's columns of `c` for the tiled and sliding-tile kernels, in staging order
 struct StatCols {
 	const void* ptr[kMaxTileCols];
 	uint32_t elem[kMaxTileCols];
 	uint32_t n;
 };
 template <class Stat>
-static StatCols tile_columns(const Cols& c);
-template <>
-StatCols tile_columns<FstStat>(const Cols& c) { return StatCols{{c.a, c.b}, {8, 8}, 2}; }
-template <>
-StatCols tile_columns<HetStat>(const Cols& c) { return StatCols{{c.g}, {1}, 1}; }
-template <>
-StatCols tile_columns<DxyStat>(const Cols& c) { return StatCols{{c.f1, c.f2, c.n1, c.n2}, {8, 8, 4, 4}, 4}; }
-template <>
-StatCols tile_columns<FusedStat>(const Cols& c) { return StatCols{{c.a, c.b, c.f1, c.f2, c.n1, c.n2, c.g}, {8, 8, 8, 8, 4, 4, 1}, 7}; }
+static StatCols tile_columns(const Cols& c) {
+	ColDesc d[8];
+	StatCols sc;
+	sc.n = (uint32_t)stat_columns(kStatOf<Stat>, PGT_MODE_SITES, d);
+	for (uint32_t i = 0; i < sc.n; ++i) {
+		sc.ptr[i] = col_ptr(c, d[i]);
+		sc.elem[i] = d[i].elem;
+	}
+	return sc;
+}
+
+// what the tiled level-1 kernel stages: bytes per site, and `nstages` stages of at most `stage_bytes` each
+// (pgt_tune "stages" / "stage_kb", at most 224 KB in all)
+struct TileBudget {
+	uint32_t bps, nstages, stage_bytes;
+};
+static TileBudget tile_budget(const StatCols& sc) {
+	TileBudget b{0, (uint32_t)g_tune_stages, (uint32_t)g_tune_stage_kb * 1024u};
+	for (uint32_t c = 0; c < sc.n; ++c) b.bps += sc.elem[c];
+	if (b.nstages * b.stage_bytes > 224u * 1024u) b.stage_bytes = 224u * 1024u / b.nstages;
+	return b;
+}
 
 template <class Stat, bool INDIRECT>
-static int launch_units_tiled(const DevPlan& P, const Cols& cols, typename Stat::Acc* units, const uint64_t* bounds, uint64_t valid_elems,
-                              uint32_t* tileseg, uint64_t tileseg_cap, cudaStream_t st) {
+static int launch_units_tiled(const DevPlan& P, const StatCols& sc, const TileBudget& tb, int minind, typename Stat::Acc* units,
+                              const uint64_t* bounds, uint64_t valid_elems, uint32_t* tileseg, uint64_t tileseg_cap, cudaStream_t st) {
 	const uint64_t nunits = P.unit_hi - P.unit_lo;
-	const StatCols sc = tile_columns<Stat>(cols);
-	uint32_t bps = 0;
-	for (uint32_t c = 0; c < sc.n; ++c) bps += sc.elem[c];
 	const int nsm = num_sms();
 	// `nstages` stages of <= `stage_kb` KB; tiles of whole units; at least ~4 tiles per SM when the input allows
-	uint32_t nstages = (uint32_t)g_tune_stages;
-	uint32_t stage_budget = (uint32_t)g_tune_stage_kb * 1024u;
-	if (nstages * stage_budget > 224u * 1024u) stage_budget = 224u * 1024u / nstages;
-	uint32_t tsites = (stage_budget - 48u * sc.n) / bps;
-	if (tsites > 16384u && bps > 1) tsites = 16384u;  // (the 1-byte genotype column alone fills a stage with ~110 K sites)
+	uint32_t tsites = (tb.stage_bytes - 48u * sc.n) / tb.bps;
+	if (tsites > 16384u && tb.bps > 1) tsites = 16384u;  // (the 1-byte genotype column alone fills a stage with ~110 K sites)
 	uint32_t m = tsites / P.g.ueff;
 	if (m < 1) m = 1;
 	{
@@ -598,8 +586,8 @@ static int launch_units_tiled(const DevPlan& P, const Cols& cols, typename Stat:
 	memset(&tc, 0, sizeof(tc));
 	tc.ncol = sc.n;
 	tc.m = m;
-	tc.nstages = nstages;
-	tc.minind = cols.minind;
+	tc.nstages = tb.nstages;
+	tc.minind = minind;
 	tc.valid_elems = valid_elems;
 	uint32_t o = 0;
 	for (uint32_t c = 0; c < sc.n; ++c) {
@@ -610,7 +598,7 @@ static int launch_units_tiled(const DevPlan& P, const Cols& cols, typename Stat:
 		o += tc.col_cap[c];
 	}
 	tc.stage_bytes = (uint32_t)align_up(o, 128);
-	const size_t smem = kTileCtlBytes + nstages * (size_t)tc.stage_bytes;
+	const size_t smem = kTileCtlBytes + tb.nstages * (size_t)tc.stage_bytes;
 	void (*kern)(DevPlan, TileCfg, typename Stat::Acc*, const uint64_t*);
 	switch (P.g.gw) {
 		case 1: kern = k_units_tiled<Stat, 1, INDIRECT>; break;
@@ -637,21 +625,6 @@ static int launch_units_tiled(const DevPlan& P, const Cols& cols, typename Stat:
 	return PGT_OK;
 }
 
-// hetWindow: the vectorised byte kernel replaces the generic direct kernel
-template <class Stat>
-static bool launch_het_vec(const DevPlan&, const Cols&, typename Stat::Acc*, const uint64_t*, uint64_t, cudaStream_t) {
-	return false;
-}
-template <>
-bool launch_het_vec<HetStat>(const DevPlan& P, const Cols& cols, HetStat::Acc* units, const uint64_t* bounds, uint64_t want, cudaStream_t st) {
-	const uint64_t cap = (uint64_t)num_sms() * 8;
-	const unsigned grid = (unsigned)(want < cap ? want : cap);
-	ProfScope prof(0, st);
-	if (bounds) k_units_het_vec<true><<<grid, 256, 0, st>>>(P, cols.g, units, bounds);
-	else k_units_het_vec<false><<<grid, 256, 0, st>>>(P, cols.g, units, bounds);
-	return true;
-}
-
 // valid_elems: number of elements every column is known to hold from element 0
 template <class Stat>
 static int launch_units(const DevPlan& P, const Cols& cols, typename Stat::Acc* units, const uint64_t* bounds, uint64_t valid_elems,
@@ -664,31 +637,30 @@ static int launch_units(const DevPlan& P, const Cols& cols, typename Stat::Acc* 
 	// matter (measured on B200, profiles/): the TMA-staged tiled kernel wins on big inputs
 	// (no sector over-fetch, bytes in flight without registers), the direct kernel on small ones
 	// (no pipeline fill) and for the 1-byte genotype column.
-	uint32_t bps = 0;
-	{
-		const StatCols sc = tile_columns<Stat>(cols);
-		for (uint32_t c = 0; c < sc.n; ++c) bps += sc.elem[c];
-	}
-	const uint64_t approx_bytes = nunits * (uint64_t)P.g.ueff * bps;
+	const StatCols sc = tile_columns<Stat>(cols);
+	const TileBudget tb = tile_budget(sc);
+	const uint64_t approx_bytes = nunits * (uint64_t)P.g.ueff * tb.bps;
 	// (hetWindow's 1-byte column stays on the vectorised direct kernel: measured at 3e9 sites, 4096-site units,
 	// 6.14 TB/s direct against 5.44 TB/s through the ring -- both were issue-bound on the byte counting, 4.5 and
 	// 4.3 TB/s, until it went from POPC to dp4a; the ring's het consumer remains for forced / short-unit runs)
-	bool tiled = P.g.gw != 32 || (bps > 1 && approx_bytes >= (256ull << 20));
+	bool tiled = P.g.gw != 32 || (tb.bps > 1 && approx_bytes >= (256ull << 20));
 	if (g_tune_level1 == 2) tiled = true;
 	if (g_tune_level1 == 1 && P.g.gw == 32) tiled = false;
-	{
-		// a tile holds whole units: very long units (unit_sites up to 4096) may not fit a stage;
-		// they always have gw == 32, so the direct kernel applies
-		uint32_t nst = (uint32_t)g_tune_stages, budget = (uint32_t)g_tune_stage_kb * 1024u;
-		if (nst * budget > 224u * 1024u) budget = 224u * 1024u / nst;
-		if ((uint64_t)P.g.ueff * bps + 64ull * kMaxTileCols > budget) tiled = false;
-	}
+	// a tile holds whole units: very long units (unit_sites up to 4096) may not fit a stage;
+	// they always have gw == 32, so the direct kernel applies
+	if ((uint64_t)P.g.ueff * tb.bps + 64ull * kMaxTileCols > tb.stage_bytes) tiled = false;
 	if (tiled)
-		return bounds ? launch_units_tiled<Stat, true>(P, cols, units, bounds, valid_elems, nullptr, 0, st)
-		              : launch_units_tiled<Stat, false>(P, cols, units, bounds, valid_elems, tileseg, tileseg_cap, st);
+		return bounds ? launch_units_tiled<Stat, true>(P, sc, tb, cols.minind, units, bounds, valid_elems, nullptr, 0, st)
+		              : launch_units_tiled<Stat, false>(P, sc, tb, cols.minind, units, bounds, valid_elems, tileseg, tileseg_cap, st);
 	const int threads = 256;
 	const uint64_t want = (nunits + 7) / 8;  // one warp per unit, 8 warps per block
-	if (launch_het_vec<Stat>(P, cols, units, bounds, want, st)) {
+	if constexpr (std::is_same<Stat, HetStat>::value) {  // hetWindow: the vectorised byte kernel replaces the generic direct kernel
+		const unsigned grid = capped_grid(want);
+		{
+			ProfScope prof(0, st);
+			if (bounds) k_units_het_vec<true><<<grid, 256, 0, st>>>(P, cols.g, units, bounds);
+			else k_units_het_vec<false><<<grid, 256, 0, st>>>(P, cols.g, units, bounds);
+		}
 		g_launches++;
 		PGT_CUDA(cudaGetLastError());
 		return PGT_OK;
@@ -712,9 +684,7 @@ static int launch_units(const DevPlan& P, const Cols& cols, typename Stat::Acc* 
 
 static int launch_bounds_kernel(const DevPlan& P, const uint32_t* pos, uint64_t ndata, uint64_t* bounds, cudaStream_t st) {
 	const uint64_t nb = P.unit_hi - P.unit_lo + 1;
-	const uint64_t want = (nb + 255) / 256;
-	const uint64_t cap = (uint64_t)num_sms() * 8;
-	k_bp_bounds<<<(unsigned)(want < cap ? want : cap), 256, 0, st>>>(P, pos, ndata, bounds);
+	k_bp_bounds<<<capped_grid((nb + 255) / 256), 256, 0, st>>>(P, pos, ndata, bounds);
 	g_launches++;
 	PGT_CUDA(cudaGetLastError());
 	return PGT_OK;
@@ -726,15 +696,11 @@ static int launch_windows(const DevPlan& P, typename Stat::Acc* units, uint64_t 
                           bool hgw, typename Stat::Acc* pre, uint64_t blk_lo, uint64_t blk_hi, cudaStream_t st) {
 	const uint64_t nwin = P.win_hi - P.win_lo;
 	if (nwin == 0) return PGT_OK;
-	const uint64_t cap = (uint64_t)num_sms() * 8;
 	ProfScope prof(1, st);
 	if (hgw) {
-		const uint64_t nblk = blk_hi - blk_lo;
-		const uint64_t bcap = (uint64_t)num_sms() * 8;
-		k_block_scan<Stat><<<(unsigned)(nblk < bcap ? nblk : bcap), 256, 0, st>>>(P, units, pre, units_base, blk_lo, blk_hi);
+		k_block_scan<Stat><<<capped_grid(blk_hi - blk_lo), 256, 0, st>>>(P, units, pre, units_base, blk_lo, blk_hi);
 		g_launches++;
-		const uint64_t want = (nwin + 255) / 256;
-		k_windows_hgw<Stat><<<(unsigned)(want < cap ? want : cap), 256, 0, st>>>(P, units, pre, units_base, pos, out);
+		k_windows_hgw<Stat><<<capped_grid((nwin + 255) / 256), 256, 0, st>>>(P, units, pre, units_base, pos, out);
 	} else if (P.g.wunits <= 32 && g_tune_level2 != 1) {
 		// fine windows: a thread per window
 		void (*kern)(DevPlan, const typename Stat::Acc*, uint64_t, const uint32_t*, pgt_windows);
@@ -745,47 +711,35 @@ static int launch_windows(const DevPlan& P, typename Stat::Acc* units, uint64_t 
 		else if (wu <= 8) kern = k_windows_small<Stat, 8>;
 		else if (wu <= 16) kern = k_windows_small<Stat, 16>;
 		else kern = k_windows_small<Stat, 32>;
-		const uint64_t want = (nwin + 255) / 256;
-		kern<<<(unsigned)(want < cap ? want : cap), 256, 0, st>>>(P, units, units_base, pos, out);
+		kern<<<capped_grid((nwin + 255) / 256), 256, 0, st>>>(P, units, units_base, pos, out);
 	} else {
-		const uint64_t want = (nwin + 7) / 8;  // few windows: a warp each; many: runs per block, stored 32 rows at a time
-		k_windows<Stat><<<(unsigned)(want < cap ? want : cap), 256, 0, st>>>(P, units, units_base, pos, out);
+		// few windows: a warp each; many: runs per block, stored 32 rows at a time
+		k_windows<Stat><<<capped_grid((nwin + 7) / 8), 256, 0, st>>>(P, units, units_base, pos, out);
 	}
 	g_launches++;
 	PGT_CUDA(cudaGetLastError());
 	return PGT_OK;
 }
 
+// dxyWindow's global line from the unit partials (two stages); nothing for the statistics without one
 template <class Stat>
-static int launch_global(const typename Stat::Acc*, uint64_t, double*, double*, cudaStream_t) {
-	return PGT_OK;
-}
-template <>
-int launch_global<DxyStat>(const DxyStat::Acc* units, uint64_t n, double* scratch, double* g3, cudaStream_t st) {
-	k_global_partial<DxyStat><<<kGlobalBlocks, 1024, 0, st>>>(units, n, scratch);
-	k_global_final<<<1, kGlobalBlocks, 0, st>>>(scratch, kGlobalBlocks, g3);
-	g_launches += 2;
-	PGT_CUDA(cudaGetLastError());
-	return PGT_OK;
-}
-template <>
-int launch_global<FusedStat>(const FusedStat::Acc* units, uint64_t n, double* scratch, double* g3, cudaStream_t st) {
-	k_global_partial<FusedStat><<<kGlobalBlocks, 1024, 0, st>>>(units, n, scratch);
-	k_global_final<<<1, kGlobalBlocks, 0, st>>>(scratch, kGlobalBlocks, g3);
-	g_launches += 2;
-	PGT_CUDA(cudaGetLastError());
+static int launch_global(const typename Stat::Acc* units, uint64_t n, double* scratch, double* g3, cudaStream_t st) {
+	if constexpr (GlobalTerm<Stat>::has) {
+		k_global_partial<Stat><<<kGlobalBlocks, 1024, 0, st>>>(units, n, scratch);
+		k_global_final<<<1, kGlobalBlocks, 0, st>>>(scratch, kGlobalBlocks, g3);
+		g_launches += 2;
+		PGT_CUDA(cudaGetLastError());
+	}
 	return PGT_OK;
 }
 
-// Sliding-tile scan of the windows [P.win_lo, P.win_hi): the columns' element 0 is site P.site_origin and
-// they hold `valid_elems` elements.  `pos` may be NULL (host mode gathers positions on the host).
+// Sliding-tile scan of the windows [P.win_lo, P.win_hi) in the shape `sh` (Layout::slide): the columns' element 0 is
+// site P.site_origin and they hold `valid_elems` elements.  `pos` may be NULL (host mode gathers positions on the host).
 template <class Stat>
-static int launch_slide(const pgt_plan* plan, pgt_stat stat, const DevPlan& P, const Cols& cols, uint64_t valid_elems, const uint32_t* pos,
-                        const pgt_windows& out, double* gpart, double* g3, cudaStream_t st) {
+static int launch_slide(const pgt_plan* plan, const SlideShape& sh, const DevPlan& P, const Cols& cols, uint64_t valid_elems,
+                        const uint32_t* pos, const pgt_windows& out, double* gpart, double* g3, cudaStream_t st) {
 	const uint64_t nwin = P.win_hi - P.win_lo;
 	if (nwin == 0) return PGT_OK;
-	SlideShape sh;
-	if (!slide_shape(plan->g, plan->mode, stat, &sh)) return pgt_set_error(PGT_ERR_ARGS, "internal: sliding-tile scan not applicable");
 	const StatCols scol = tile_columns<Stat>(cols);
 	TileCfg tc;
 	memset(&tc, 0, sizeof(tc));
@@ -812,72 +766,58 @@ static int launch_slide(const pgt_plan* plan, pgt_stat stat, const DevPlan& P, c
 	sc.pos_col = pos ? scol.n : 0xffffffffu;
 	sc.stage_off = sh.stage_off;
 	sc.gpart = gpart;
-	auto finish_global = [&](unsigned grid) -> int {  // one partial triple per CTA -> the line
-		if (!gpart) return PGT_OK;
-		k_global_final<<<1, kGlobalBlocks, 0, st>>>(gpart, grid, g3);
-		g_launches++;
-		PGT_CUDA(cudaGetLastError());
-		return PGT_OK;
-	};
+	void (*kern)(DevPlan, TileCfg, SlideCfg, pgt_windows) = nullptr;
+	void (*k2)(DevPlan, TileCfg, SlideCfg, SlideCfg2, pgt_windows) = nullptr;
+	SlideCfg2 s2;
+	uint64_t slots;  // CTAs resident at once
+	if (std::is_same<Stat, FusedStat>::value && sh.G == 1 && g_tune_fused2 != 1) {
+		// two crews (fst + het, dxy) share the staged block; their SUF / PRE arrays partition the fused ones
+		const uint32_t part[2] = {24u, 16u};  // accumulator bytes per site: FstHetStat, DxyStat
+		uint32_t so = sh.sf_off, po = sh.pr_off;
+		for (int c = 0; c < 2; ++c) {
+			s2.wt_off[c] = kTileCtlBytes + 256u * c;
+			s2.sf_off[c] = so;
+			s2.pr_off[c] = po;
+			so += 2u * sh.wp * part[c];
+			po += sh.wp * part[c];
+		}
+		k2 = sh.E <= 4 ? k_slide_fused2<4> : (sh.E == 5 ? k_slide_fused2<5> : k_slide_fused2<6>);
+		PGT_CUDA(cudaFuncSetAttribute(k2, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sh.smem));
+		slots = (uint64_t)num_sms();
+	} else {
+		if (sh.G > 1) {
+			if (sh.E <= 2) kern = k_slide<Stat, 2, true>;
+			else if (sh.E <= 4) kern = k_slide<Stat, 4, true>;
+			else kern = k_slide<Stat, 6, true>;
+		} else {
+			if (sh.E <= 4) kern = k_slide<Stat, 4, false>;
+			else if (sh.E == 5) kern = k_slide<Stat, 5, false>;  // W = 1000
+			else kern = k_slide<Stat, 6, false>;
+		}
+		PGT_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sh.smem));
+		int per_sm = 0;
+		PGT_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, kSlideThreads, sh.smem));
+		slots = (uint64_t)num_sms() * (per_sm < 1 ? 1 : per_sm);
+	}
 	// chunks: ~4 per resident CTA for balance, but long enough (>= 32 steps of windows) that the W - S sites
 	// shared with the next chunk stay a few percent of what a chunk reads
 	const uint64_t wps = ((uint64_t)sh.G * plan->g.W + plan->g.S - 1) / plan->g.S;  // windows starting in one step
-	auto set_chunks = [&](uint64_t slots) {
-		sc.chunk_windows = std::max<uint64_t>(32 * wps, (nwin + slots * 4 - 1) / (slots * 4));
-		sc.nchunks = (nwin + sc.chunk_windows - 1) / sc.chunk_windows;
-	};
-	if constexpr (std::is_same<Stat, FusedStat>::value) {
-		if (sh.G == 1 && g_tune_fused2 != 1) {
-			// two crews (fst + het, dxy) share the staged block; their SUF / PRE arrays partition the fused ones
-			SlideCfg2 s2;
-			const uint32_t part[2] = {24u, 16u};  // accumulator bytes per site: FstHetStat, DxyStat
-			uint32_t so = sh.sf_off, po = sh.pr_off;
-			for (int c = 0; c < 2; ++c) {
-				s2.wt_off[c] = kTileCtlBytes + 256u * c;
-				s2.sf_off[c] = so;
-				s2.pr_off[c] = po;
-				so += 2u * sh.wp * part[c];
-				po += sh.wp * part[c];
-			}
-			void (*k2)(DevPlan, TileCfg, SlideCfg, SlideCfg2, pgt_windows) =
-			    sh.E <= 4 ? k_slide_fused2<4> : (sh.E == 5 ? k_slide_fused2<5> : k_slide_fused2<6>);
-			PGT_CUDA(cudaFuncSetAttribute(k2, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sh.smem));
-			const uint64_t slots = (uint64_t)num_sms();
-			set_chunks(slots);
-			const unsigned grid2 = (unsigned)std::min<uint64_t>(sc.nchunks, slots);
-			{
-				ProfScope prof(0, st);
-				k2<<<grid2, kSlide2Threads, sh.smem, st>>>(P, tc, sc, s2, out);
-			}
-			g_launches++;
-			PGT_CUDA(cudaGetLastError());
-			return finish_global(grid2);
-		}
-	}
-	void (*kern)(DevPlan, TileCfg, SlideCfg, pgt_windows);
-	if (sh.G > 1) {
-		if (sh.E <= 2) kern = k_slide<Stat, 2, true>;
-		else if (sh.E <= 4) kern = k_slide<Stat, 4, true>;
-		else kern = k_slide<Stat, 6, true>;
-	} else {
-		if (sh.E <= 4) kern = k_slide<Stat, 4, false>;
-		else if (sh.E == 5) kern = k_slide<Stat, 5, false>;  // W = 1000
-		else kern = k_slide<Stat, 6, false>;
-	}
-	PGT_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sh.smem));
-	int per_sm = 0;
-	PGT_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, kSlideThreads, sh.smem));
-	if (per_sm < 1) per_sm = 1;
-	const uint64_t slots = (uint64_t)num_sms() * per_sm;
-	set_chunks(slots);
+	sc.chunk_windows = std::max<uint64_t>(32 * wps, (nwin + slots * 4 - 1) / (slots * 4));
+	sc.nchunks = (nwin + sc.chunk_windows - 1) / sc.chunk_windows;
 	const unsigned grid = (unsigned)std::min<uint64_t>(sc.nchunks, slots);
 	{
 		ProfScope prof(0, st);
-		kern<<<grid, kSlideThreads, sh.smem, st>>>(P, tc, sc, out);
+		if (k2) k2<<<grid, kSlide2Threads, sh.smem, st>>>(P, tc, sc, s2, out);
+		else kern<<<grid, kSlideThreads, sh.smem, st>>>(P, tc, sc, out);
 	}
 	g_launches++;
 	PGT_CUDA(cudaGetLastError());
-	return finish_global(grid);
+	if (gpart) {  // one partial triple per CTA -> the line
+		k_global_final<<<1, kGlobalBlocks, 0, st>>>(gpart, grid, g3);
+		g_launches++;
+		PGT_CUDA(cudaGetLastError());
+	}
+	return PGT_OK;
 }
 
 // Do the sites the sliding-tile kernel counts as owned by its runs -- per segment from the first window's start to the
@@ -905,8 +845,8 @@ static bool slide_runs_cover_owned_sites(const pgt_plan* plan, const Layout& L) 
 // W = S = 1: the vectorised kernel when its preconditions hold (one segment; every used column and output pointer
 // 16-byte aligned at the scan's first window -- 4-byte aligned for the genotype column), else the scalar one.
 template <class Stat>
-static int launch_persite(const pgt_plan* plan, pgt_stat stat, const DevPlan& P, const Cols& C, const pgt_windows& out, double* gpart,
-                          double* g3, cudaStream_t st) {
+static int launch_persite(const pgt_plan* plan, const DevPlan& P, const Cols& C, const pgt_windows& out, double* gpart, double* g3,
+                          cudaStream_t st) {
 	const uint64_t nwin = P.win_hi - P.win_lo;
 	if (nwin == 0) return PGT_OK;
 	bool vec = g_tune_persite != 1 && plan->segs.size() == 1 && nwin >= 4;
@@ -915,21 +855,10 @@ static int launch_persite(const pgt_plan* plan, pgt_stat stat, const DevPlan& P,
 		site0 = plan->segs[0].site_base + (P.win_lo - plan->segs[0].win_base) - P.site_origin;
 		auto ok = [&](const void* p, size_t elem, size_t align) { return !p || (((uintptr_t)p + site0 * elem) & (align - 1)) == 0; };
 		ColDesc d[8];
-		pgt_columns pc;
-		memset(&pc, 0, sizeof(pc));
-		pc.a = C.a;
-		pc.b = C.b;
-		pc.geno = C.g;
-		pc.f1 = C.f1;
-		pc.f2 = C.f2;
-		pc.n1 = C.n1;
-		pc.n2 = C.n2;
-		const int nc = stat_columns(stat, PGT_MODE_SITES, &pc, d);
-		for (int i = 0; i < nc; ++i) vec = vec && d[i].ptr && ok(d[i].ptr, d[i].elem, d[i].elem == 1 ? 4 : 16);
+		const int nc = stat_columns(kStatOf<Stat>, PGT_MODE_SITES, d);
+		for (int i = 0; i < nc; ++i) vec = vec && col_ptr(C, d[i]) && ok(col_ptr(C, d[i]), d[i].elem, d[i].elem == 1 ? 4 : 16);
 		vec = vec && ok(C.pos, 4, 16);
-		const void* outs[14] = {out.label, out.start_pos, out.end_pos, out.mid_pos, out.nsites, out.sum_a, out.sum_b, out.fst,
-		                        out.nhet, out.nonmissing, out.het, out.dxy, out.neffective, out.nskip};
-		for (const void* p : outs) vec = vec && (((uintptr_t)p) & 15) == 0;
+		for_each_field([&](const void* p) { vec = vec && (((uintptr_t)p) & 15) == 0; }, out);
 	}
 	ProfScope prof(1, st);
 	unsigned grid;
@@ -977,18 +906,345 @@ static uint64_t host_site_lower_bound(const pgt_plan* plan, const uint64_t* site
 	return std::min(std::max(res, origin), origin + ndata);
 }
 
-struct HostStreams {
+// What the checks and set-up shared by both memory spaces establish for a scan.
+struct Scan {
+	const pgt_plan* plan;
+	pgt_stat stat;
+	Layout L;
+	DevPlan P;
+	Cols C;  // the caller's columns (device or host pointers)
+	const uint64_t* site_offsets;
+	const pgt_windows* out;
+	char* ws;
+	uint64_t* bounds;  // bp mode / unit table: unit bounds in the workspace
+	uint64_t ndata;    // bp mode: sites the columns hold
+	uint64_t nglobal;  // units the global line sums
+	bool bp, want_global;
+	cudaStream_t st;
+};
+
+// ---- PGT_MEM_DEVICE: the columns are read in place
+template <class Stat>
+static int scan_device(const Scan& s) {
+	const pgt_plan* plan = s.plan;
+	const Layout& L = s.L;
+	DevPlan P = s.P;
+	const uint64_t nunits = L.u_hi - L.u_lo;
+	const uint64_t nwin = L.w_hi - L.w_lo;
+	double* gpart = (double*)(s.ws + L.gpart_off);
+	if (L.path != PGT_PATH_UNITS) {
+		// windows straight from the sites: W = S = 1 (default arguments of fstWindow / hetWindow: an
+		// elementwise map) or the sliding tile for fine steps; no unit array, no level 2
+		bool global_done = false;
+		if (nwin) {
+			uint64_t first_site, last_site;
+			pgt_plan_window(plan, L.w_lo, &first_site, nullptr, nullptr);
+			pgt_plan_window(plan, L.w_hi - 1, nullptr, &last_site, nullptr);
+			P.col_elems = last_site + 1 - L.origin;
+			if (L.path == PGT_PATH_PERSITE) {
+				// the windows ARE the sites: when the owned range of the global line is exactly their span (always, unless the
+				// scan owns sites outside any window) the kernel adds its sites up on the way and the dxy columns are read once
+				global_done = s.want_global && GlobalTerm<Stat>::has && L.gsite_lo == first_site && L.gsite_hi == last_site + 1;
+				PGT_TRY(launch_persite<Stat>(plan, P, s.C, *s.out, global_done ? gpart : nullptr, s.out->dxy_global, s.st));
+			} else {
+				global_done = s.want_global && GlobalTerm<Stat>::has && g_tune_slideglobal != 1 && slide_runs_cover_owned_sites(plan, L);
+				PGT_TRY(launch_slide<Stat>(plan, L.slide, P, s.C, last_site + 1 - L.origin, s.C.pos, *s.out, global_done ? gpart : nullptr,
+				                           s.out->dxy_global, s.st));
+			}
+		}
+		if (s.want_global && !global_done) {
+			if (L.gsite_lo < L.origin) return pgt_set_error(PGT_ERR_ARGS, "site_origin lies after the first site this scan must read");
+			PGT_TRY(launch_global_sites(s.C, L.gsite_lo - L.origin, L.gsite_hi - L.origin, gpart, s.out->dxy_global, s.st));
+		}
+		return PGT_OK;
+	}
+	if (s.bp && nunits) PGT_TRY(launch_bounds_kernel(P, s.C.pos, s.ndata, s.bounds, s.st));
+	if (L.unit_table) {  // very many segments: unit starts once, then the INDIRECT level-1 kernels
+		k_unit_starts<<<capped_grid((nunits + 256) / 256), 256, 0, s.st>>>(P, s.bounds);
+		g_launches++;
+		PGT_CUDA(cudaGetLastError());
+	}
+	// elements the caller's columns are known to hold: up to the end of the last unit read
+	P.col_elems = s.bp ? s.ndata : pgt_plan_unit_start(plan, L.u_hi) - L.origin;
+	typename Stat::Acc* units = (typename Stat::Acc*)(s.ws + L.units_off);
+	PGT_TRY(launch_units<Stat>(P, s.C, units, s.bounds, P.col_elems, L.tileseg_cap ? (uint32_t*)(s.ws + L.tileseg_off) : nullptr,
+	                           L.tileseg_cap, s.st));
+	// the global line reads the raw unit partials: before level 2, which may scan them in place
+	if (s.want_global) PGT_TRY(launch_global<Stat>(units, s.nglobal, gpart, s.out->dxy_global, s.st));
+	return launch_windows<Stat>(P, units, L.u_lo, s.C.pos, *s.out, L.hgw, (typename Stat::Acc*)(s.ws + L.pre_off), L.blk_lo, L.blk_hi, s.st);
+}
+
+// ---- PGT_MEM_HOST: slabs of the axis are staged H2D on a copy stream (double-buffered) while the previous slab is
+// reduced; only unit partials stay on the device.  Positions are not copied in site mode: the two edge positions per
+// window are gathered on the host.
+struct HostStaging {
 	cudaStream_t copy = nullptr;
-	cudaEvent_t ready[2] = {nullptr, nullptr};
-	cudaEvent_t freed[2] = {nullptr, nullptr};
-	~HostStreams() {
+	cudaEvent_t ready[2] = {nullptr, nullptr};  // slot filled (copy stream)
+	cudaEvent_t freed[2] = {nullptr, nullptr};  // slot read by its kernels (`st`)
+	char* buf[2][8];                            // per slot, per column of `cd`
+	ColDesc cd[8];
+	int ncol = 0;
+	int slot = 0;
+	bool used[2] = {false, false};
+	~HostStaging() {
 		for (int i = 0; i < 2; ++i) {
 			if (ready[i]) cudaEventDestroy(ready[i]);
 			if (freed[i]) cudaEventDestroy(freed[i]);
 		}
 		if (copy) cudaStreamDestroy(copy);
 	}
+	// H2D of sites [s0, s0 + ns) of every column into the current slot, ordered after the kernels that last read it
+	int stage(const Scan& s, uint64_t s0, uint64_t ns, Cols* C) {
+		if (used[slot]) PGT_CUDA(cudaStreamWaitEvent(copy, freed[slot], 0));
+		*C = Cols{};
+		C->minind = s.C.minind;
+		for (int i = 0; i < ncol; ++i) {
+			const char* src = (const char*)col_ptr(s.C, cd[i]) + (s0 - s.L.origin) * cd[i].elem;
+			if (ns) PGT_CUDA(cudaMemcpyAsync(buf[slot][i], src, ns * cd[i].elem, cudaMemcpyHostToDevice, copy));
+			set_col_ptr(C, cd[i], buf[slot][i]);
+		}
+		PGT_CUDA(cudaEventRecord(ready[slot], copy));
+		PGT_CUDA(cudaStreamWaitEvent(s.st, ready[slot], 0));
+		return PGT_OK;
+	}
+	// the kernels enqueued on `st` since stage() are the last to read the slot; the next slab takes the other one
+	int release(cudaStream_t st) {
+		PGT_CUDA(cudaEventRecord(freed[slot], st));
+		used[slot] = true;
+		slot ^= 1;
+		return PGT_OK;
+	}
 };
+
+// Window bookkeeping on the host -- label, nsites, the two edge positions per window -- runs on worker threads next to
+// the copy pipeline.  (It cannot simply follow the slab loop: enqueueing ~10 operations per slab blocks once the
+// driver's queue is full, so the host would only get to it when most of the transfer is over; 3e7 windows take ~1 s on
+// one thread.)
+struct Bookkeeper {
+	std::vector<std::thread> th;
+	void join() {
+		for (auto& t : th)
+			if (t.joinable()) t.join();
+	}
+	~Bookkeeper() { join(); }
+};
+static void start_bookkeeping(const Scan& s, Bookkeeper* book) {
+	const pgt_windows* out = s.out;
+	const uint64_t nwin = s.L.w_hi - s.L.w_lo;
+	if (!nwin || !(out->label || out->nsites || out->start_pos || out->end_pos || out->mid_pos)) return;
+	unsigned nt = nwin < (1u << 16) ? 1u : std::min<unsigned>(8u, std::max(1u, std::thread::hardware_concurrency()));
+	const uint64_t per = (nwin + nt - 1) / nt;
+	for (unsigned t = 0; t < nt; ++t) {
+		const uint64_t wa = s.L.w_lo + per * t, wb = std::min<uint64_t>(s.L.w_hi, wa + per);
+		if (wa >= wb) break;
+		book->th.emplace_back([plan = s.plan, out, pos = s.C.pos, bp = s.bp, wa, wb, origin = s.L.origin, w_lo = s.L.w_lo]() {
+			uint32_t si = pgt_plan_seg_of_window(plan, wa);
+			for (uint64_t w = wa; w < wb; ++w) {
+				while (w >= plan->segs[si].win_base + plan->segs[si].nwin) ++si;
+				const pgt_seg& sg = plan->segs[si];
+				uint64_t fs;
+				const uint32_t n = pgt_window_sites(plan->g, sg, w - sg.win_base, &fs);
+				const uint64_t first = sg.site_base + fs, last = first + n - 1;
+				const uint32_t label = pgt_plan_contig_of(plan, last);
+				const uint64_t o = w - w_lo;
+				if (out->label) out->label[o] = label;
+				if (out->nsites) out->nsites[o] = n;
+				uint32_t sp = 0, ep = 0;
+				bool have = false;
+				if (bp) {
+					sp = (uint32_t)(first - plan->off[pgt_plan_contig_of(plan, first)]) + 1u;
+					ep = (uint32_t)(last - plan->off[label]) + 1u;
+					have = true;
+				} else if (pos) {
+					sp = pos[first - origin];
+					ep = pos[last - origin];
+					have = true;
+				}
+				if (have) {
+					if (out->start_pos) out->start_pos[o] = sp;
+					if (out->end_pos) out->end_pos[o] = ep;
+					if (out->mid_pos) out->mid_pos[o] = (sp + ep) / 2u;
+				}
+			}
+		});
+	}
+}
+
+// Per-window values are produced into device tables, then copied back: one table for the whole scan, or -- when the
+// windows come straight from the sites, slab by slab -- two slab-sized tables used in turn.  A table has 12 slots:
+// the nine values in slots 0-8, the global triple in slot 11.
+static pgt_windows device_table(const Scan& s, int which) {
+	const uint64_t rows = s.L.path == PGT_PATH_UNITS ? s.L.w_hi - s.L.w_lo : s.L.out_slab_rows;
+	const size_t ob = align_up((size_t)rows * 8 + 8, 256);
+	char* t = s.ws + s.L.outs_off + (size_t)which * 12 * ob;
+	pgt_windows d;
+	memset(&d, 0, sizeof(d));
+	int k = 0;
+	auto slot = [&](auto*& dp, auto* want) {
+		if (want) dp = (decltype(want))(t + ob * k);
+		++k;
+	};
+	for_each_value(slot, d, *s.out);
+	d.dxy_global = s.want_global ? (double*)(t + ob * 11) : nullptr;
+	return d;
+}
+// rows [row0, row0 + n) of the caller's arrays <- rows [0, n) of a device table, on `st`
+static int copy_back(const Scan& s, const pgt_windows& d, uint64_t row0, uint64_t n) {
+	cudaError_t e = cudaSuccess;
+	auto back = [&](auto* h, auto* dp) {
+		if (e == cudaSuccess && h && dp && n) e = cudaMemcpyAsync(h + row0, dp, n * sizeof(*h), cudaMemcpyDeviceToHost, s.st);
+	};
+	for_each_value(back, *s.out, d);
+	if (e != cudaSuccess) return cuda_fail(e, "cudaMemcpyAsync(window table -> host)");
+	return PGT_OK;
+}
+
+// Windows straight from the sites (sliding tile / W = S = 1): slabs of consecutive WINDOWS; a slab holds the sites of
+// its windows, neighbours share the W - S sites of the overlap.  The global line is taken from the same staged sites:
+// every slab folds the part of the owned range [gsite_lo, gsite_hi) that no earlier slab has folded, one partial
+// triple per slab, added in slab order on the host.
+template <class Stat>
+static int host_window_slabs(const Scan& s, HostStaging& hs) {
+	const pgt_plan* plan = s.plan;
+	const Layout& L = s.L;
+	const uint64_t slab_target = L.slab_sites - kSlabSlack;
+	double* gslab = (double*)(s.ws + L.gslab_off);
+	uint64_t ngslab = 0, gcursor = L.gsite_lo;
+	auto fold_global = [&](const Cols& C, uint64_t s0, uint64_t s1) -> int {  // owned sites inside the staged [s0, s1)
+		const uint64_t a = std::max(gcursor, s0), b = std::min(L.gsite_hi, s1);
+		if (!s.want_global || b <= a) return PGT_OK;
+		if (ngslab >= L.gslab_cap) return pgt_set_error(PGT_ERR_NOMEM, "internal: global-line slab table too small");
+		PGT_TRY(launch_global_sites(C, a - s0, b - s0, (double*)(s.ws + L.gpart_off), gslab + 3 * ngslab, s.st));
+		++ngslab;
+		gcursor = b;
+		return PGT_OK;
+	};
+	uint64_t w = L.w_lo;
+	while (w < L.w_hi) {
+		uint64_t fs, last;
+		pgt_plan_window(plan, w, &fs, nullptr, nullptr);
+		const uint64_t wb = pgt_plan_windows_within(plan, w, std::min<uint64_t>(L.w_hi, w + L.out_slab_rows), fs + slab_target);
+		pgt_plan_window(plan, wb - 1, nullptr, &last, nullptr);
+		// (in site mode no owned site precedes the scan's first window: only an EOF segment can lack windows)
+		const uint64_t s0 = fs;
+		const uint64_t ns = last + 1 - s0;
+		if (ns > L.slab_sites) return pgt_set_error(PGT_ERR_ARGS, "internal: window slab larger than the staging buffers");
+		Cols C;
+		PGT_TRY(hs.stage(s, s0, ns, &C));
+		DevPlan Ps = s.P;
+		Ps.win_lo = w;
+		Ps.win_hi = wb;
+		Ps.site_origin = s0;
+		Ps.col_elems = ns;
+		const pgt_windows o = device_table(s, hs.slot);  // rewritten two slabs later, after this slab's copy-back (order of `st`)
+		// (global line: fold_global below)
+		if (L.path == PGT_PATH_PERSITE) PGT_TRY(launch_persite<Stat>(plan, Ps, C, o, nullptr, nullptr, s.st));
+		else PGT_TRY(launch_slide<Stat>(plan, L.slide, Ps, C, ns, nullptr, o, nullptr, nullptr, s.st));
+		PGT_TRY(fold_global(C, s0, s0 + ns));
+		PGT_TRY(copy_back(s, o, w - L.w_lo, wb - w));
+		PGT_TRY(hs.release(s.st));
+		w = wb;
+	}
+	// owned sites after the last window (dropped EOF partial) or of a scan without windows
+	while (s.want_global && gcursor < L.gsite_hi) {
+		const uint64_t ns = std::min<uint64_t>(L.gsite_hi - gcursor, slab_target);
+		const uint64_t s0 = gcursor;
+		Cols C;
+		PGT_TRY(hs.stage(s, s0, ns, &C));
+		PGT_TRY(fold_global(C, s0, s0 + ns));
+		PGT_TRY(hs.release(s.st));
+	}
+	if (s.want_global) {
+		std::vector<double> part(3 * ngslab + 3, 0.0);
+		if (ngslab) PGT_CUDA(cudaMemcpyAsync(part.data(), gslab, 3 * ngslab * sizeof(double), cudaMemcpyDeviceToHost, s.st));
+		PGT_CUDA(cudaStreamSynchronize(s.st));
+		double g3[3] = {0.0, 0.0, 0.0};
+		for (uint64_t i = 0; i < ngslab; ++i)
+			for (int q = 0; q < 3; ++q) g3[q] += part[3 * i + q];
+		memcpy(s.out->dxy_global, g3, sizeof(g3));
+	}
+	return PGT_OK;
+}
+
+// Level 1 over slabs of consecutive UNITS into the unit array on the device.
+template <class Stat>
+static int host_unit_slabs(const Scan& s, HostStaging& hs, typename Stat::Acc* units) {
+	const pgt_plan* plan = s.plan;
+	const Layout& L = s.L;
+	const uint64_t slab_target = L.slab_sites - kSlabSlack;
+	const uint64_t axis_end = plan->off[0] + plan->nsites;
+	uint64_t ua = L.u_lo;
+	while (ua < L.u_hi) {
+		const uint64_t e0 = pgt_plan_unit_start(plan, ua);
+		uint64_t ub;
+		if (e0 + slab_target >= axis_end) ub = L.u_hi;
+		else ub = std::min<uint64_t>(L.u_hi, pgt_plan_unit_containing(plan, e0 + slab_target));
+		if (ub <= ua) ub = ua + 1;
+		const uint64_t e1 = pgt_plan_unit_start(plan, ub);
+		uint64_t s0 = e0, s1 = e1;  // data-site range of this slab
+		if (s.bp) {
+			s0 = host_site_lower_bound(plan, s.site_offsets, s.C.pos, L.origin, s.ndata, e0);
+			s1 = host_site_lower_bound(plan, s.site_offsets, s.C.pos, L.origin, s.ndata, e1);
+		}
+		const uint64_t ns = s1 - s0;
+		if (ns > L.slab_sites) return pgt_set_error(PGT_ERR_INPUT, "bp mode: more sites than bp in a slab (positions not strictly increasing?)");
+		Cols C;
+		PGT_TRY(hs.stage(s, s0, ns, &C));
+		DevPlan Ps = s.P;
+		Ps.unit_lo = ua;
+		Ps.unit_hi = ub;
+		Ps.site_origin = s0;
+		Ps.col_elems = ns;
+		uint64_t* sb = s.bounds ? s.bounds + (ua - L.u_lo) : nullptr;
+		// bp: bounds are relative to the staged slice.  Slab i writes entries [ua, ub]; the shared
+		// entry ub is rewritten by slab i+1 relative to ITS slice, after slab i's unit kernel
+		// (stream order on `st`).
+		if (s.bp) PGT_TRY(launch_bounds_kernel(Ps, C.pos, ns, sb, s.st));
+		PGT_TRY(launch_units<Stat>(Ps, C, units + (ua - L.u_lo), sb, ns, L.tileseg_cap ? (uint32_t*)(s.ws + L.tileseg_off) : nullptr,
+		                           L.tileseg_cap, s.st));
+		PGT_TRY(hs.release(s.st));
+		ua = ub;
+	}
+	return PGT_OK;
+}
+
+template <class Stat>
+static int scan_host(const Scan& s) {
+	const Layout& L = s.L;
+	HostStaging hs;
+	PGT_CUDA(cudaStreamCreateWithFlags(&hs.copy, cudaStreamNonBlocking));
+	for (int i = 0; i < 2; ++i) {
+		PGT_CUDA(cudaEventCreateWithFlags(&hs.ready[i], cudaEventDisableTiming));
+		PGT_CUDA(cudaEventCreateWithFlags(&hs.freed[i], cudaEventDisableTiming));
+	}
+	// the copy stream must not start before the caller's stream reaches this point
+	PGT_CUDA(cudaEventRecord(hs.freed[0], s.st));
+	PGT_CUDA(cudaStreamWaitEvent(hs.copy, hs.freed[0], 0));
+	Bookkeeper book;
+	start_bookkeeping(s, &book);
+	hs.ncol = stat_columns(s.stat, s.plan->mode, hs.cd);
+	size_t o = L.stage_off;
+	for (int k = 0; k < 2; ++k)
+		for (int i = 0; i < hs.ncol; ++i) {
+			hs.buf[k][i] = s.ws + o;
+			o += L.stage_col_bytes[i];
+		}
+	if (L.path != PGT_PATH_UNITS) {
+		PGT_TRY(host_window_slabs<Stat>(s, hs));
+	} else {
+		typename Stat::Acc* units = (typename Stat::Acc*)(s.ws + L.units_off);
+		PGT_TRY(host_unit_slabs<Stat>(s, hs, units));
+		const pgt_windows dev = device_table(s, 0);
+		if (s.want_global) PGT_TRY(launch_global<Stat>(units, s.nglobal, (double*)(s.ws + L.gpart_off), dev.dxy_global, s.st));
+		PGT_TRY(launch_windows<Stat>(s.P, units, L.u_lo, nullptr, dev, L.hgw, (typename Stat::Acc*)(s.ws + L.pre_off), L.blk_lo, L.blk_hi, s.st));
+		PGT_TRY(copy_back(s, dev, 0, L.w_hi - L.w_lo));
+		if (s.want_global) PGT_CUDA(cudaMemcpyAsync(s.out->dxy_global, dev.dxy_global, 3 * sizeof(double), cudaMemcpyDeviceToHost, s.st));
+	}
+	book.join();
+	PGT_CUDA(cudaStreamSynchronize(s.st));
+	PGT_CUDA(cudaStreamSynchronize(hs.copy));
+	return PGT_OK;
+}
 
 template <class Stat>
 static int run_scan(const pgt_plan* plan, const pgt_range* range, pgt_stat stat, const pgt_columns* cols, int minind,
@@ -997,7 +1253,8 @@ static int run_scan(const pgt_plan* plan, const pgt_range* range, pgt_stat stat,
 	int ndev = 0;
 	if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0)
 		return pgt_set_error(PGT_ERR_CUDA, "no usable CUDA device (libpgtscan has no CPU fallback)");
-	Layout L;
+	Scan s;
+	Layout& L = s.L;
 	PGT_TRY(make_layout(plan, range, stat, mem, &L));
 	if (!workspace) return pgt_set_error(PGT_ERR_ARGS, "workspace is NULL");
 	if (workspace_bytes < L.total) return pgt_set_error(PGT_ERR_NOMEM, "workspace too small, see pgt_scan_workspace_bytes");
@@ -1005,12 +1262,12 @@ static int run_scan(const pgt_plan* plan, const pgt_range* range, pgt_stat stat,
 	if (bp && stat != PGT_STAT_DXY) return pgt_set_error(PGT_ERR_ARGS, "PGT_MODE_BP plans are for PGT_STAT_DXY only");
 	if (bp && (!site_offsets || !cols->pos)) return pgt_set_error(PGT_ERR_ARGS, "bp mode needs site_offsets and pos");
 	const uint64_t nunits = L.u_hi - L.u_lo;
-	const uint64_t nwin = L.w_hi - L.w_lo;
-	if (nunits == 0 && nwin == 0) return PGT_OK;  // empty input / empty shard: nothing to read or write
+	if (nunits == 0 && L.w_hi == L.w_lo) return PGT_OK;  // empty input / empty shard: nothing to read or write
+	const Cols C = cols_from(*cols, minind);
 	ColDesc cd[8];
-	const int ncol = stat_columns(stat, plan->mode, cols, cd);
+	const int ncol = stat_columns(stat, plan->mode, cd);
 	for (int i = 0; i < ncol; ++i)
-		if (!cd[i].ptr) return pgt_set_error(PGT_ERR_ARGS, "a column required by this statistic is NULL");
+		if (!col_ptr(C, cd[i])) return pgt_set_error(PGT_ERR_ARGS, "a column required by this statistic is NULL");
 	if (!bp && nunits > 0 && pgt_plan_unit_start(plan, L.u_lo) < L.origin)
 		return pgt_set_error(PGT_ERR_ARGS, "site_origin lies after the first site this scan must read");
 
@@ -1024,7 +1281,7 @@ static int run_scan(const pgt_plan* plan, const pgt_range* range, pgt_stat stat,
 	}
 	if (bp) PGT_CUDA(cudaMemcpyAsync(ws + L.siteoff_off, site_offsets, off_bytes, cudaMemcpyHostToDevice, st));
 
-	DevPlan P;
+	DevPlan& P = s.P;
 	P.g = plan->g;
 	P.segs = resident ? (const pgt_seg*)plan->d_tables : (const pgt_seg*)(ws + L.segs_off);
 	P.off = resident ? (const uint64_t*)(plan->d_tables + align_up(seg_bytes, 256)) : (const uint64_t*)(ws + L.off_off);
@@ -1040,324 +1297,23 @@ static int run_scan(const pgt_plan* plan, const pgt_range* range, pgt_stat stat,
 	P.col_elems = ~0ull;
 	P.mode = (int)plan->mode;
 
-	typename Stat::Acc* units = (typename Stat::Acc*)(ws + L.units_off);
-	uint64_t* bounds = (bp || L.unit_table) ? (uint64_t*)(ws + L.bounds_off) : nullptr;
-	uint64_t ndata = 0;  // bp mode: sites the columns hold
+	s.ndata = 0;
 	if (bp) {
 		if (site_offsets[P.ncontig] < L.origin) return pgt_set_error(PGT_ERR_ARGS, "site_origin beyond the last site");
-		ndata = (range && range->site_count) ? range->site_count : site_offsets[P.ncontig] - L.origin;
+		s.ndata = (range && range->site_count) ? range->site_count : site_offsets[P.ncontig] - L.origin;
 	}
-	const bool want_global = out->dxy_global && (stat == PGT_STAT_DXY || stat == PGT_STAT_FUSED);
-	const uint64_t nglobal = L.g_hi > L.u_lo ? L.g_hi - L.u_lo : 0;
-
-	if (mem == PGT_MEM_DEVICE) {
-		Cols C;
-		memset(&C, 0, sizeof(C));
-		C.pos = cols->pos;
-		C.a = cols->a;
-		C.b = cols->b;
-		C.g = cols->geno;
-		C.f1 = cols->f1;
-		C.f2 = cols->f2;
-		C.n1 = cols->n1;
-		C.n2 = cols->n2;
-		C.minind = minind;
-		if (L.persite || L.slide) {
-			// windows straight from the sites: W = S = 1 (default arguments of fstWindow / hetWindow: an
-			// elementwise map) or the sliding tile for fine steps; no unit array, no level 2
-			if (nwin) {
-				uint64_t last_site;
-				pgt_plan_window(plan, L.w_hi - 1, nullptr, &last_site, nullptr);
-				P.col_elems = last_site + 1 - L.origin;
-			}
-			bool global_done = false;
-			if (nwin && L.persite) {
-				// the windows ARE the sites: when the owned range of the global line is exactly their span (always, unless the
-				// scan owns sites outside any window) the kernel adds its sites up on the way and the dxy columns are read once
-				uint64_t first_site, last_site;
-				pgt_plan_window(plan, L.w_lo, &first_site, nullptr, nullptr);
-				pgt_plan_window(plan, L.w_hi - 1, nullptr, &last_site, nullptr);
-				global_done = want_global && GlobalTerm<Stat>::has && L.gsite_lo == first_site && L.gsite_hi == last_site + 1;
-				PGT_TRY(launch_persite<Stat>(plan, stat, P, C, *out, global_done ? (double*)(ws + L.gpart_off) : nullptr, out->dxy_global, st));
-			} else if (nwin) {
-				uint64_t last;
-				pgt_plan_window(plan, L.w_hi - 1, nullptr, &last, nullptr);
-				global_done = want_global && GlobalTerm<Stat>::has && g_tune_slideglobal != 1 && slide_runs_cover_owned_sites(plan, L);
-				PGT_TRY(launch_slide<Stat>(plan, stat, P, C, last + 1 - L.origin, cols->pos, *out,
-				                           global_done ? (double*)(ws + L.gpart_off) : nullptr, out->dxy_global, st));
-			}
-			if (want_global && !global_done) {
-				if (L.gsite_lo < L.origin) return pgt_set_error(PGT_ERR_ARGS, "site_origin lies after the first site this scan must read");
-				PGT_TRY(launch_global_sites(C, L.gsite_lo - L.origin, L.gsite_hi - L.origin, (double*)(ws + L.gpart_off), out->dxy_global, st));
-			}
-			return PGT_OK;
-		}
-		if (bp && nunits) PGT_TRY(launch_bounds_kernel(P, cols->pos, ndata, bounds, st));
-		if (L.unit_table) {  // very many segments: unit starts once, then the INDIRECT level-1 kernels
-			const uint64_t want = (nunits + 256) / 256, cap = (uint64_t)num_sms() * 8;
-			k_unit_starts<<<(unsigned)(want < cap ? want : cap), 256, 0, st>>>(P, bounds);
-			g_launches++;
-			PGT_CUDA(cudaGetLastError());
-		}
-		// elements the caller's columns are known to hold: up to the end of the last unit read
-		const uint64_t valid = bp ? ndata : pgt_plan_unit_start(plan, L.u_hi) - L.origin;
-		P.col_elems = valid;
-		PGT_TRY(launch_units<Stat>(P, C, units, bounds, valid, L.tileseg_cap ? (uint32_t*)(ws + L.tileseg_off) : nullptr, L.tileseg_cap, st));
-		// the global line reads the raw unit partials: before level 2, which may scan them in place
-		if (want_global) PGT_TRY(launch_global<Stat>(units, nglobal, (double*)(ws + L.gpart_off), out->dxy_global, st));
-		PGT_TRY(launch_windows<Stat>(P, units, L.u_lo, cols->pos, *out, L.hgw, (typename Stat::Acc*)(ws + L.pre_off), L.blk_lo, L.blk_hi, st));
-		return PGT_OK;
-	}
-
-	// ---- PGT_MEM_HOST: slabs of the axis are staged H2D on a copy stream (double-buffered) while
-	// the previous slab is reduced; only unit partials stay on the device.  Positions are not
-	// copied in site mode: the two edge positions per window are gathered on the host.
-	HostStreams hs;
-	PGT_CUDA(cudaStreamCreateWithFlags(&hs.copy, cudaStreamNonBlocking));
-	for (int i = 0; i < 2; ++i) {
-		PGT_CUDA(cudaEventCreateWithFlags(&hs.ready[i], cudaEventDisableTiming));
-		PGT_CUDA(cudaEventCreateWithFlags(&hs.freed[i], cudaEventDisableTiming));
-	}
-	// the copy stream must not start before the caller's stream reaches this point
-	PGT_CUDA(cudaEventRecord(hs.freed[0], st));
-	PGT_CUDA(cudaStreamWaitEvent(hs.copy, hs.freed[0], 0));
-	// Window bookkeeping on the host -- label, nsites, the two edge positions per window -- runs on
-	// worker threads from here on, next to the copy pipeline.  (It cannot simply follow the slab
-	// loop: enqueueing ~10 operations per slab blocks once the driver's queue is full, so the host
-	// would only get to it when most of the transfer is over; 3e7 windows take ~1 s on one thread.)
-	struct Bookkeeper {
-		std::vector<std::thread> th;
-		void join() {
-			for (auto& t : th)
-				if (t.joinable()) t.join();
-		}
-		~Bookkeeper() { join(); }
-	} book;
-	if (nwin && (out->label || out->nsites || out->start_pos || out->end_pos || out->mid_pos)) {
-		unsigned nt = nwin < (1u << 16) ? 1u : std::min<unsigned>(8u, std::max(1u, std::thread::hardware_concurrency()));
-		const uint64_t per = (nwin + nt - 1) / nt;
-		const uint64_t origin = L.origin;
-		for (unsigned t = 0; t < nt; ++t) {
-			const uint64_t wa = L.w_lo + per * t, wb = std::min<uint64_t>(L.w_hi, wa + per);
-			if (wa >= wb) break;
-			book.th.emplace_back([plan, out, cols, bp, wa, wb, origin, w_lo = L.w_lo]() {
-				uint32_t si = pgt_plan_seg_of_window(plan, wa);
-				for (uint64_t w = wa; w < wb; ++w) {
-					while (w >= plan->segs[si].win_base + plan->segs[si].nwin) ++si;
-					const pgt_seg& sg = plan->segs[si];
-					uint64_t fs;
-					const uint32_t n = pgt_window_sites(plan->g, sg, w - sg.win_base, &fs);
-					const uint64_t first = sg.site_base + fs, last = first + n - 1;
-					const uint32_t label = pgt_plan_contig_of(plan, last);
-					const uint64_t o = w - w_lo;
-					if (out->label) out->label[o] = label;
-					if (out->nsites) out->nsites[o] = n;
-					uint32_t sp = 0, ep = 0;
-					bool have = false;
-					if (bp) {
-						sp = (uint32_t)(first - plan->off[pgt_plan_contig_of(plan, first)]) + 1u;
-						ep = (uint32_t)(last - plan->off[label]) + 1u;
-						have = true;
-					} else if (cols->pos) {
-						sp = cols->pos[first - origin];
-						ep = cols->pos[last - origin];
-						have = true;
-					}
-					if (have) {
-						if (out->start_pos) out->start_pos[o] = sp;
-						if (out->end_pos) out->end_pos[o] = ep;
-						if (out->mid_pos) out->mid_pos[o] = (sp + ep) / 2u;
-					}
-				}
-			});
-		}
-	}
-	char* stage[2][8];
-	{
-		size_t o = L.stage_off;
-		for (int s = 0; s < 2; ++s)
-			for (int i = 0; i < ncol; ++i) {
-				stage[s][i] = ws + o;
-				o += L.stage_col_bytes[i];
-			}
-	}
-	// per-window values are produced into device staging, then copied back: one table for the whole scan, or --
-	// when the windows come straight from the sites, slab by slab -- two slab-sized tables used in turn
-	const bool from_units = !(L.slide || L.persite);
-	const uint64_t out_rows = from_units ? nwin : L.out_slab_rows;
-	const size_t ob = align_up((size_t)out_rows * 8 + 8, 256);
-	auto device_table = [&](int which) -> pgt_windows {
-		pgt_windows d;
-		memset(&d, 0, sizeof(d));
-		char* ob0 = ws + L.outs_off + (size_t)which * 12 * ob;
-		int k = 0;
-		auto dptr = [&](const void* want) -> void* {
-			void* r = want ? (void*)(ob0 + ob * k) : nullptr;
-			++k;
-			return r;
-		};
-		d.sum_a = (double*)dptr(out->sum_a);
-		d.sum_b = (double*)dptr(out->sum_b);
-		d.fst = (double*)dptr(out->fst);
-		d.nhet = (uint32_t*)dptr(out->nhet);
-		d.nonmissing = (uint32_t*)dptr(out->nonmissing);
-		d.het = (double*)dptr(out->het);
-		d.dxy = (double*)dptr(out->dxy);
-		d.neffective = (uint32_t*)dptr(out->neffective);
-		d.nskip = (uint32_t*)dptr(out->nskip);
-		d.dxy_global = want_global ? (double*)(ob0 + ob * 11) : nullptr;
-		return d;
-	};
-	// rows [row0, row0 + n) of the caller's arrays <- rows [0, n) of a device table, on `st`
-	auto copy_back = [&](const pgt_windows& d, uint64_t row0, uint64_t n) -> int {
-		auto back = [&](void* h, const void* dp, size_t elem) -> cudaError_t {
-			return (h && dp && n) ? cudaMemcpyAsync((char*)h + row0 * elem, dp, n * elem, cudaMemcpyDeviceToHost, st) : cudaSuccess;
-		};
-		PGT_CUDA(back(out->sum_a, d.sum_a, 8));
-		PGT_CUDA(back(out->sum_b, d.sum_b, 8));
-		PGT_CUDA(back(out->fst, d.fst, 8));
-		PGT_CUDA(back(out->nhet, d.nhet, 4));
-		PGT_CUDA(back(out->nonmissing, d.nonmissing, 4));
-		PGT_CUDA(back(out->het, d.het, 8));
-		PGT_CUDA(back(out->dxy, d.dxy, 8));
-		PGT_CUDA(back(out->neffective, d.neffective, 4));
-		PGT_CUDA(back(out->nskip, d.nskip, 4));
-		return PGT_OK;
-	};
-	const pgt_windows dev = device_table(0);
-	const uint64_t slab_target = L.slab_sites - kSlabSlack;
-	const uint64_t axis_end = plan->off[0] + plan->nsites;
-	int slot = 0;
-	bool slot_used[2] = {false, false};
-	// one slab: H2D of sites [s0, s0 + ns) of every column into `slot`, ordered after the kernels that last read it
-	auto stage_slab = [&](uint64_t s0, uint64_t ns, Cols* C) -> int {
-		if (slot_used[slot]) PGT_CUDA(cudaStreamWaitEvent(hs.copy, hs.freed[slot], 0));
-		memset(C, 0, sizeof(*C));
-		C->minind = minind;
-		for (int i = 0; i < ncol; ++i) {
-			const char* src = (const char*)cd[i].ptr + (s0 - L.origin) * cd[i].elem;
-			if (ns) PGT_CUDA(cudaMemcpyAsync(stage[slot][i], src, ns * cd[i].elem, cudaMemcpyHostToDevice, hs.copy));
-			const void* p = stage[slot][i];
-			memcpy((char*)C + cd[i].offset_in_cols, &p, sizeof(p));
-		}
-		PGT_CUDA(cudaEventRecord(hs.ready[slot], hs.copy));
-		PGT_CUDA(cudaStreamWaitEvent(st, hs.ready[slot], 0));
-		return PGT_OK;
-	};
-	auto release_slab = [&]() -> int {
-		PGT_CUDA(cudaEventRecord(hs.freed[slot], st));
-		slot_used[slot] = true;
-		slot ^= 1;
-		return PGT_OK;
-	};
-	if (L.slide || L.persite) {
-		// ---- windows straight from the sites (sliding tile / W = S = 1): slabs of consecutive WINDOWS; a
-		// slab holds the sites of its windows, neighbours share the W - S sites of the overlap.  The global
-		// line is taken from the same staged sites: every slab folds the part of the owned range
-		// [gsite_lo, gsite_hi) that no earlier slab has folded, one partial triple per slab, added in slab
-		// order on the host.
-		double* gslab = (double*)(ws + L.gslab_off);
-		uint64_t ngslab = 0, gcursor = L.gsite_lo;
-		auto fold_global = [&](const Cols& C, uint64_t s0, uint64_t s1) -> int {  // owned sites inside the staged [s0, s1)
-			const uint64_t a = std::max(gcursor, s0), b = std::min(L.gsite_hi, s1);
-			if (!want_global || b <= a) return PGT_OK;
-			if (ngslab >= L.gslab_cap) return pgt_set_error(PGT_ERR_NOMEM, "internal: global-line slab table too small");
-			PGT_TRY(launch_global_sites(C, a - s0, b - s0, (double*)(ws + L.gpart_off), gslab + 3 * ngslab, st));
-			++ngslab;
-			gcursor = b;
-			return PGT_OK;
-		};
-		uint64_t w = L.w_lo;
-		while (w < L.w_hi) {
-			uint64_t fs, last;
-			pgt_plan_window(plan, w, &fs, nullptr, nullptr);
-			const uint64_t wb = pgt_plan_windows_within(plan, w, std::min<uint64_t>(L.w_hi, w + L.out_slab_rows), fs + slab_target);
-			pgt_plan_window(plan, wb - 1, nullptr, &last, nullptr);
-			// (in site mode no owned site precedes the scan's first window: only an EOF segment can lack windows)
-			const uint64_t s0 = fs;
-			const uint64_t ns = last + 1 - s0;
-			if (ns > L.slab_sites) return pgt_set_error(PGT_ERR_ARGS, "internal: window slab larger than the staging buffers");
-			Cols C;
-			PGT_TRY(stage_slab(s0, ns, &C));
-			DevPlan Ps = P;
-			Ps.win_lo = w;
-			Ps.win_hi = wb;
-			Ps.site_origin = s0;
-			Ps.col_elems = ns;
-			const pgt_windows o = device_table(slot);  // rewritten two slabs later, after this slab's copy-back (order of `st`)
-			if (L.persite) {
-				PGT_TRY(launch_persite<Stat>(plan, stat, Ps, C, o, nullptr, nullptr, st));  // (global line: fold_global below)
-			} else {
-				PGT_TRY(launch_slide<Stat>(plan, stat, Ps, C, ns, nullptr, o, nullptr, nullptr, st));  // (global line: fold_global below)
-			}
-			PGT_TRY(fold_global(C, s0, s0 + ns));
-			PGT_TRY(copy_back(o, w - L.w_lo, wb - w));
-			PGT_TRY(release_slab());
-			w = wb;
-		}
-		// owned sites after the last window (dropped EOF partial) or of a scan without windows
-		while (want_global && gcursor < L.gsite_hi) {
-			const uint64_t ns = std::min<uint64_t>(L.gsite_hi - gcursor, slab_target);
-			const uint64_t s0 = gcursor;
-			Cols C;
-			PGT_TRY(stage_slab(s0, ns, &C));
-			PGT_TRY(fold_global(C, s0, s0 + ns));
-			PGT_TRY(release_slab());
-		}
-		if (want_global) {
-			std::vector<double> part(3 * ngslab + 3, 0.0);
-			if (ngslab) PGT_CUDA(cudaMemcpyAsync(part.data(), gslab, 3 * ngslab * sizeof(double), cudaMemcpyDeviceToHost, st));
-			PGT_CUDA(cudaStreamSynchronize(st));
-			double g3[3] = {0.0, 0.0, 0.0};
-			for (uint64_t i = 0; i < ngslab; ++i)
-				for (int q = 0; q < 3; ++q) g3[q] += part[3 * i + q];
-			memcpy(out->dxy_global, g3, sizeof(g3));
-		}
-	}
-	uint64_t ua = (L.slide || L.persite) ? L.u_hi : L.u_lo;
-	while (ua < L.u_hi) {
-		const uint64_t e0 = pgt_plan_unit_start(plan, ua);
-		uint64_t ub;
-		if (e0 + slab_target >= axis_end) ub = L.u_hi;
-		else ub = std::min<uint64_t>(L.u_hi, pgt_plan_unit_containing(plan, e0 + slab_target));
-		if (ub <= ua) ub = ua + 1;
-		const uint64_t e1 = pgt_plan_unit_start(plan, ub);
-		uint64_t s0 = e0, s1 = e1;  // data-site range of this slab
-		if (bp) {
-			s0 = host_site_lower_bound(plan, site_offsets, cols->pos, L.origin, ndata, e0);
-			s1 = host_site_lower_bound(plan, site_offsets, cols->pos, L.origin, ndata, e1);
-		}
-		const uint64_t ns = s1 - s0;
-		if (ns > L.slab_sites) return pgt_set_error(PGT_ERR_INPUT, "bp mode: more sites than bp in a slab (positions not strictly increasing?)");
-		Cols C;
-		PGT_TRY(stage_slab(s0, ns, &C));
-		DevPlan Ps = P;
-		Ps.unit_lo = ua;
-		Ps.unit_hi = ub;
-		Ps.site_origin = s0;
-		Ps.col_elems = ns;
-		uint64_t* sb = bounds ? bounds + (ua - L.u_lo) : nullptr;
-		// bp: bounds are relative to the staged slice.  Slab i writes entries [ua, ub]; the shared
-		// entry ub is rewritten by slab i+1 relative to ITS slice, after slab i's unit kernel
-		// (stream order on `st`).
-		if (bp) PGT_TRY(launch_bounds_kernel(Ps, C.pos, ns, sb, st));
-		PGT_TRY(launch_units<Stat>(Ps, C, units + (ua - L.u_lo), sb, ns, L.tileseg_cap ? (uint32_t*)(ws + L.tileseg_off) : nullptr,
-		                           L.tileseg_cap, st));
-		PGT_TRY(release_slab());
-		ua = ub;
-	}
-
-	if (from_units) {
-		if (want_global) PGT_TRY(launch_global<Stat>(units, nglobal, (double*)(ws + L.gpart_off), dev.dxy_global, st));
-		PGT_TRY(launch_windows<Stat>(P, units, L.u_lo, nullptr, dev, L.hgw, (typename Stat::Acc*)(ws + L.pre_off), L.blk_lo, L.blk_hi, st));
-		PGT_TRY(copy_back(dev, 0, nwin));
-		if (want_global) PGT_CUDA(cudaMemcpyAsync(out->dxy_global, dev.dxy_global, 3 * sizeof(double), cudaMemcpyDeviceToHost, st));
-	}
-
-	book.join();
-	PGT_CUDA(cudaStreamSynchronize(st));
-	PGT_CUDA(cudaStreamSynchronize(hs.copy));
-	return PGT_OK;
+	s.plan = plan;
+	s.stat = stat;
+	s.C = C;
+	s.site_offsets = site_offsets;
+	s.out = out;
+	s.ws = ws;
+	s.bounds = (bp || L.unit_table) ? (uint64_t*)(ws + L.bounds_off) : nullptr;
+	s.nglobal = L.g_hi > L.u_lo ? L.g_hi - L.u_lo : 0;
+	s.bp = bp;
+	s.want_global = out->dxy_global && (stat == PGT_STAT_DXY || stat == PGT_STAT_FUSED);
+	s.st = st;
+	return mem == PGT_MEM_DEVICE ? scan_device<Stat>(s) : scan_host<Stat>(s);
 }
 
 extern "C" int pgt_scan(const pgt_plan* plan, const pgt_range* range, pgt_stat stat, const pgt_columns* cols, int minind,

@@ -16,7 +16,6 @@
 #include <thread>
 #include <vector>
 
-#include "../../include/pgt_extreme.h"
 #include "pgt_internal.h"
 
 namespace {
@@ -35,23 +34,7 @@ struct ShardJob {
 
 pgt_windows rows_from(const pgt_windows& o, uint64_t d) {
 	pgt_windows r = o;
-	auto adv = [d](auto*& p) {
-		if (p) p += d;
-	};
-	adv(r.label);
-	adv(r.start_pos);
-	adv(r.end_pos);
-	adv(r.mid_pos);
-	adv(r.nsites);
-	adv(r.sum_a);
-	adv(r.sum_b);
-	adv(r.fst);
-	adv(r.nhet);
-	adv(r.nonmissing);
-	adv(r.het);
-	adv(r.dxy);
-	adv(r.neffective);
-	adv(r.nskip);
+	for_each_field([d](auto*& p) { p = p ? p + d : p; }, r);
 	return r;
 }
 
@@ -204,12 +187,7 @@ extern "C" int pgt_scan_extreme_sharded(const pgt_xplan* plan, pgt_xstat stat, d
 		}
 		pgt_xwindows rows = *out;
 		const uint64_t d = job->range.w_lo;
-		if (rows.ext_value) rows.ext_value += d;
-		if (rows.ext_pos) rows.ext_pos += d;
-		if (rows.ext_site) rows.ext_site += d;
-		if (rows.nbig) rows.nbig += d;
-		if (rows.nsites) rows.nsites += d;
-		if (rows.prop) rows.prop += d;
+		for_each_xfield([d](auto*& p) { p = p ? p + d : p; }, rows);
 		const uint64_t s0 = job->range.site_origin;
 		const int rc = pgt_scan_extreme(plan, &job->range, stat, cutoff, pos ? pos + s0 : nullptr, score + s0, &rows, ws, bytes, PGT_MEM_HOST, st);
 		if (rc != PGT_OK) {
