@@ -35,6 +35,7 @@
 #include <new>
 #include <string>
 #include <thread>
+#include <type_traits>
 #include <vector>
 
 #include "../../include/pgt_synth.h"
@@ -390,6 +391,16 @@ __device__ __forceinline__ void x_emit(uint64_t w, double val, uint64_t best, ui
 	if (out.prop) out.prop[w] = (double)nbig / (double)(uint32_t)n;  // ihsWindow.cpp:79: double / unsigned
 }
 
+// the reference's "NA NA NA 0" row of an empty window (ihsWindow.cpp:82)
+__device__ __forceinline__ void x_emit_empty(uint64_t w, const pgt_xwindows& out) {
+	if (out.ext_value) out.ext_value[w] = CUDART_NAN;
+	if (out.ext_pos) out.ext_pos[w] = 0u;
+	if (out.ext_site) out.ext_site[w] = ~0ull;
+	if (out.nbig) out.nbig[w] = 0u;
+	if (out.nsites) out.nsites[w] = 0u;
+	if (out.prop) out.prop[w] = CUDART_NAN;
+}
+
 // Level 2: thread per window.  Empty windows get the "NA" defaults, single-unit windows copy their
 // partial, windows of 2..32 units are combined by their thread, longer ones by the whole warp.
 template <int MODE>
@@ -404,13 +415,8 @@ __global__ void __launch_bounds__(256) k_xwindows(XDev P, const uint32_t* __rest
 		u0 = P.unit0[w] - P.unit_base;
 		nu = P.unit0[w + 1] - P.unit_base - u0;
 	}
-	if (valid && n == 0) {  // the reference's "NA NA NA 0" row (ihsWindow.cpp:82)
-		if (out.ext_value) out.ext_value[w] = CUDART_NAN;
-		if (out.ext_pos) out.ext_pos[w] = 0u;
-		if (out.ext_site) out.ext_site[w] = ~0ull;
-		if (out.nbig) out.nbig[w] = 0u;
-		if (out.nsites) out.nsites[w] = 0u;
-		if (out.prop) out.prop[w] = CUDART_NAN;
+	if (valid && n == 0) {
+		x_emit_empty(w, out);
 	} else if (valid && nu <= 32) {
 		const double v0 = part.val[u0];
 		XAcc a{x_key<MODE>(v0), v0, part.idx[u0], part.nbig[u0]};
@@ -508,13 +514,8 @@ __global__ void __launch_bounds__(256) k_xsmall(XDev P, uint64_t nbatches, const
 			for (uint64_t w = w_lo + threadIdx.x; w < w_hi; w += 256u) {
 				const uint64_t a = P.xoff[w], b = P.xoff[w + 1];
 				const uint32_t len = (uint32_t)(b - a);
-				if (len == 0) {  // the reference's "NA NA NA 0" row (ihsWindow.cpp:82)
-					if (out.ext_value) out.ext_value[w] = CUDART_NAN;
-					if (out.ext_pos) out.ext_pos[w] = 0u;
-					if (out.ext_site) out.ext_site[w] = ~0ull;
-					if (out.nbig) out.nbig[w] = 0u;
-					if (out.nsites) out.nsites[w] = 0u;
-					if (out.prop) out.prop[w] = CUDART_NAN;
+				if (len == 0) {
+					x_emit_empty(w, out);
 					continue;
 				}
 				const double* __restrict__ p = x_tile + (a - s_lo);
@@ -557,14 +558,10 @@ extern "C" int pgt_synth_score(uint64_t seed, uint64_t site0, uint64_t n, double
 
 namespace {
 
-size_t xalign(size_t x) { return (x + 255) / 256 * 256; }
-
 struct XLayout {
 	uint64_t w_lo = 0, w_hi = 0, nw = 0, site_lo = 0, site_hi = 0, nsite = 0, unit_lo = 0, nunit = 0;
 	bool resident = false;  // window tables are bound on the device (pgt_xplan_bind_device)
-	size_t off_xoff = 0, off_unit0 = 0, p_val = 0, p_idx = 0, p_nbig = 0, off_score = 0, total = 0;
-	// host mode staging of the outputs, one block per field
-	size_t o_value = 0, o_site = 0, o_nbig = 0, o_nsites = 0, o_prop = 0;
+	size_t off_xoff = 0, off_unit0 = 0, p_val = 0, p_idx = 0, p_nbig = 0, off_score = 0, off_outs = 0, total = 0;
 };
 
 int x_layout(const pgt_xplan* plan, const pgt_range* range, pgt_mem mem, XLayout* L) {
@@ -587,39 +584,26 @@ int x_layout(const pgt_xplan* plan, const pgt_range* range, pgt_mem mem, XLayout
 	size_t o = 0;
 	if (!L->resident) {
 		L->off_xoff = o;
-		o += xalign((L->nw + 1) * sizeof(uint64_t));
+		o += align_up((L->nw + 1) * sizeof(uint64_t), 256);
 		L->off_unit0 = o;
-		o += xalign((L->nw + 1) * sizeof(uint64_t));
+		o += align_up((L->nw + 1) * sizeof(uint64_t), 256);
 	}
 	L->p_val = o;
-	o += xalign(L->nunit * sizeof(double));
+	o += align_up(L->nunit * sizeof(double), 256);
 	L->p_idx = o;
-	o += xalign(L->nunit * sizeof(uint64_t));
+	o += align_up(L->nunit * sizeof(uint64_t), 256);
 	L->p_nbig = o;
-	o += xalign(L->nunit * sizeof(uint32_t));
+	o += align_up(L->nunit * sizeof(uint32_t), 256);
 	if (mem == PGT_MEM_HOST) {
 		L->off_score = o;
-		o += xalign(L->nsite * sizeof(double));
-		L->o_value = o;
-		o += xalign(L->nw * sizeof(double));
-		L->o_site = o;
-		o += xalign(L->nw * sizeof(uint64_t));
-		L->o_prop = o;
-		o += xalign(L->nw * sizeof(double));
-		L->o_nbig = o;
-		o += xalign(L->nw * sizeof(uint32_t));
-		L->o_nsites = o;
-		o += xalign(L->nw * sizeof(uint32_t));
+		o += align_up(L->nsite * sizeof(double), 256);
+		// staged outputs: one block per field in for_each_xfield order, none for ext_pos (gathered on the host)
+		L->off_outs = o;
+		pgt_xwindows t{};
+		for_each_xfield([&](auto*& p) { o += (void*)&p == (void*)&t.ext_pos ? 0 : align_up(L->nw * sizeof(*p), 256); }, t);
 	}
 	L->total = o + 256;
 	return PGT_OK;
-}
-
-int x_num_sms() {
-	int dev = 0, n = 0;
-	if (cudaGetDevice(&dev) != cudaSuccess) return 148;
-	cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev);
-	return n > 0 ? n : 148;
 }
 
 template <int MODE, int G>
@@ -628,7 +612,7 @@ void x_launch_units(const XDev& P, uint64_t nsite, const double* score, const XP
 	// one wave of resident CTAs (grid = multiple of the SM count)
 	int per_sm = 0;
 	if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_xunits<MODE, G>, 256, 0) != cudaSuccess || per_sm < 1) per_sm = 4;
-	const uint64_t max_groups = (uint64_t)x_num_sms() * (uint64_t)per_sm * 256ull / G;
+	const uint64_t max_groups = (uint64_t)num_sms() * (uint64_t)per_sm * 256ull / G;
 	uint64_t chunk = (nsite + max_groups - 1) / max_groups;
 	const uint64_t min_chunk = 64ull * G;
 	if (chunk < min_chunk) chunk = min_chunk;
@@ -647,14 +631,11 @@ int x_run(const XDev& P, uint64_t nsite, uint64_t nunit, const double* score, co
 		const uint64_t nbatches = (P.site_hi - P.site_lo) / kXTileStep + 1;
 		const size_t smem = (size_t)kXTileSites * sizeof(double);
 		PGT_CUDA(cudaFuncSetAttribute(k_xsmall<MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-		int per_sm = 0;
-		if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_xsmall<MODE>, 256, smem) != cudaSuccess || per_sm < 1) per_sm = 1;
-		const uint64_t cap = (uint64_t)x_num_sms() * per_sm;
 		ProfScope prof(2, st);
 		uint64_t* bw = part.idx;  // the partials are not used on this path: >= nw entries, and nw >= nbatches + 1 (checked by the caller)
 		k_xbatches<<<(unsigned)((nbatches + 256) / 256), 256, 0, st>>>(P, nbatches, bw);
 		pgt_count_launch();
-		k_xsmall<MODE><<<(unsigned)(nbatches < cap ? nbatches : cap), 256, smem, st>>>(P, nbatches, bw, score, pos, out);
+		k_xsmall<MODE><<<one_wave_grid(k_xsmall<MODE>, 256, nbatches, smem), 256, smem, st>>>(P, nbatches, bw, score, pos, out);
 		pgt_count_launch();
 		PGT_CUDA(cudaGetLastError());
 		return PGT_OK;
@@ -687,7 +668,7 @@ int x_run(const XDev& P, uint64_t nsite, uint64_t nunit, const double* score, co
 }  // namespace
 
 extern "C" size_t pgt_xplan_device_bytes(const pgt_xplan* plan) {
-	return plan ? 2 * xalign((plan->nwin + 1) * sizeof(uint64_t)) + 256 : 0;
+	return plan ? table_pair_bytes((plan->nwin + 1) * sizeof(uint64_t), (plan->nwin + 1) * sizeof(uint64_t)) : 0;
 }
 
 extern "C" int pgt_xplan_bind_device(pgt_xplan* plan, void* buffer, size_t bytes, void* stream) {
@@ -697,14 +678,8 @@ extern "C" int pgt_xplan_bind_device(pgt_xplan* plan, void* buffer, size_t bytes
 		return PGT_OK;
 	}
 	if (bytes < pgt_xplan_device_bytes(plan)) return pgt_set_error(PGT_ERR_NOMEM, "pgt_xplan_bind_device: buffer too small");
-	cudaStream_t st = (cudaStream_t)stream;
-	unsigned char* b = (unsigned char*)(((uintptr_t)buffer + 255) / 256 * 256);
 	const size_t tb = (plan->nwin + 1) * sizeof(uint64_t);
-	PGT_CUDA(cudaMemcpyAsync(b, plan->xoff.data(), tb, cudaMemcpyHostToDevice, st));
-	PGT_CUDA(cudaMemcpyAsync(b + xalign(tb), plan->unit0.data(), tb, cudaMemcpyHostToDevice, st));
-	PGT_CUDA(cudaStreamSynchronize(st));
-	plan->d_tables = b;
-	return PGT_OK;
+	return bind_table_pair(buffer, plan->xoff.data(), tb, plan->unit0.data(), tb, stream, &plan->d_tables);
 }
 
 extern "C" size_t pgt_scan_extreme_workspace_bytes(const pgt_xplan* plan, const pgt_range* range, pgt_mem mem) {
@@ -740,7 +715,7 @@ extern "C" int pgt_scan_extreme(const pgt_xplan* plan, const pgt_range* range, p
 	if (L.resident) {  // tables bound once with pgt_xplan_bind_device: nothing to upload
 		const uint64_t* t = (const uint64_t*)plan->d_tables;
 		P.xoff = t + L.w_lo;
-		P.unit0 = (const uint64_t*)(plan->d_tables + xalign((plan->nwin + 1) * sizeof(uint64_t))) + L.w_lo;
+		P.unit0 = (const uint64_t*)(plan->d_tables + align_up((plan->nwin + 1) * sizeof(uint64_t), 256)) + L.w_lo;
 	} else {
 		uint64_t* d_xoff = (uint64_t*)(ws + L.off_xoff);
 		uint64_t* d_unit0 = (uint64_t*)(ws + L.off_unit0);
@@ -775,11 +750,14 @@ extern "C" int pgt_scan_extreme(const pgt_xplan* plan, const pgt_range* range, p
 		d_score = stage;
 		d_pos = nullptr;
 		memset(&dout, 0, sizeof(dout));
-		if (out->ext_value) dout.ext_value = (double*)(ws + L.o_value);
-		if (out->ext_site || out->ext_pos) dout.ext_site = (uint64_t*)(ws + L.o_site);
-		if (out->prop) dout.prop = (double*)(ws + L.o_prop);
-		if (out->nbig) dout.nbig = (uint32_t*)(ws + L.o_nbig);
-		if (out->nsites) dout.nsites = (uint32_t*)(ws + L.o_nsites);
+		size_t o = L.off_outs;  // the blocks of x_layout; ext_site is staged for ext_pos too
+		for_each_xfield(
+		    [&](auto*& d, auto* h) {
+			    if ((void*)&d == (void*)&dout.ext_pos) return;
+			    if (h || ((void*)&d == (void*)&dout.ext_site && out->ext_pos)) d = (std::remove_reference_t<decltype(d)>)(ws + o);
+			    o += align_up(L.nw * sizeof(*d), 256);
+		    },
+		    dout, *out);
 	}
 	// short windows (a function of the plan only: longest window <= 2048 sites, fewer than 160 sites per unit on average)
 	// Measured (1e9 sites, profiles/r02z_extreme_small_windows.txt): 33 sites per window 2.79 ms against 3.32 ms for

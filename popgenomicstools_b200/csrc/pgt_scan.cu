@@ -183,30 +183,10 @@ static int g_tune_slide = 0;
 // 0: the sliding tile also takes dxyWindow's global line when its runs own exactly the line's sites; 1: always a separate pass
 static int g_tune_slideglobal = 0;
 
-static int num_sms() {
-	int dev = 0, n = 0;
-	if (cudaGetDevice(&dev) != cudaSuccess) return 0;
-	cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev);
-	return n;
-}
-
-static size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
-
 // Grid of a grid-stride kernel that wants `want` blocks: at most 8 per SM.
 static unsigned capped_grid(uint64_t want) {
 	const uint64_t cap = (uint64_t)num_sms() * 8;
 	return (unsigned)(want < cap ? want : cap);
-}
-
-// Grid of a grid-stride kernel: the blocks that are resident at once (one wave), or fewer when the work is small.
-// (A fixed cap of 8 blocks per SM launched the per-site kernel -- 6 resident blocks at 40 registers -- as one full wave
-// plus a third of one: ncu "waves per SM 1.33", profiles/r02h_persite_ncu_details.txt.)
-template <class K>
-static unsigned one_wave_grid(K kern, int threads, uint64_t want_blocks) {
-	int per_sm = 0;
-	if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, threads, 0) != cudaSuccess || per_sm < 1) per_sm = 1;
-	const uint64_t cap = (uint64_t)num_sms() * per_sm;
-	return (unsigned)(want_blocks < cap ? (want_blocks ? want_blocks : 1) : cap);
 }
 
 #include "pgt_kernels_common.cuh"
@@ -475,7 +455,7 @@ extern "C" int pgt_plan_scan_path(const pgt_plan* plan, pgt_stat stat) {
 
 extern "C" size_t pgt_plan_device_bytes(const pgt_plan* plan) {
 	if (!plan) return 0;
-	return align_up(plan->segs.size() * sizeof(pgt_seg), 256) + align_up(plan->off.size() * sizeof(uint64_t), 256) + 256;
+	return table_pair_bytes(plan->segs.size() * sizeof(pgt_seg), plan->off.size() * sizeof(uint64_t));
 }
 
 extern "C" int pgt_plan_bind_device(pgt_plan* plan, void* buffer, size_t bytes, void* stream) {
@@ -485,14 +465,8 @@ extern "C" int pgt_plan_bind_device(pgt_plan* plan, void* buffer, size_t bytes, 
 		return PGT_OK;
 	}
 	if (bytes < pgt_plan_device_bytes(plan)) return pgt_set_error(PGT_ERR_NOMEM, "pgt_plan_bind_device: buffer too small");
-	cudaStream_t st = (cudaStream_t)stream;
-	unsigned char* b = (unsigned char*)(((uintptr_t)buffer + 255) / 256 * 256);
-	const size_t seg_bytes = plan->segs.size() * sizeof(pgt_seg);
-	if (seg_bytes) PGT_CUDA(cudaMemcpyAsync(b, plan->segs.data(), seg_bytes, cudaMemcpyHostToDevice, st));
-	PGT_CUDA(cudaMemcpyAsync(b + align_up(seg_bytes, 256), plan->off.data(), plan->off.size() * sizeof(uint64_t), cudaMemcpyHostToDevice, st));
-	PGT_CUDA(cudaStreamSynchronize(st));
-	plan->d_tables = b;
-	return PGT_OK;
+	return bind_table_pair(buffer, plan->segs.data(), plan->segs.size() * sizeof(pgt_seg), plan->off.data(), plan->off.size() * sizeof(uint64_t),
+	                       stream, &plan->d_tables);
 }
 
 extern "C" size_t pgt_scan_workspace_bytes(const pgt_plan* plan, const pgt_range* range, pgt_stat stat, pgt_mem mem) {

@@ -16,75 +16,74 @@
 #include <thread>
 #include <vector>
 
-#include "pgt_internal.h"
+#include "pgt_cuda.h"
 
 namespace {
 
-struct ShardJob {
-	uint32_t shard = 0;
-	int device = 0;
-	uint64_t w_lo = 0, w_hi = 0;
+// One shard of a multi-GPU scan.  The caller's describe() sets its windows (and sites), whether it is idle (nothing to
+// scan) and its workspace: the caller's own, or ws = nullptr and the bytes to allocate for the call.
+struct Shard {
+	pgt_range range{};
+	bool idle = false;
 	void* ws = nullptr;
 	size_t ws_bytes = 0;
-	bool own_ws = false;
-	double global3[3] = {0.0, 0.0, 0.0};
+	double global3[3] = {0.0, 0.0, 0.0};  // the window scan's part of dxyWindow's global line
 	int rc = PGT_OK;
 	std::string err;
 };
 
-pgt_windows rows_from(const pgt_windows& o, uint64_t d) {
-	pgt_windows r = o;
-	for_each_field([d](auto*& p) { p = p ? p + d : p; }, r);
-	return r;
-}
-
-void run_shard(const pgt_plan* plan, pgt_stat stat, const pgt_columns* cols, int minind, const uint64_t* site_offsets, const pgt_windows* out,
-               ShardJob* job) {
-	auto fail = [job](int rc, const std::string& msg) {
-		job->rc = rc;
-		job->err = msg;
+// The shards of a multi-GPU scan: after the device list is checked, describe(i, shard) sets up shard i, and every shard
+// that is not idle runs scan(shard, stream) on devices[i] from a host thread of its own (inline for one device), on a
+// stream of its own and in its workspace.  The caller's current device is restored; the first failing shard is reported.
+template <class Describe, class Scan>
+int run_shards(const char* who, const int* devices, uint32_t ndev, std::vector<Shard>& shards, Describe&& describe, Scan&& scan) {
+	if (!devices || ndev == 0) return pgt_set_error(PGT_ERR_ARGS, std::string(who) + ": no devices given");
+	int have = 0;
+	if (cudaGetDeviceCount(&have) != cudaSuccess || have == 0)
+		return pgt_set_error(PGT_ERR_CUDA, "no usable CUDA device (libpgtscan has no CPU fallback)");
+	// (a device may be listed more than once: its shards then run side by side on it, each on its own stream)
+	for (uint32_t i = 0; i < ndev; ++i)
+		if (devices[i] < 0 || devices[i] >= have) return pgt_set_error(PGT_ERR_ARGS, std::string(who) + ": device index out of range");
+	shards.assign(ndev, Shard());
+	for (uint32_t i = 0; i < ndev; ++i) PGT_TRY(describe(i, shards[i]));
+	auto run = [&](uint32_t i) {
+		Shard& s = shards[i];
+		if (s.idle) return;
+		auto fail = [&s](int rc, const std::string& msg) {
+			s.rc = rc;
+			s.err = msg;
+		};
+		cudaError_t e = cudaSetDevice(devices[i]);
+		if (e != cudaSuccess) return fail(PGT_ERR_CUDA, std::string("cudaSetDevice: ") + cudaGetErrorString(e));
+		const bool own_ws = !s.ws;
+		if (own_ws) {
+			e = cudaMalloc(&s.ws, s.ws_bytes ? s.ws_bytes : 1);
+			if (e != cudaSuccess) return fail(PGT_ERR_CUDA, std::string("cudaMalloc(workspace): ") + cudaGetErrorString(e));
+		}
+		cudaStream_t st = nullptr;
+		e = cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking);
+		if (e != cudaSuccess) {
+			fail(PGT_ERR_CUDA, std::string("cudaStreamCreate: ") + cudaGetErrorString(e));
+		} else {
+			const int rc = scan(s, st);
+			if (rc != PGT_OK) fail(rc, pgt_last_error());
+			cudaStreamDestroy(st);
+		}
+		if (own_ws) cudaFree(s.ws);
 	};
-	cudaError_t e = cudaSetDevice(job->device);
-	if (e != cudaSuccess) return fail(PGT_ERR_CUDA, std::string("cudaSetDevice: ") + cudaGetErrorString(e));
-	// the whole axis is addressable from element 0 of the caller's columns; the scan touches only its slabs
-	pgt_range range;
-	range.w_lo = job->w_lo;
-	range.w_hi = job->w_hi;
-	range.site_origin = 0;
-	range.site_count = 0;
-	if (job->w_lo == job->w_hi && (pgt_plan_num_windows(plan) != 0 || job->shard != 0)) {
-		// a shard without windows has nothing to do ({0, 0} would even mean "all windows" to pgt_scan) -- except
-		// shard 0 of a plan without any window: it owns the axis, whose sites still count for the global line
-		return;
+	int prev = 0;
+	cudaGetDevice(&prev);
+	if (ndev == 1) {
+		run(0);
+	} else {
+		std::vector<std::thread> th;
+		for (uint32_t i = 0; i < ndev; ++i) th.emplace_back(run, i);
+		for (auto& t : th) t.join();
 	}
-	if (!job->ws) {
-		job->ws_bytes = pgt_scan_workspace_bytes(plan, &range, stat, PGT_MEM_HOST);
-		e = cudaMalloc(&job->ws, job->ws_bytes ? job->ws_bytes : 1);
-		if (e != cudaSuccess) return fail(PGT_ERR_CUDA, std::string("cudaMalloc(workspace): ") + cudaGetErrorString(e));
-		job->own_ws = true;
-	}
-	cudaStream_t st = nullptr;
-	e = cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking);
-	if (e != cudaSuccess) return fail(PGT_ERR_CUDA, std::string("cudaStreamCreate: ") + cudaGetErrorString(e));
-	pgt_windows rows = rows_from(*out, job->w_lo);
-	rows.dxy_global = out->dxy_global ? job->global3 : nullptr;
-	const int rc = pgt_scan(plan, &range, stat, cols, minind, site_offsets, &rows, job->ws, job->ws_bytes, PGT_MEM_HOST, st);
-	if (rc != PGT_OK) fail(rc, pgt_last_error());
-	cudaStreamDestroy(st);
-	if (job->own_ws) {
-		cudaFree(job->ws);
-		job->ws = nullptr;
-	}
-}
-
-int shard_ranges(const pgt_plan* plan, uint32_t ndev, std::vector<ShardJob>* jobs) {
-	jobs->resize(ndev);
-	for (uint32_t i = 0; i < ndev; ++i) {
-		ShardJob& j = (*jobs)[i];
-		j.shard = i;
-		const int rc = pgt_plan_shard(plan, i, ndev, &j.w_lo, &j.w_hi, nullptr, nullptr);
-		if (rc != PGT_OK) return rc;
-	}
+	cudaSetDevice(prev);
+	for (uint32_t i = 0; i < ndev; ++i)
+		if (shards[i].rc != PGT_OK)
+			return pgt_set_error(shards[i].rc, "shard " + std::to_string(i) + " on device " + std::to_string(devices[i]) + ": " + shards[i].err);
 	return PGT_OK;
 }
 
@@ -104,42 +103,35 @@ extern "C" int pgt_scan_sharded(const pgt_plan* plan, pgt_stat stat, const pgt_c
                                 const pgt_windows* out, const int* devices, uint32_t ndev, void* const* workspaces,
                                 const size_t* workspace_bytes) {
 	if (!plan || !cols || !out) return pgt_set_error(PGT_ERR_ARGS, "pgt_scan_sharded: plan, cols and out must not be NULL");
-	if (!devices || ndev == 0) return pgt_set_error(PGT_ERR_ARGS, "pgt_scan_sharded: no devices given");
 	if ((workspaces == nullptr) != (workspace_bytes == nullptr))
 		return pgt_set_error(PGT_ERR_ARGS, "pgt_scan_sharded: workspaces and workspace_bytes go together (both NULL = allocate per call)");
-	int have = 0;
-	if (cudaGetDeviceCount(&have) != cudaSuccess || have == 0)
-		return pgt_set_error(PGT_ERR_CUDA, "no usable CUDA device (libpgtscan has no CPU fallback)");
 	if (plan->d_tables) return pgt_set_error(PGT_ERR_ARGS, "pgt_scan_sharded: the plan is bound to one device (pgt_plan_bind_device); unbind it first");
-	// (a device may be listed more than once: its shards then run side by side on it, each on its own stream)
-	for (uint32_t i = 0; i < ndev; ++i)
-		if (devices[i] < 0 || devices[i] >= have) return pgt_set_error(PGT_ERR_ARGS, "pgt_scan_sharded: device index out of range");
-	std::vector<ShardJob> jobs;
-	const int rc0 = shard_ranges(plan, ndev, &jobs);
-	if (rc0 != PGT_OK) return rc0;
-	for (uint32_t i = 0; i < ndev; ++i) {
-		jobs[i].device = devices[i];
-		if (workspaces) {
-			jobs[i].ws = workspaces[i];
-			jobs[i].ws_bytes = workspace_bytes[i];
+	auto describe = [&](uint32_t i, Shard& s) -> int {
+		// the whole axis is addressable from element 0 of the caller's columns; the scan touches only its slabs
+		PGT_TRY(pgt_plan_shard(plan, i, ndev, &s.range.w_lo, &s.range.w_hi, nullptr, nullptr));
+		// a shard without windows has nothing to do ({0, 0} would even mean "all windows" to pgt_scan) -- except
+		// shard 0 of a plan without any window: it owns the axis, whose sites still count for the global line
+		s.idle = s.range.w_lo == s.range.w_hi && (pgt_plan_num_windows(plan) != 0 || i != 0);
+		if (workspaces && workspaces[i]) {
+			s.ws = workspaces[i];
+			s.ws_bytes = workspace_bytes[i];
+		} else if (!s.idle) {
+			s.ws_bytes = pgt_scan_workspace_bytes(plan, &s.range, stat, PGT_MEM_HOST);
 		}
-	}
-	int prev = 0;
-	cudaGetDevice(&prev);
-	if (ndev == 1) {
-		run_shard(plan, stat, cols, minind, site_offsets, out, &jobs[0]);
-	} else {
-		std::vector<std::thread> th;
-		for (uint32_t i = 0; i < ndev; ++i) th.emplace_back(run_shard, plan, stat, cols, minind, site_offsets, out, &jobs[i]);
-		for (auto& t : th) t.join();
-	}
-	cudaSetDevice(prev);
-	for (const ShardJob& j : jobs)
-		if (j.rc != PGT_OK) return pgt_set_error(j.rc, "shard " + std::to_string(j.shard) + " on device " + std::to_string(j.device) + ": " + j.err);
+		return PGT_OK;
+	};
+	auto scan = [&](Shard& s, cudaStream_t st) {
+		pgt_windows rows = *out;
+		for_each_field([d = s.range.w_lo](auto*& p) { p = p ? p + d : p; }, rows);
+		rows.dxy_global = out->dxy_global ? s.global3 : nullptr;
+		return pgt_scan(plan, &s.range, stat, cols, minind, site_offsets, &rows, s.ws, s.ws_bytes, PGT_MEM_HOST, st);
+	};
+	std::vector<Shard> shards;
+	PGT_TRY(run_shards("pgt_scan_sharded", devices, ndev, shards, describe, scan));
 	if (out->dxy_global) {  // the shards own disjoint parts of the axis (pgt_plan_shard): their lines add up, in shard order
 		double g3[3] = {0.0, 0.0, 0.0};
-		for (const ShardJob& j : jobs)
-			for (int q = 0; q < 3; ++q) g3[q] += j.global3[q];
+		for (const Shard& s : shards)
+			for (int q = 0; q < 3; ++q) g3[q] += s.global3[q];
 		for (int q = 0; q < 3; ++q) out->dxy_global[q] = g3[q];
 	}
 	return PGT_OK;
@@ -150,65 +142,21 @@ extern "C" int pgt_scan_sharded(const pgt_plan* plan, pgt_stat stat, const pgt_c
 extern "C" int pgt_scan_extreme_sharded(const pgt_xplan* plan, pgt_xstat stat, double cutoff, const uint32_t* pos, const double* score,
                                         const pgt_xwindows* out, const int* devices, uint32_t ndev) {
 	if (!plan || !score || !out) return pgt_set_error(PGT_ERR_ARGS, "pgt_scan_extreme_sharded: plan, score and out must not be NULL");
-	if (!devices || ndev == 0) return pgt_set_error(PGT_ERR_ARGS, "pgt_scan_extreme_sharded: no devices given");
-	int have = 0;
-	if (cudaGetDeviceCount(&have) != cudaSuccess || have == 0)
-		return pgt_set_error(PGT_ERR_CUDA, "no usable CUDA device (libpgtscan has no CPU fallback)");
-	for (uint32_t i = 0; i < ndev; ++i)
-		if (devices[i] < 0 || devices[i] >= have) return pgt_set_error(PGT_ERR_ARGS, "pgt_scan_extreme_sharded: device index out of range");
-	struct XJob {
-		int device = 0;
-		pgt_range range;
-		int rc = PGT_OK;
-		std::string err;
-	};
-	std::vector<XJob> jobs(ndev);
-	for (uint32_t i = 0; i < ndev; ++i) {
+	auto describe = [&](uint32_t i, Shard& s) -> int {
 		uint64_t slo = 0, shi = 0;
-		jobs[i].device = devices[i];
-		const int rc = pgt_xplan_shard(plan, i, ndev, &jobs[i].range.w_lo, &jobs[i].range.w_hi, &slo, &shi);
-		if (rc != PGT_OK) return rc;
-		jobs[i].range.site_origin = slo;
-		jobs[i].range.site_count = shi - slo;
-	}
-	auto run = [&](XJob* job) {
-		if (job->range.w_hi <= job->range.w_lo) return;
-		cudaError_t e = cudaSetDevice(job->device);
-		void* ws = nullptr;
-		const size_t bytes = pgt_scan_extreme_workspace_bytes(plan, &job->range, PGT_MEM_HOST);
-		if (e == cudaSuccess) e = cudaMalloc(&ws, bytes ? bytes : 1);
-		cudaStream_t st = nullptr;
-		if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking);
-		if (e != cudaSuccess) {
-			job->rc = PGT_ERR_CUDA;
-			job->err = cudaGetErrorString(e);
-			if (ws) cudaFree(ws);
-			return;
-		}
-		pgt_xwindows rows = *out;
-		const uint64_t d = job->range.w_lo;
-		for_each_xfield([d](auto*& p) { p = p ? p + d : p; }, rows);
-		const uint64_t s0 = job->range.site_origin;
-		const int rc = pgt_scan_extreme(plan, &job->range, stat, cutoff, pos ? pos + s0 : nullptr, score + s0, &rows, ws, bytes, PGT_MEM_HOST, st);
-		if (rc != PGT_OK) {
-			job->rc = rc;
-			job->err = pgt_last_error();
-		}
-		cudaStreamDestroy(st);
-		cudaFree(ws);
+		PGT_TRY(pgt_xplan_shard(plan, i, ndev, &s.range.w_lo, &s.range.w_hi, &slo, &shi));
+		s.range.site_origin = slo;
+		s.range.site_count = shi - slo;
+		s.idle = s.range.w_hi <= s.range.w_lo;
+		if (!s.idle) s.ws_bytes = pgt_scan_extreme_workspace_bytes(plan, &s.range, PGT_MEM_HOST);
+		return PGT_OK;
 	};
-	int prev = 0;
-	cudaGetDevice(&prev);
-	if (ndev == 1) {
-		run(&jobs[0]);
-	} else {
-		std::vector<std::thread> th;
-		for (uint32_t i = 0; i < ndev; ++i) th.emplace_back(run, &jobs[i]);
-		for (auto& t : th) t.join();
-	}
-	cudaSetDevice(prev);
-	for (uint32_t i = 0; i < ndev; ++i)
-		if (jobs[i].rc != PGT_OK)
-			return pgt_set_error(jobs[i].rc, "shard " + std::to_string(i) + " on device " + std::to_string(jobs[i].device) + ": " + jobs[i].err);
-	return PGT_OK;
+	auto scan = [&](Shard& s, cudaStream_t st) {
+		pgt_xwindows rows = *out;
+		for_each_xfield([d = s.range.w_lo](auto*& p) { p = p ? p + d : p; }, rows);
+		const uint64_t s0 = s.range.site_origin;
+		return pgt_scan_extreme(plan, &s.range, stat, cutoff, pos ? pos + s0 : nullptr, score + s0, &rows, s.ws, s.ws_bytes, PGT_MEM_HOST, st);
+	};
+	std::vector<Shard> shards;
+	return run_shards("pgt_scan_extreme_sharded", devices, ndev, shards, describe, scan);
 }

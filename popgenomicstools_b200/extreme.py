@@ -12,29 +12,26 @@ import numpy as np
 
 from . import _cabi
 from ._cabi import PgtRange, PgtXWindows, check
+from .scan import _Plan, _columns, _table, _torch
 
 XWINDOW_FIELDS = _cabi.XWINDOW_FIELDS
-_X_DTYPES = {"ext_value": np.float64, "ext_pos": np.uint32, "ext_site": np.uint64, "nbig": np.uint32,
-             "nsites": np.uint32, "prop": np.float64}
+_X_DTYPES = {"ext_value": "float64", "ext_pos": "uint32", "ext_site": "uint64", "nbig": "uint32", "nsites": "uint32",
+             "prop": "float64"}
+_XFIELDS_NO_POS = tuple(k for k in XWINDOW_FIELDS if k != "ext_pos")
 
 
-def _torch():
-    import torch
-    return torch
-
-
-class ExtremePlan:
+class ExtremePlan(_Plan):
     """Window bookkeeping of ihsWindow / xpehhWindow (pgt_xplan_*): which rows the reference prints
     and which sites each window holds.
 
     pos: HOST position column (numpy uint32, file order); contig_offsets: cumulative site counts of
     the runs of equal chromosome name; chrlen: per-run -chrlen length (0 = not listed) or None.
     """
+    _destroy, _device_bytes, _bind_device, _shard = (
+        "pgt_xplan_destroy", "pgt_xplan_device_bytes", "pgt_xplan_bind_device", "pgt_xplan_shard")
 
     def __init__(self, pos, contig_offsets, winsize=100000, chrlen=None, unit_sites=0):
-        lib = _cabi.load()
-        self._lib = lib
-        self._h = None
+        super().__init__()
         self.pos = np.ascontiguousarray(pos, dtype=np.uint32)
         self.offsets = np.ascontiguousarray(contig_offsets, dtype=np.uint64)
         ncontig = len(self.offsets) - 1
@@ -49,21 +46,10 @@ class ExtremePlan:
             raise _cabi.PgtError(_cabi.PGT_ERR_ARGS, "winsize out of range")
         self.winsize = int(winsize)
         h = C.c_void_p()
-        check(lib.pgt_xplan_create(C.byref(h), self.pos.ctypes.data, self.offsets.ctypes.data,
-                                   self.chrlen.ctypes.data if self.chrlen is not None else None, ncontig, self.winsize,
-                                   int(unit_sites)))
+        check(self._lib.pgt_xplan_create(C.byref(h), self.pos.ctypes.data, self.offsets.ctypes.data,
+                                         self.chrlen.ctypes.data if self.chrlen is not None else None, ncontig, self.winsize,
+                                         int(unit_sites)))
         self._h = h
-        self._workspaces = {}
-        self._bound = None
-
-    def __del__(self):
-        h, self._h = getattr(self, "_h", None), None
-        if h:
-            self._lib.pgt_xplan_destroy(h)
-
-    @property
-    def handle(self):
-        return self._h
 
     @property
     def num_windows(self):
@@ -85,36 +71,12 @@ class ExtremePlan:
         check(self._lib.pgt_xplan_windows(self._h, *[o[k].ctypes.data for k in ("label", "start", "end", "first_site", "nsites")]))
         return o
 
-    def shard(self, rank, nranks):
-        """Window range [w_lo, w_hi) and site range [site_lo, site_hi) of shard `rank` (no halo)."""
-        v = [C.c_uint64() for _ in range(4)]
-        check(self._lib.pgt_xplan_shard(self._h, rank, nranks, *[C.byref(x) for x in v]))
-        return tuple(x.value for x in v)
-
-    def bind(self, device):
-        """Keep the window tables resident on `device` (pgt_xplan_bind_device); later scans on that
-        device skip the per-call table upload."""
-        torch = _torch()
-        device = torch.device(device)
-        if self._bound is not None and self._bound[0] == device:
-            return
-        buf = torch.empty(int(self._lib.pgt_xplan_device_bytes(self._h)), dtype=torch.uint8, device=device)
-        with torch.cuda.device(device):
-            check(self._lib.pgt_xplan_bind_device(self._h, buf.data_ptr(), buf.numel(),
-                                                  C.c_void_p(torch.cuda.current_stream(device).cuda_stream)))
-        self._bound = (device, buf)
-        self._workspaces = {}
+    def _workspace_bytes(self, mem, window_range, site_origin):
+        r = _xrange(self, window_range, site_origin)
+        return int(self._lib.pgt_scan_extreme_workspace_bytes(self._h, C.byref(r), mem))
 
     def workspace(self, device, mem, window_range=None, site_origin=0):
-        torch = _torch()
-        key = (str(device), mem, window_range, site_origin)
-        ws = self._workspaces.get(key)
-        if ws is None:
-            r = _xrange(self, window_range, site_origin)
-            ws = torch.empty(int(self._lib.pgt_scan_extreme_workspace_bytes(self._h, C.byref(r), mem)), dtype=torch.uint8,
-                             device=device)
-            self._workspaces[key] = ws
-        return ws
+        return self._workspace(device, mem, window_range, site_origin)
 
 
 def _xrange(plan, window_range, site_origin):
@@ -129,54 +91,20 @@ def scan_extreme(plan, stat, cutoff, pos, score, window_range=None, site_origin=
     lib = plan._lib
     on_device = isinstance(score, torch.Tensor) and score.is_cuda
     r = _xrange(plan, window_range, site_origin)
-    nwin = r.w_hi - r.w_lo
-    keep = []
-
-    def ptr(v, want, name):
-        if v is None:
-            return None
-        if on_device:
-            if not (isinstance(v, torch.Tensor) and v.is_cuda and v.is_contiguous()):
-                raise TypeError(f"{name}: expected a contiguous CUDA tensor")
-            if name == "pos" and v.dtype == torch.int32:
-                v = v.view(torch.uint32)
-            if str(v.dtype) != "torch." + np.dtype(want).name:
-                raise TypeError(f"{name}: expected {np.dtype(want).name}, got {v.dtype}")
-            keep.append(v)
-            return v.data_ptr()
-        if isinstance(v, torch.Tensor):
-            v = v.numpy()
-        if v.dtype != np.dtype(want) or not v.flags["C_CONTIGUOUS"]:
-            raise TypeError(f"{name}: expected contiguous {np.dtype(want).name}, got {v.dtype}")
-        keep.append(v)
-        return v.ctypes.data
-
-    p_pos, p_score = ptr(pos, np.uint32, "pos"), ptr(score, np.float64, "score")
+    ptrs, keep = _columns(dict(pos=pos, score=score), ("pos", "score"), (), on_device)
     dev = score.device if on_device else torch.device(device if device is not None else f"cuda:{torch.cuda.current_device()}")
-    if out is None:
-        out = {}
-        for k in XWINDOW_FIELDS:
-            if k == "ext_pos" and pos is None:
-                continue
-            if on_device:
-                out[k] = torch.empty(nwin, dtype=getattr(torch, np.dtype(_X_DTYPES[k]).name), device=dev)
-            else:
-                out[k] = np.empty(nwin, _X_DTYPES[k])
-    w = PgtXWindows()
-    for k in XWINDOW_FIELDS:
-        v = out.get(k)
-        if v is not None:
-            setattr(w, k, v.data_ptr() if on_device else v.ctypes.data)
+    names = XWINDOW_FIELDS if pos is not None else _XFIELDS_NO_POS
+    out, w = _table(PgtXWindows, out, names, _X_DTYPES, r.w_hi - r.w_lo, dev if on_device else None)
     mem = _cabi.PGT_MEM_DEVICE if on_device else _cabi.PGT_MEM_HOST
     if on_device:
         plan.bind(dev)
     elif plan._bound is not None and plan._bound[0] != dev:
         raise ValueError(f"plan is bound to {plan._bound[0]}, scan requested on {dev}")
-    ws = plan.workspace(dev, mem, window_range, site_origin)
+    ws = plan._workspace(dev, mem, window_range, site_origin)
     with torch.cuda.device(dev):
         stream = torch.cuda.current_stream(dev).cuda_stream
-        check(lib.pgt_scan_extreme(plan.handle, C.byref(r), int(stat), float(cutoff), p_pos, p_score, C.byref(w), ws.data_ptr(),
-                                   ws.numel(), mem, C.c_void_p(stream)))
+        check(lib.pgt_scan_extreme(plan.handle, C.byref(r), int(stat), float(cutoff), ptrs.get("pos"), ptrs.get("score"), C.byref(w),
+                                   ws.data_ptr(), ws.numel(), mem, C.c_void_p(stream)))
     return out
 
 
@@ -186,10 +114,7 @@ def scan_extreme_sharded(plan, stat, cutoff, pos, score, devices):
     lib = plan._lib
     pos = None if pos is None else np.ascontiguousarray(pos, np.uint32)
     score = np.ascontiguousarray(score, np.float64)
-    out = {k: np.empty(plan.num_windows, _X_DTYPES[k]) for k in XWINDOW_FIELDS if not (k == "ext_pos" and pos is None)}
-    w = PgtXWindows()
-    for k, v in out.items():
-        setattr(w, k, v.ctypes.data)
+    out, w = _table(PgtXWindows, None, XWINDOW_FIELDS if pos is not None else _XFIELDS_NO_POS, _X_DTYPES, plan.num_windows, None)
     dev = (C.c_int * len(devices))(*[int(d) for d in devices])
     check(lib.pgt_scan_extreme_sharded(plan.handle, int(stat), float(cutoff), pos.ctypes.data if pos is not None else None,
                                        score.ctypes.data, C.byref(w), dev, len(devices)))

@@ -12,7 +12,7 @@ import ctypes as C
 import numpy as np
 
 from . import _cabi
-from ._cabi import COLUMN_FIELDS, WINDOW_FIELDS, PgtColumns, PgtRange, PgtWindows, check
+from ._cabi import WINDOW_FIELDS, PgtColumns, PgtRange, PgtWindows, check
 
 
 def _torch():
@@ -20,16 +20,68 @@ def _torch():
     return torch
 
 
-class WindowPlan:
+class _Plan:
+    """What WindowPlan and ExtremePlan share: the library handle, the device tables (bind), shard ranges and the cache
+    of scan workspaces.  A subclass names its C functions and answers _workspace_bytes(*key)."""
+    _destroy = _device_bytes = _bind_device = _shard = None  # names of the plan kind's pgt_* functions
+
+    def __init__(self):
+        self._lib = _cabi.load()
+        self._h = None
+        self._workspaces = {}
+        self._bound = None
+
+    def __del__(self):
+        h, self._h = getattr(self, "_h", None), None
+        if h:
+            getattr(self._lib, self._destroy)(h)
+
+    @property
+    def handle(self):
+        return self._h
+
+    def bind(self, device):
+        """Keep the plan's device tables resident on `device`: later scans on that device upload nothing.  Called
+        automatically by device-mode scans."""
+        torch = _torch()
+        device = torch.device(device)
+        if self._bound is not None and self._bound[0] == device:
+            return
+        buf = torch.empty(int(getattr(self._lib, self._device_bytes)(self._h)), dtype=torch.uint8, device=device)
+        with torch.cuda.device(device):
+            check(getattr(self._lib, self._bind_device)(self._h, buf.data_ptr(), buf.numel(),
+                                                        C.c_void_p(torch.cuda.current_stream(device).cuda_stream)))
+        self._bound = (device, buf)
+        self._workspaces = {}
+
+    def shard(self, rank, nranks):
+        """Window range [w_lo, w_hi) and site range [site_lo, site_hi) of shard `rank`."""
+        v = [C.c_uint64() for _ in range(4)]
+        check(getattr(self._lib, self._shard)(self._h, rank, nranks, *[C.byref(x) for x in v]))
+        return tuple(x.value for x in v)
+
+    def _workspace(self, device, *key):
+        """Device scratch for a scan, cached per (device, tune epoch, key); `key` are the arguments of _workspace_bytes."""
+        full = (str(device), _tune_epoch[0]) + key
+        ws = self._workspaces.get(full)
+        if ws is None:
+            torch = _torch()
+            ws = torch.empty(self._workspace_bytes(*key), dtype=torch.uint8, device=device)
+            self._workspaces[full] = ws
+        return ws
+
+
+class WindowPlan(_Plan):
     """Closed-form window enumeration (pgt_plan_*): which windows the reference would print.
 
     contig_offsets: cumulative site counts (mode='sites') or chromosome lengths in bp
     (mode='bp'), length ncontig+1, in file order.
     """
+    _destroy, _device_bytes, _bind_device, _shard = (
+        "pgt_plan_destroy", "pgt_plan_device_bytes", "pgt_plan_bind_device", "pgt_plan_shard")
 
     def __init__(self, contig_offsets, winsize=1, stepsize=1, mode="sites", unit_sites=0):
-        lib = _cabi.load()
-        self._lib = lib
+        super().__init__()
         self.offsets = np.ascontiguousarray(contig_offsets, dtype=np.uint64)
         if self.offsets.ndim != 1 or len(self.offsets) < 1:
             raise ValueError("contig_offsets must be a 1-D array of length ncontig+1")
@@ -38,33 +90,9 @@ class WindowPlan:
         if not (0 <= self.winsize < 2**32 and 0 <= self.stepsize < 2**32):
             raise _cabi.PgtError(_cabi.PGT_ERR_ARGS, "winsize/stepsize out of range")
         h = C.c_void_p()
-        check(lib.pgt_plan_create(C.byref(h), self.mode, self.offsets.ctypes.data, len(self.offsets) - 1,
-                                  self.winsize, self.stepsize, int(unit_sites)))
+        check(self._lib.pgt_plan_create(C.byref(h), self.mode, self.offsets.ctypes.data, len(self.offsets) - 1,
+                                        self.winsize, self.stepsize, int(unit_sites)))
         self._h = h
-        self._workspaces = {}
-        self._bound = None
-
-    def bind(self, device):
-        """Keep the plan's device tables resident on `device` (pgt_plan_bind_device): later scans
-        on that device upload nothing.  Called automatically by device-mode scans."""
-        torch = _torch()
-        device = torch.device(device)
-        if self._bound is not None and self._bound[0] == device:
-            return
-        buf = torch.empty(int(self._lib.pgt_plan_device_bytes(self._h)), dtype=torch.uint8, device=device)
-        with torch.cuda.device(device):
-            check(self._lib.pgt_plan_bind_device(self._h, buf.data_ptr(), buf.numel(),
-                                                 C.c_void_p(torch.cuda.current_stream(device).cuda_stream)))
-        self._bound = (device, buf)
-
-    def __del__(self):
-        h, self._h = getattr(self, "_h", None), None
-        if h:
-            self._lib.pgt_plan_destroy(h)
-
-    @property
-    def handle(self):
-        return self._h
 
     @property
     def num_windows(self):
@@ -99,12 +127,6 @@ class WindowPlan:
         check(self._lib.pgt_plan_window_units(self._h, w, C.byref(f), C.byref(c)))
         return f.value, c.value
 
-    def shard(self, rank, nranks):
-        """Window range [w_lo, w_hi) and site range [site_lo, site_hi) of shard `rank`."""
-        v = [C.c_uint64() for _ in range(4)]
-        check(self._lib.pgt_plan_shard(self._h, rank, nranks, *[C.byref(x) for x in v]))
-        return tuple(x.value for x in v)
-
     def scan_path(self, stat):
         """'units' | 'slide' | 'persite': the kernels a scan of `stat` runs (pgt_plan_scan_path)."""
         return ("units", "slide", "persite")[check(self._lib.pgt_plan_scan_path(self._h, stat))]
@@ -113,16 +135,11 @@ class WindowPlan:
         r = _range(self, window_range, site_origin, site_count)
         return int(self._lib.pgt_scan_workspace_bytes(self._h, C.byref(r), stat, mem))
 
+    _workspace_bytes = workspace_bytes
+
     def workspace(self, device, stat, mem, window_range=None, site_origin=0, site_count=0):
         """Device scratch for a scan, cached per (device, stat, mem, range)."""
-        torch = _torch()
-        key = (str(device), stat, mem, window_range, site_origin, site_count, _tune_epoch[0])
-        ws = self._workspaces.get(key)
-        if ws is None:
-            ws = torch.empty(self.workspace_bytes(stat, mem, window_range, site_origin, site_count), dtype=torch.uint8,
-                             device=device)
-            self._workspaces[key] = ws
-        return ws
+        return self._workspace(device, stat, mem, window_range, site_origin, site_count)
 
 
 def _range(plan, window_range, site_origin, site_count=0):
@@ -133,8 +150,8 @@ def _range(plan, window_range, site_origin, site_count=0):
 _tune_epoch = [0]
 
 _COL_DTYPES = {"pos": "uint32", "a": "float64", "b": "float64", "geno": "int8", "f1": "float64", "f2": "float64",
-               "n1": "int32", "n2": "int32"}
-_F64_OUT = ("sum_a", "sum_b", "fst", "het", "dxy")
+               "n1": "int32", "n2": "int32", "score": "float64"}
+_W_DTYPES = {k: "float64" if k in ("sum_a", "sum_b", "fst", "het", "dxy", "dxy_global") else "uint32" for k in WINDOW_FIELDS}
 _STAT_COLS = {
     _cabi.PGT_STAT_FST: ("a", "b"),
     _cabi.PGT_STAT_HET: ("geno",),
@@ -149,9 +166,55 @@ _STAT_OUTS = {
 }
 
 
-def _is_tensor(x):
+def _columns(cols, names, need, on_device):
+    """Data pointers of the columns `names` found in `cols` (name -> array), checked against their dtypes: contiguous
+    CUDA tensors if `on_device`, else numpy arrays (CPU tensors are viewed as numpy).  int32 positions are viewed as
+    uint32.  Every column of `need` must be present.  Returns (name -> pointer, the arrays to keep alive)."""
+    for k in need:
+        if cols.get(k) is None:
+            raise ValueError(f"column {k!r} is required")
     torch = _torch()
-    return isinstance(x, torch.Tensor)
+    ptrs, keep = {}, []
+    for k in names:
+        v = cols.get(k)
+        if v is None:
+            continue
+        want = _COL_DTYPES[k]
+        if on_device:
+            if not (isinstance(v, torch.Tensor) and v.is_cuda and v.is_contiguous()):
+                raise TypeError(f"{k}: expected a contiguous CUDA tensor")
+            if k == "pos" and v.dtype == torch.int32:
+                v = v.view(torch.uint32)
+            if str(v.dtype) != "torch." + want:
+                raise TypeError(f"{k}: expected {want}, got {v.dtype}")
+            ptrs[k] = v.data_ptr()
+        else:
+            if isinstance(v, torch.Tensor):
+                v = v.numpy()
+            if k == "pos" and v.dtype == np.int32:
+                v = v.view(np.uint32)
+            if v.dtype != np.dtype(want) or not v.flags["C_CONTIGUOUS"]:
+                raise TypeError(f"{k}: expected contiguous {want}, got {v.dtype}")
+            ptrs[k] = v.ctypes.data
+        keep.append(v)
+    return ptrs, keep
+
+
+def _table(struct, out, names, dtypes, nrows, device):
+    """A result table: `out` (name -> array), or if it is None new arrays `names` of `nrows` rows (dxy_global: 3) and
+    `dtypes` -- CUDA tensors on `device`, numpy arrays if `device` is None.  Returns (out, `struct` pointing at it)."""
+    if out is None:
+        if device is None:
+            out = {k: np.empty(3 if k == "dxy_global" else nrows, dtypes[k]) for k in names}
+        else:
+            torch = _torch()
+            out = {k: torch.empty(3 if k == "dxy_global" else nrows, dtype=getattr(torch, dtypes[k]), device=device) for k in names}
+    t = struct()
+    for k, _ in struct._fields_:
+        v = out.get(k)
+        if v is not None:
+            setattr(t, k, v.ctypes.data if device is None else v.data_ptr())
+    return out, t
 
 
 def scan(plan, stat, cols, minind=1, site_offsets=None, window_range=None, site_origin=0, site_count=0, out=None,
@@ -162,56 +225,13 @@ def scan(plan, stat, cols, minind=1, site_offsets=None, window_range=None, site_
     torch = _torch()
     lib = plan._lib
     need = _STAT_COLS[stat]
-    for k in need:
-        if cols.get(k) is None:
-            raise ValueError(f"column {k!r} is required")
-    sample = cols[need[0]]
-    on_device = _is_tensor(sample) and sample.is_cuda
+    sample = cols.get(need[0])
+    on_device = isinstance(sample, torch.Tensor) and sample.is_cuda
+    ptrs, keep = _columns(cols, ("pos",) + need, need, on_device)
+    c = PgtColumns(**ptrs)
     r = _range(plan, window_range, site_origin, site_count)
-    nwin = r.w_hi - r.w_lo
-    c = PgtColumns()
-    keep = []
-    for k in COLUMN_FIELDS:
-        v = cols.get(k)
-        if v is None or (k != "pos" and k not in need):
-            continue
-        want = _COL_DTYPES[k]
-        if on_device:
-            if not (_is_tensor(v) and v.is_cuda and v.is_contiguous()):
-                raise TypeError(f"{k}: expected a contiguous CUDA tensor")
-            if k == "pos" and v.dtype == torch.int32:
-                v = v.view(torch.uint32)
-            if str(v.dtype) != "torch." + want:
-                raise TypeError(f"{k}: expected {want}, got {v.dtype}")
-            setattr(c, k, v.data_ptr())
-        else:
-            if _is_tensor(v):
-                v = v.numpy()
-            if k == "pos" and v.dtype == np.int32:
-                v = v.view(np.uint32)
-            if v.dtype != np.dtype(want) or not v.flags["C_CONTIGUOUS"]:
-                raise TypeError(f"{k}: expected contiguous {want}, got {v.dtype}")
-            setattr(c, k, v.ctypes.data)
-        keep.append(v)
-    if on_device:
-        dev = sample.device
-    else:
-        dev = torch.device(device if device is not None else f"cuda:{torch.cuda.current_device()}")
-    names = _STAT_OUTS[stat]
-    if out is None:
-        out = {}
-        for k in names:
-            n = 3 if k == "dxy_global" else nwin
-            f64 = k in _F64_OUT or k == "dxy_global"
-            if on_device:
-                out[k] = torch.empty(n, dtype=torch.float64 if f64 else torch.uint32, device=dev)
-            else:
-                out[k] = np.empty(n, np.float64 if f64 else np.uint32)
-    w = PgtWindows()
-    for k in WINDOW_FIELDS:
-        v = out.get(k)
-        if v is not None:
-            setattr(w, k, v.data_ptr() if on_device else v.ctypes.data)
+    dev = sample.device if on_device else torch.device(device if device is not None else f"cuda:{torch.cuda.current_device()}")
+    out, w = _table(PgtWindows, out, _STAT_OUTS[stat], _W_DTYPES, r.w_hi - r.w_lo, dev if on_device else None)
     so = None
     if site_offsets is not None:
         so = np.ascontiguousarray(site_offsets, dtype=np.uint64)
@@ -221,7 +241,7 @@ def scan(plan, stat, cols, minind=1, site_offsets=None, window_range=None, site_
         plan.bind(dev)
     elif plan._bound is not None and plan._bound[0] != dev:
         raise ValueError(f"plan is bound to {plan._bound[0]}, scan requested on {dev}")
-    ws = plan.workspace(dev, stat, mem, window_range, site_origin, site_count)
+    ws = plan._workspace(dev, stat, mem, window_range, site_origin, site_count)
     with torch.cuda.device(dev):
         stream = torch.cuda.current_stream(dev).cuda_stream
         check(lib.pgt_scan(plan.handle, C.byref(r), stat, C.byref(c), int(minind), so.ctypes.data if so is not None else None,
@@ -235,35 +255,10 @@ def scan_sharded(plan, stat, cols, devices, minind=1, site_offsets=None, out=Non
     windows; per-window results are bit-identical for any device list."""
     lib = plan._lib
     need = _STAT_COLS[stat]
-    c = PgtColumns()
-    keep = []
-    for k in COLUMN_FIELDS:
-        v = cols.get(k)
-        if v is None or (k != "pos" and k not in need):
-            continue
-        if _is_tensor(v):
-            v = v.numpy()
-        if k == "pos" and v.dtype == np.int32:
-            v = v.view(np.uint32)
-        if v.dtype != np.dtype(_COL_DTYPES[k]) or not v.flags["C_CONTIGUOUS"]:
-            raise TypeError(f"{k}: expected contiguous {_COL_DTYPES[k]}, got {v.dtype}")
-        setattr(c, k, v.ctypes.data)
-        keep.append(v)
-    for k in need:
-        if cols.get(k) is None:
-            raise ValueError(f"column {k!r} is required")
-    nwin = plan.num_windows
-    if out is None:
-        out = {k: np.empty(3 if k == "dxy_global" else nwin, np.float64 if (k in _F64_OUT or k == "dxy_global") else np.uint32)
-               for k in _STAT_OUTS[stat]}
-    w = PgtWindows()
-    for k in WINDOW_FIELDS:
-        v = out.get(k)
-        if v is not None:
-            setattr(w, k, v.ctypes.data)
-    so = None
-    if site_offsets is not None:
-        so = np.ascontiguousarray(site_offsets, dtype=np.uint64)
+    ptrs, keep = _columns(cols, ("pos",) + need, need, False)
+    c = PgtColumns(**ptrs)
+    out, w = _table(PgtWindows, out, _STAT_OUTS[stat], _W_DTYPES, plan.num_windows, None)
+    so = None if site_offsets is None else np.ascontiguousarray(site_offsets, dtype=np.uint64)
     dev = (C.c_int * len(devices))(*[int(d) for d in devices])
     check(lib.pgt_scan_sharded(plan.handle, stat, C.byref(c), int(minind), so.ctypes.data if so is not None else None, C.byref(w),
                                dev, len(devices), None, None))
