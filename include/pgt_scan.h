@@ -61,7 +61,12 @@ typedef enum {
 	PGT_MODE_SITES = 0,
 	/* windows of W bp stepping S bp over the dense per-bp entry stream of every chromosome:
 	 * dxyWindow -fixedsite 0 (dxyWindow.cpp:336-355,363-373,407-426).  `contig_offsets` then
-	 * holds cumulative chromosome LENGTHS IN BP (from -sizefile), not site counts. */
+	 * holds cumulative chromosome LENGTHS IN BP (from -sizefile), not site counts.  Every
+	 * statistic can be scanned over such a plan: the windows are the ones dxyWindow -fixedsite 0
+	 * prints (its quirks included), so the tables of all statistics over one plan line up row for
+	 * row, and a window reduces the sites whose positions fall on its bp (site i of chromosome c
+	 * sits on entry contig_offsets[c] + pos[i] - 1; bp without a site contribute nothing).
+	 * nsites then counts bp; pgt_scan_bp_sites gives the sites per window. */
 	PGT_MODE_BP = 1
 } pgt_mode;
 
@@ -155,10 +160,11 @@ typedef struct {
 } pgt_range;
 
 typedef enum {
-	PGT_STAT_FST = 0,   /* fstWindow */
-	PGT_STAT_HET = 1,   /* hetWindow */
+	PGT_STAT_FST = 0,   /* fstWindow (PGT_MODE_BP plan: fixed-bp windows, as ANGSD's realSFS fst stats2 -win/-step) */
+	PGT_STAT_HET = 1,   /* hetWindow (PGT_MODE_BP plan: fixed-bp windows) */
 	PGT_STAT_DXY = 2,   /* dxyWindow (-fixedsite 1: PGT_MODE_SITES plan; -fixedsite 0: PGT_MODE_BP plan) */
-	PGT_STAT_FUSED = 3  /* fst + dxy + het over one site axis in one pass (BASELINE config 5) */
+	PGT_STAT_FUSED = 3  /* fst + dxy + het over one site axis in one pass (BASELINE config 5), either mode; each
+	                       statistic equals its single scan bit for bit */
 } pgt_stat;
 
 /* Input columns, one element per site; only the columns of the requested statistic are read.
@@ -192,7 +198,7 @@ typedef struct {
 	uint32_t* start_pos;   /* pos of first site (bp mode: first bp of the window) */
 	uint32_t* end_pos;     /* pos of last site  (bp mode: last bp of the window) */
 	uint32_t* mid_pos;     /* (start+end)/2 in uint32 arithmetic (fstWindow.cpp:73) */
-	uint32_t* nsites;      /* sites (entries) in the window */
+	uint32_t* nsites;      /* sites in the window (PGT_MODE_BP: bp; see pgt_scan_bp_sites) */
 	double* sum_a;         /* fst */
 	double* sum_b;
 	double* fst;           /* sum_b != 0 ? sum_a/sum_b : 0 (fstWindow.cpp:85) */
@@ -225,6 +231,18 @@ size_t pgt_scan_workspace_bytes(const pgt_plan* plan, const pgt_range* range, pg
 int pgt_scan(const pgt_plan* plan, const pgt_range* range, pgt_stat stat, const pgt_columns* cols, int minind,
              const uint64_t* site_offsets, const pgt_windows* out, void* workspace, size_t workspace_bytes,
              pgt_mem mem, void* stream);
+
+/* Sites per window of a PGT_MODE_BP plan: nsites_data[w - w_lo] = number of sites whose positions fall on the bp of
+ * window w, for the windows of `range` (the rows of a pgt_scan over the same plan and range; its `nsites` counts bp).
+ * pos and site_offsets as for pgt_scan: pos addresses element range->site_origin of the position column and holds
+ * range->site_count elements (0 = up to the end of the genome).  The call
+ * also checks that every chromosome's first and last site it reads lie on the chromosome (1 <= pos <= length) and
+ * returns PGT_ERR_INPUT otherwise; to report that it waits for `stream` in both memory spaces.  PGT_MEM_HOST stages
+ * the positions of the chromosomes the windows touch through the workspace (4 bytes per site).  The workspace is
+ * device memory of at least pgt_scan_bp_sites_workspace_bytes() (site_offsets may be NULL for PGT_MEM_DEVICE). */
+size_t pgt_scan_bp_sites_workspace_bytes(const pgt_plan* plan, const pgt_range* range, const uint64_t* site_offsets, pgt_mem mem);
+int pgt_scan_bp_sites(const pgt_plan* plan, const pgt_range* range, const uint32_t* pos, const uint64_t* site_offsets,
+                      uint32_t* nsites_data, void* workspace, size_t workspace_bytes, pgt_mem mem, void* stream);
 
 /* One host column set, several GPUs of ONE process (the reference is a single process, fstWindow.cpp:158-177: a
  * user of the drop-in tools on an 8-GPU box should not have to split the input).  The window list is cut by
@@ -264,7 +282,8 @@ void pgt_uploader_destroy(pgt_uploader* up);
 int pgt_memcpy_to_host(void* host, const void* dev, size_t bytes);
 int pgt_device_mem_info(size_t* free_bytes, size_t* total_bytes);
 
-/* Convenience entry points named after the tools they replace. */
+/* Convenience entry points named after the tools they replace.  pgt_scan_fst, _het and _fused pass no site_offsets,
+ * so they scan PGT_MODE_SITES plans only; a PGT_MODE_BP scan of those statistics goes through pgt_scan. */
 int pgt_scan_fst(const pgt_plan* plan, const pgt_range* range, const pgt_columns* cols, const pgt_windows* out,
                  void* workspace, size_t workspace_bytes, pgt_mem mem, void* stream);
 int pgt_scan_het(const pgt_plan* plan, const pgt_range* range, const pgt_columns* cols, const pgt_windows* out,

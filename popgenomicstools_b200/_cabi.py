@@ -94,6 +94,9 @@ PROTOTYPES = {
     "pgt_scan_workspace_bytes": (C.c_size_t, [C.c_void_p, C.POINTER(PgtRange), C.c_int, C.c_int]),
     "pgt_scan": (C.c_int, [C.c_void_p, C.POINTER(PgtRange), C.c_int, C.POINTER(PgtColumns), C.c_int, C.c_void_p,
                            C.POINTER(PgtWindows), C.c_void_p, C.c_size_t, C.c_int, C.c_void_p]),
+    "pgt_scan_bp_sites_workspace_bytes": (C.c_size_t, [C.c_void_p, C.POINTER(PgtRange), C.c_void_p, C.c_int]),
+    "pgt_scan_bp_sites": (C.c_int, [C.c_void_p, C.POINTER(PgtRange), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t,
+                                    C.c_int, C.c_void_p]),
     "pgt_scan_sharded_workspace_bytes": (C.c_size_t, [C.c_void_p, C.c_int, C.c_uint32, C.c_uint32]),
     "pgt_scan_sharded": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(PgtColumns), C.c_int, C.c_void_p, C.POINTER(PgtWindows),
                                    C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p]),

@@ -515,6 +515,25 @@ __global__ void __launch_bounds__(256, 4) k_units_het_vec(DevPlan P, const int8_
 	}
 }
 
+// bp mode: the first site at or after global bp entry e of chromosome c (e inside the axis), as an index relative to
+// the columns' element 0: a lower_bound of e's 1-based position in chromosome c's slice of `pos`, clipped to the
+// `ndata` sites this call holds.
+__device__ __forceinline__ uint64_t bp_entry_site(const DevPlan& P, const uint32_t* __restrict__ pos, uint64_t ndata, uint32_t c, uint64_t e) {
+	const uint32_t p = (uint32_t)(e - P.off[c]) + 1u;
+	uint64_t lo = P.site_off[c], hi = P.site_off[c + 1];
+	if (lo < P.site_origin) lo = P.site_origin;
+	if (hi > P.site_origin + ndata) hi = P.site_origin + ndata;
+	if (hi < lo) hi = lo;
+	while (lo < hi) {
+		const uint64_t mid = lo + ((hi - lo) >> 1);
+		if (__ldg(pos + (mid - P.site_origin)) < p) lo = mid + 1;
+		else hi = mid;
+	}
+	if (lo < P.site_origin) lo = P.site_origin;
+	if (lo > P.site_origin + ndata) lo = P.site_origin + ndata;
+	return lo - P.site_origin;
+}
+
 // bp mode: bounds[t] = index (relative to the columns' element 0) of the first site at or after
 // the first bp of unit unit_lo+t, t in [0, unit_hi-unit_lo]; the unit's bp -> (chromosome, pos) is
 // closed form, the site is a lower_bound in that chromosome's slice of `pos`.
@@ -526,28 +545,61 @@ __global__ void __launch_bounds__(256) k_bp_bounds(DevPlan P, const uint32_t* __
 		uint64_t res;
 		if (j >= P.nunits_total) {
 			res = P.site_off[P.ncontig];
+			if (res < P.site_origin) res = P.site_origin;
+			if (res > P.site_origin + ndata) res = P.site_origin + ndata;
+			res -= P.site_origin;
 		} else {
 			const pgt_seg sg = P.segs[find_seg<true>(P, j)];
 			uint64_t st;
 			pgt_unit_range(P.g, sg.nsites, j - sg.unit_base, &st);
 			const uint64_t e = sg.site_base + st;  // global bp entry
-			const uint32_t c = find_contig(P.off, sg.first_contig, sg.ncontig, e);
-			const uint32_t p = (uint32_t)(e - P.off[c]) + 1u;  // 1-based position on chromosome c
-			uint64_t lo = P.site_off[c], hi = P.site_off[c + 1];
-			// clip to the sites this call holds
-			if (lo < P.site_origin) lo = P.site_origin;
-			if (hi > P.site_origin + ndata) hi = P.site_origin + ndata;
-			if (hi < lo) hi = lo;
-			while (lo < hi) {
-				const uint64_t mid = lo + ((hi - lo) >> 1);
-				if (__ldg(pos + (mid - P.site_origin)) < p) lo = mid + 1;
-				else hi = mid;
-			}
-			res = lo;
+			res = bp_entry_site(P, pos, ndata, find_contig(P.off, sg.first_contig, sg.ncontig, e), e);
 		}
-		if (res < P.site_origin) res = P.site_origin;
-		if (res > P.site_origin + ndata) res = P.site_origin + ndata;
-		bounds[t] = res - P.site_origin;
+		bounds[t] = res;
+	}
+}
+
+// bp mode, pgt_scan_bp_sites: the number of sites on the entries of every window [win_lo, win_hi) -- the difference of
+// the lower bounds of its first entry and of the entry after its last, the same searches k_bp_bounds makes for the
+// units at the window's two edges.  Also the position check: the first and last site this call holds of every
+// chromosome must lie on the chromosome (1 <= pos <= length); *bad receives the smallest global index of a site that
+// does not (left as it is when all do).
+__global__ void __launch_bounds__(256) k_bp_sites(DevPlan P, const uint32_t* __restrict__ pos, uint64_t ndata, uint32_t* __restrict__ nsites,
+                                                  unsigned long long* __restrict__ bad) {
+	const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
+	const uint64_t t0 = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+	const uint64_t axis_end = P.off[P.ncontig];
+	uint32_t si = 0xffffffffu;
+	pgt_seg sg;
+	sg.win_base = 0;
+	sg.nwin = 0;
+	for (uint64_t w = P.win_lo + t0; w < P.win_hi; w += stride) {
+		if (si == 0xffffffffu || w - sg.win_base >= sg.nwin) {
+			si = find_seg<false>(P, w);
+			sg = P.segs[si];
+		}
+		uint64_t fs;
+		const uint32_t n = pgt_window_sites(P.g, sg, w - sg.win_base, &fs);
+		const uint64_t e0 = sg.site_base + fs, e1 = e0 + n;
+		const uint64_t s0 = bp_entry_site(P, pos, ndata, find_contig(P.off, sg.first_contig, sg.ncontig, e0), e0);
+		uint64_t s1;
+		if (e1 >= axis_end) {
+			s1 = P.site_off[P.ncontig];
+			s1 = (s1 < P.site_origin ? P.site_origin : (s1 > P.site_origin + ndata ? P.site_origin + ndata : s1)) - P.site_origin;
+		} else {
+			s1 = bp_entry_site(P, pos, ndata, find_contig(P.off, 0, P.ncontig, e1), e1);
+		}
+		PGT_CHECK(s0 <= s1 && s1 <= ndata);
+		nsites[w - P.win_lo] = (uint32_t)(s1 - s0);
+	}
+	for (uint64_t c = t0; c < P.ncontig; c += stride) {
+		uint64_t lo = P.site_off[c], hi = P.site_off[c + 1];
+		if (lo < P.site_origin) lo = P.site_origin;
+		if (hi > P.site_origin + ndata) hi = P.site_origin + ndata;
+		if (hi <= lo) continue;
+		const uint64_t len = P.off[c + 1] - P.off[c];
+		if (__ldg(pos + (lo - P.site_origin)) < 1u) atomicMin(bad, (unsigned long long)lo);
+		else if (__ldg(pos + (hi - 1 - P.site_origin)) > len) atomicMin(bad, (unsigned long long)(hi - 1));
 	}
 }
 

@@ -1220,6 +1220,24 @@ static int scan_host(const Scan& s) {
 	return PGT_OK;
 }
 
+// The device view of a plan whose tables were uploaded to `segs` / `off` of a workspace (or are resident: bound), with
+// bp mode's site offsets at `site_off`; the unit, window and site ranges are the caller's to set.
+static DevPlan dev_plan(const pgt_plan* plan, const char* segs, const char* off, const char* site_off) {
+	DevPlan P;
+	memset(&P, 0, sizeof(P));
+	const bool resident = plan->d_tables != nullptr;
+	P.g = plan->g;
+	P.segs = resident ? (const pgt_seg*)plan->d_tables : (const pgt_seg*)segs;
+	P.off = resident ? (const uint64_t*)(plan->d_tables + align_up(plan->segs.size() * sizeof(pgt_seg), 256)) : (const uint64_t*)off;
+	P.site_off = (const uint64_t*)site_off;
+	P.nseg = (uint32_t)plan->segs.size();
+	P.ncontig = (uint32_t)plan->off.size() - 1;
+	P.nunits_total = plan->nunits;
+	P.col_elems = ~0ull;
+	P.mode = (int)plan->mode;
+	return P;
+}
+
 template <class Stat>
 static int run_scan(const pgt_plan* plan, const pgt_range* range, pgt_stat stat, const pgt_columns* cols, int minind,
                     const uint64_t* site_offsets, const pgt_windows* out, void* workspace, size_t workspace_bytes, pgt_mem mem,
@@ -1233,7 +1251,6 @@ static int run_scan(const pgt_plan* plan, const pgt_range* range, pgt_stat stat,
 	if (!workspace) return pgt_set_error(PGT_ERR_ARGS, "workspace is NULL");
 	if (workspace_bytes < L.total) return pgt_set_error(PGT_ERR_NOMEM, "workspace too small, see pgt_scan_workspace_bytes");
 	const bool bp = plan->mode == PGT_MODE_BP;
-	if (bp && stat != PGT_STAT_DXY) return pgt_set_error(PGT_ERR_ARGS, "PGT_MODE_BP plans are for PGT_STAT_DXY only");
 	if (bp && (!site_offsets || !cols->pos)) return pgt_set_error(PGT_ERR_ARGS, "bp mode needs site_offsets and pos");
 	const uint64_t nunits = L.u_hi - L.u_lo;
 	if (nunits == 0 && L.w_hi == L.w_lo) return PGT_OK;  // empty input / empty shard: nothing to read or write
@@ -1256,20 +1273,12 @@ static int run_scan(const pgt_plan* plan, const pgt_range* range, pgt_stat stat,
 	if (bp) PGT_CUDA(cudaMemcpyAsync(ws + L.siteoff_off, site_offsets, off_bytes, cudaMemcpyHostToDevice, st));
 
 	DevPlan& P = s.P;
-	P.g = plan->g;
-	P.segs = resident ? (const pgt_seg*)plan->d_tables : (const pgt_seg*)(ws + L.segs_off);
-	P.off = resident ? (const uint64_t*)(plan->d_tables + align_up(seg_bytes, 256)) : (const uint64_t*)(ws + L.off_off);
-	P.site_off = bp ? (const uint64_t*)(ws + L.siteoff_off) : nullptr;
-	P.nseg = (uint32_t)plan->segs.size();
-	P.ncontig = (uint32_t)plan->off.size() - 1;
+	P = dev_plan(plan, ws + L.segs_off, ws + L.off_off, bp ? ws + L.siteoff_off : nullptr);
 	P.unit_lo = L.u_lo;
 	P.unit_hi = L.u_hi;
 	P.win_lo = L.w_lo;
 	P.win_hi = L.w_hi;
 	P.site_origin = L.origin;
-	P.nunits_total = plan->nunits;
-	P.col_elems = ~0ull;
-	P.mode = (int)plan->mode;
 
 	s.ndata = 0;
 	if (bp) {
@@ -1325,4 +1334,113 @@ extern "C" int pgt_scan_dxy(const pgt_plan* plan, const pgt_range* range, const 
 extern "C" int pgt_scan_fused(const pgt_plan* plan, const pgt_range* range, const pgt_columns* cols, int minind,
                               const pgt_windows* out, void* workspace, size_t workspace_bytes, pgt_mem mem, void* stream) {
 	return pgt_scan(plan, range, PGT_STAT_FUSED, cols, minind, nullptr, out, workspace, workspace_bytes, mem, stream);
+}
+
+// ---- sites per bp window (pgt_scan_bp_sites): plan tables and bp site offsets in the workspace, one 8-byte slot for the
+// position check, and in host mode the positions of the chromosomes the windows touch plus the staged counts.
+struct BpSitesLayout {
+	uint64_t w_lo, w_hi, origin, ndata;
+	uint64_t s_lo, s_hi;  // host mode: global sites staged
+	size_t segs_off, off_off, siteoff_off, flag_off, pos_off, rows_off, total;
+};
+
+static int bp_sites_layout(const pgt_plan* plan, const pgt_range* range, const uint64_t* site_offsets, pgt_mem mem, BpSitesLayout* L) {
+	if (!plan) return pgt_set_error(PGT_ERR_ARGS, "plan is NULL");
+	if (plan->mode != PGT_MODE_BP) return pgt_set_error(PGT_ERR_ARGS, "pgt_scan_bp_sites needs a PGT_MODE_BP plan");
+	if (mem != PGT_MEM_DEVICE && mem != PGT_MEM_HOST) return pgt_set_error(PGT_ERR_ARGS, "unknown memory space");
+	memset(L, 0, sizeof(*L));
+	L->w_hi = plan->nwin;
+	if (range) {
+		if (range->w_hi != 0 || range->w_lo != 0) {
+			L->w_lo = range->w_lo;
+			L->w_hi = range->w_hi;
+		}
+		L->origin = range->site_origin;
+	}
+	if (L->w_lo > L->w_hi || L->w_hi > plan->nwin) return pgt_set_error(PGT_ERR_ARGS, "window range out of bounds");
+	const uint32_t nc = (uint32_t)plan->off.size() - 1;
+	if (site_offsets) {
+		if (site_offsets[nc] < L->origin) return pgt_set_error(PGT_ERR_ARGS, "site_origin beyond the last site");
+		L->ndata = (range && range->site_count) ? range->site_count : site_offsets[nc] - L->origin;
+	}
+	const uint64_t nwin = L->w_hi - L->w_lo;
+	if (mem == PGT_MEM_HOST && nwin) {
+		if (!site_offsets) return pgt_set_error(PGT_ERR_ARGS, "host-memory pgt_scan_bp_sites needs site_offsets");
+		uint64_t e0, e1;
+		pgt_plan_window(plan, L->w_lo, &e0, nullptr, nullptr);
+		pgt_plan_window(plan, L->w_hi - 1, nullptr, &e1, nullptr);
+		L->s_lo = std::max(site_offsets[pgt_plan_contig_of(plan, e0)], L->origin);
+		L->s_hi = std::max(L->s_lo, std::min(site_offsets[pgt_plan_contig_of(plan, e1) + 1], L->origin + L->ndata));
+	}
+	size_t o = 0;
+	L->segs_off = o;
+	o += align_up(plan->segs.size() * sizeof(pgt_seg) + 8, 256);
+	L->off_off = o;
+	o += align_up(plan->off.size() * sizeof(uint64_t), 256);
+	L->siteoff_off = o;
+	o += align_up(plan->off.size() * sizeof(uint64_t), 256);
+	L->flag_off = o;
+	o += 256;
+	L->pos_off = o;
+	if (mem == PGT_MEM_HOST) o += align_up((size_t)(L->s_hi - L->s_lo) * sizeof(uint32_t), 256);
+	L->rows_off = o;
+	if (mem == PGT_MEM_HOST) o += align_up((size_t)nwin * sizeof(uint32_t), 256);
+	L->total = o + 256;
+	return PGT_OK;
+}
+
+extern "C" size_t pgt_scan_bp_sites_workspace_bytes(const pgt_plan* plan, const pgt_range* range, const uint64_t* site_offsets, pgt_mem mem) {
+	BpSitesLayout L;
+	if (bp_sites_layout(plan, range, site_offsets, mem, &L) != PGT_OK) return 0;
+	return L.total;
+}
+
+extern "C" int pgt_scan_bp_sites(const pgt_plan* plan, const pgt_range* range, const uint32_t* pos, const uint64_t* site_offsets,
+                                 uint32_t* nsites_data, void* workspace, size_t workspace_bytes, pgt_mem mem, void* stream) {
+	if (!plan || !pos || !site_offsets || !nsites_data)
+		return pgt_set_error(PGT_ERR_ARGS, "pgt_scan_bp_sites: plan, pos, site_offsets and nsites_data must not be NULL");
+	int ndev = 0;
+	if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0)
+		return pgt_set_error(PGT_ERR_CUDA, "no usable CUDA device (libpgtscan has no CPU fallback)");
+	BpSitesLayout L;
+	PGT_TRY(bp_sites_layout(plan, range, site_offsets, mem, &L));
+	if (!workspace) return pgt_set_error(PGT_ERR_ARGS, "workspace is NULL");
+	if (workspace_bytes < L.total) return pgt_set_error(PGT_ERR_NOMEM, "workspace too small, see pgt_scan_bp_sites_workspace_bytes");
+	const uint64_t nwin = L.w_hi - L.w_lo;
+	if (nwin == 0) return PGT_OK;
+	cudaStream_t st = (cudaStream_t)stream;
+	char* ws = (char*)workspace;
+	const size_t seg_bytes = plan->segs.size() * sizeof(pgt_seg), off_bytes = plan->off.size() * sizeof(uint64_t);
+	if (!plan->d_tables) {
+		if (seg_bytes) PGT_CUDA(cudaMemcpyAsync(ws + L.segs_off, plan->segs.data(), seg_bytes, cudaMemcpyHostToDevice, st));
+		PGT_CUDA(cudaMemcpyAsync(ws + L.off_off, plan->off.data(), off_bytes, cudaMemcpyHostToDevice, st));
+	}
+	PGT_CUDA(cudaMemcpyAsync(ws + L.siteoff_off, site_offsets, off_bytes, cudaMemcpyHostToDevice, st));
+	unsigned long long* d_bad = (unsigned long long*)(ws + L.flag_off);
+	PGT_CUDA(cudaMemsetAsync(d_bad, 0xff, sizeof(*d_bad), st));
+	DevPlan P = dev_plan(plan, ws + L.segs_off, ws + L.off_off, ws + L.siteoff_off);
+	P.win_lo = L.w_lo;
+	P.win_hi = L.w_hi;
+	const uint32_t* dpos = pos;
+	uint32_t* drows = nsites_data;
+	uint64_t ndata = L.ndata;
+	P.site_origin = L.origin;
+	if (mem == PGT_MEM_HOST) {  // the positions of the chromosomes the windows touch, staged once
+		ndata = L.s_hi - L.s_lo;
+		P.site_origin = L.s_lo;
+		dpos = (const uint32_t*)(ws + L.pos_off);
+		drows = (uint32_t*)(ws + L.rows_off);
+		if (ndata) PGT_CUDA(cudaMemcpyAsync(ws + L.pos_off, pos + (L.s_lo - L.origin), ndata * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
+	}
+	P.col_elems = ndata;
+	k_bp_sites<<<capped_grid((std::max<uint64_t>(nwin, P.ncontig) + 255) / 256), 256, 0, st>>>(P, dpos, ndata, drows, d_bad);
+	g_launches++;
+	PGT_CUDA(cudaGetLastError());
+	if (mem == PGT_MEM_HOST) PGT_CUDA(cudaMemcpyAsync(nsites_data, drows, nwin * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+	unsigned long long bad = 0;
+	PGT_CUDA(cudaMemcpyAsync(&bad, d_bad, sizeof(bad), cudaMemcpyDeviceToHost, st));
+	PGT_CUDA(cudaStreamSynchronize(st));
+	if (bad != ~0ull)
+		return pgt_set_error(PGT_ERR_INPUT, "site " + std::to_string(bad) + " lies outside its chromosome (bp positions run from 1 to the chromosome length)");
+	return PGT_OK;
 }

@@ -265,18 +265,21 @@ def scan_sharded(plan, stat, cols, devices, minind=1, site_offsets=None, out=Non
     return out
 
 
-def fst_window(plan, pos, a, b, **kw):
-    """Sliding-window FST = sum(a)/sum(b) (/root/reference/fstWindow.cpp:69-107).
+def fst_window(plan, pos, a, b, site_offsets=None, **kw):
+    """Sliding-window FST = sum(a)/sum(b) (/root/reference/fstWindow.cpp:69-107).  plan mode 'sites' = windows of
+    sites as fstWindow; 'bp' = fixed-bp windows over the sites whose positions fall on them (then site_offsets =
+    cumulative sites per chromosome, and nsites counts bp: see bp_window_sites).
     Returns label, start_pos, end_pos, mid_pos, nsites, sum_a, sum_b, fst per window."""
-    return scan(plan, _cabi.PGT_STAT_FST, dict(pos=pos, a=a, b=b), **kw)
+    return scan(plan, _cabi.PGT_STAT_FST, dict(pos=pos, a=a, b=b), site_offsets=site_offsets, **kw)
 
 
-def het_window(plan, pos, geno, **kw):
+def het_window(plan, pos, geno, site_offsets=None, **kw):
     """Sliding-window heterozygosity = #(g==1) / #(g>=0) (/root/reference/hetWindow.cpp:66-105).
     The counts are integers, so any unit size gives identical results; build the plan with
-    ``unit_sites=4096`` for the fastest scan of the 1-byte genotype column.
+    ``unit_sites=4096`` for the fastest scan of the 1-byte genotype column.  plan mode and site_offsets as for
+    fst_window.
     Returns label, start_pos, end_pos, mid_pos, nsites, nhet, nonmissing, het per window."""
-    return scan(plan, _cabi.PGT_STAT_HET, dict(pos=pos, geno=geno), **kw)
+    return scan(plan, _cabi.PGT_STAT_HET, dict(pos=pos, geno=geno), site_offsets=site_offsets, **kw)
 
 
 def dxy_window(plan, pos, f1, f2, n1, n2, minind=1, site_offsets=None, **kw):
@@ -289,10 +292,42 @@ def dxy_window(plan, pos, f1, f2, n1, n2, minind=1, site_offsets=None, **kw):
                 site_offsets=site_offsets, **kw)
 
 
-def fused_window(plan, pos, a, b, geno, f1, f2, n1, n2, minind=1, **kw):
-    """fst + dxy + het over one site axis in a single pass (BASELINE config 5)."""
+def fused_window(plan, pos, a, b, geno, f1, f2, n1, n2, minind=1, site_offsets=None, **kw):
+    """fst + dxy + het over one site axis in a single pass (BASELINE config 5); plan mode and site_offsets as for
+    dxy_window.  Each statistic equals its single scan bit for bit."""
     return scan(plan, _cabi.PGT_STAT_FUSED, dict(pos=pos, a=a, b=b, geno=geno, f1=f1, f2=f2, n1=n1, n2=n2),
-                minind=minind, **kw)
+                minind=minind, site_offsets=site_offsets, **kw)
+
+
+def bp_window_sites(plan, pos, site_offsets, window_range=None, site_origin=0, site_count=0, out=None, device=None):
+    """Sites per window of a bp plan (pgt_scan_bp_sites): the number of sites whose positions fall on each window's
+    bp, for the rows of a scan over the same plan and window range (whose ``nsites`` counts bp).  `pos` a CUDA
+    tensor (PGT_MEM_DEVICE: enqueued on the current stream, returns a CUDA uint32 tensor) or a numpy array
+    (PGT_MEM_HOST: returns a numpy uint32 array).  Raises PgtError (PGT_ERR_INPUT) when a site lies outside its
+    chromosome; the call waits for the stream to report that."""
+    torch = _torch()
+    lib = plan._lib
+    on_device = isinstance(pos, torch.Tensor) and pos.is_cuda
+    ptrs, keep = _columns(dict(pos=pos), ("pos",), ("pos",), on_device)
+    r = _range(plan, window_range, site_origin, site_count)
+    so = np.ascontiguousarray(site_offsets, dtype=np.uint64)
+    nrows = r.w_hi - r.w_lo
+    dev = pos.device if on_device else torch.device(device if device is not None else f"cuda:{torch.cuda.current_device()}")
+    if out is None:
+        out = torch.empty(nrows, dtype=torch.uint32, device=dev) if on_device else np.empty(nrows, np.uint32)
+    mem = _cabi.PGT_MEM_DEVICE if on_device else _cabi.PGT_MEM_HOST
+    if on_device:
+        plan.bind(dev)
+    elif plan._bound is not None and plan._bound[0] != dev:
+        raise ValueError(f"plan is bound to {plan._bound[0]}, scan requested on {dev}")
+    ws = torch.empty(int(lib.pgt_scan_bp_sites_workspace_bytes(plan.handle, C.byref(r), so.ctypes.data, mem)), dtype=torch.uint8,
+                     device=dev)
+    with torch.cuda.device(dev):
+        stream = torch.cuda.current_stream(dev).cuda_stream
+        check(lib.pgt_scan_bp_sites(plan.handle, C.byref(r), ptrs["pos"], so.ctypes.data,
+                                    out.data_ptr() if on_device else out.ctypes.data, ws.data_ptr(), ws.numel(), mem,
+                                    C.c_void_p(stream)))
+    return out
 
 
 # ---- synthetic inputs (device) -------------------------------------------------------------
