@@ -108,6 +108,42 @@ int pgt_scan_extreme(const pgt_xplan* plan, const pgt_range* range, pgt_xstat st
 int pgt_scan_extreme_sharded(const pgt_xplan* plan, pgt_xstat stat, double cutoff, const uint32_t* pos, const double* score,
                              const pgt_xwindows* out, const int* devices, uint32_t ndev);
 
+/* ---- the same statistics over the windows of a pgt_plan (pgt_scan.h): sliding site or bp windows whose rows line up
+ * row for row with pgt_scan's fst / het / dxy / fused rows of the same plan and range.
+ *
+ * Window w reduces the sites pgt_scan reduces for it: sites first..last in site mode; in bp mode the sites whose
+ * positions fall on the window's bp (`site_offsets` = cumulative sites per chromosome, as for pgt_scan).  Per row:
+ *   key       PGT_XSTAT_IHS |v|; PGT_XSTAT_XPEHH v (cutoff >= 0) or -v (cutoff < 0); a NaN key counts as -inf
+ *   big       IHS |v| > cutoff; XPEHH v > cutoff, or v < cutoff when cutoff < 0 (strict; NaN is never big)
+ *   ext_site  the smallest global site index among the window's sites of largest key (a non-empty window always
+ *             has one, even when every score is NaN); ext_value = score[ext_site], ext_pos = pos[ext_site]
+ *   nbig      big sites; nsites = the window's sites (in bp mode = pgt_scan_bp_sites); prop = nbig / nsites
+ *   empty     (bp windows without sites) ext_value = prop = NaN, ext_pos = 0, ext_site = UINT64_MAX, nbig = nsites = 0
+ * `rows` (may be NULL) receives the geometry pgt_scan writes for the same plan: only label, start_pos, end_pos,
+ * mid_pos and nsites (bp: counts bp) may be set, anything else is PGT_ERR_ARGS.  These rows do not reproduce
+ * ihsWindow's own window layout or its NaN-first-site quirk (that is pgt_scan_extreme).
+ *
+ * `range`, its site_origin / site_count, `site_offsets` and `mem` mean what they mean for pgt_scan; column pointers
+ * address element range->site_origin.  `pos` is required in bp mode and for ext_pos, start_pos, end_pos and mid_pos.
+ * Errors: those of pgt_scan, PGT_ERR_ARGS for an unknown `stat` or a NULL `score`, PGT_ERR_INPUT in bp mode when a
+ * site lies outside its chromosome (a device-memory bp scan waits for its stream to report that).
+ *
+ * Kernel path (results do not depend on it): W = S = 1 in site mode maps every site to its row (one kernel); all
+ * other plans take pgt_scan's units path -- level 1 per-unit extremes (direct or TMA-tiled, unit-start table, bp
+ * unit bounds), level 2 warp / thread per window, or scan mode (block prefix / suffix, exact for a maximum) for
+ * fine steps -- under the same pgt_tune knobs.  The sliding tile (PGT_PATH_SLIDE) is not used.  The level 1 / 2
+ * timings appear under pgt_profile_read. */
+size_t pgt_scan_plan_extreme_workspace_bytes(const pgt_plan* plan, const pgt_range* range, pgt_mem mem);
+int pgt_scan_plan_extreme(const pgt_plan* plan, const pgt_range* range, pgt_xstat stat, double cutoff, const uint32_t* pos,
+                          const double* score, const uint64_t* site_offsets, const pgt_windows* rows, const pgt_xwindows* out,
+                          void* workspace, size_t workspace_bytes, pgt_mem mem, void* stream);
+/* Host columns over ALL sites, several GPUs of one process: windows cut by pgt_plan_shard, shard i on devices[i]
+ * (see pgt_scan_sharded); scratch is allocated by the call; `rows` / `out` are host arrays of pgt_plan_num_windows
+ * elements.  Bit-identical for any device list, a device listed more than once included. */
+int pgt_scan_plan_extreme_sharded(const pgt_plan* plan, pgt_xstat stat, double cutoff, const uint32_t* pos, const double* score,
+                                  const uint64_t* site_offsets, const pgt_windows* rows, const pgt_xwindows* out, const int* devices,
+                                  uint32_t ndev);
+
 /* Synthetic score column of global sites [site0, site0+n): ~N(0,1) with heavy ties removed
  * (counter-based, bit-identical to the CPU twin in pgt_synth.h).  Device pointer. */
 int pgt_synth_score(uint64_t seed, uint64_t site0, uint64_t n, double* score, void* stream);

@@ -134,6 +134,11 @@ PROTOTYPES = {
                                    C.POINTER(PgtXWindows), C.c_void_p, C.c_size_t, C.c_int, C.c_void_p]),
     "pgt_scan_extreme_sharded": (C.c_int, [C.c_void_p, C.c_int, C.c_double, C.c_void_p, C.c_void_p, C.POINTER(PgtXWindows), C.c_void_p,
                                            C.c_uint32]),
+    "pgt_scan_plan_extreme_workspace_bytes": (C.c_size_t, [C.c_void_p, C.POINTER(PgtRange), C.c_int]),
+    "pgt_scan_plan_extreme": (C.c_int, [C.c_void_p, C.POINTER(PgtRange), C.c_int, C.c_double, C.c_void_p, C.c_void_p, C.c_void_p,
+                                        C.POINTER(PgtWindows), C.POINTER(PgtXWindows), C.c_void_p, C.c_size_t, C.c_int, C.c_void_p]),
+    "pgt_scan_plan_extreme_sharded": (C.c_int, [C.c_void_p, C.c_int, C.c_double, C.c_void_p, C.c_void_p, C.c_void_p,
+                                                C.POINTER(PgtWindows), C.POINTER(PgtXWindows), C.c_void_p, C.c_uint32]),
     "pgt_synth_score": (C.c_int, [C.c_uint64, C.c_uint64, C.c_uint64, C.c_void_p, C.c_void_p]),
     "pgt_profile_read_extreme": (C.c_int, [C.POINTER(C.c_double), _u64p, C.POINTER(C.c_double), _u64p]),
 }

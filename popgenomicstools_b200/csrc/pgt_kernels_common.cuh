@@ -1,4 +1,4 @@
-// pgt_kernels_common.cuh -- device-side plan, search helpers, the PGT_BOUNDS check and the four statistics (what one site contributes, how partials combine, what a window row holds)
+// pgt_kernels_common.cuh -- device-side plan, search helpers, the PGT_BOUNDS check and the statistics (what one site contributes, how partials combine, what a window row holds)
 // Part of the one translation unit pgt_scan.cu (device code only; included from there, in this order:
 // pgt_kernels_common.cuh, pgt_level1.cuh, pgt_level2.cuh, pgt_slide.cuh).
 #ifndef PGT_KERNELS_COMMON_CUH
@@ -32,7 +32,9 @@ struct Cols {
 	const double* f2;
 	const int32_t* n1;
 	const int32_t* n2;
+	const double* score;  // extreme scan over a window plan (XStat)
 	int minind;
+	double cutoff;  // XStat
 };
 
 struct DevPlan {
@@ -91,10 +93,13 @@ __device__ __forceinline__ uint32_t shfl_xor_u32(uint32_t v, int m) { return __s
 //
 // A Stat describes: the per-site record loaded from the columns (Site), the unit partial (Acc,
 // stored as-is in the unit array), how one site is folded into a lane's partial (the per-site
-// statistic), the combine used by the butterflies, and the window epilogue.
+// statistic; fold also gets dxyWindow's -minind, the extreme scan's cutoff and the site's global
+// index, which only XStat reads), the combine used by the butterflies, and the window epilogue
+// into the rows of type Out.
 
 // --- fstWindow: asum += a; bsum += b (fstWindow.cpp:80-83); fst = bsum != 0 ? asum/bsum : 0 (:85)
 struct FstStat {
+	typedef pgt_windows Out;
 	struct Acc {
 		double a, b;
 	};
@@ -107,7 +112,7 @@ struct FstStat {
 	static __device__ __forceinline__ Site load_tile(const char* const* cp, uint32_t i) {
 		return Site{((const double*)cp[0])[i], ((const double*)cp[1])[i]};
 	}
-	static __device__ __forceinline__ void fold(Acc& acc, const Site& s, int) {
+	static __device__ __forceinline__ void fold(Acc& acc, const Site& s, int, double, uint64_t) {
 		acc.a = __dadd_rn(acc.a, s.a);
 		acc.b = __dadd_rn(acc.b, s.b);
 	}
@@ -125,6 +130,7 @@ struct FstStat {
 
 // --- hetWindow: nonmissing += (g >= 0); nhet += (g == 1) (hetWindow.cpp:77-82); h = nhet/nonmissing (:84)
 struct HetStat {
+	typedef pgt_windows Out;
 	struct Acc {
 		uint32_t nonmissing, nhet;
 	};
@@ -134,7 +140,7 @@ struct HetStat {
 	static __device__ __forceinline__ Acc zero() { return Acc{0u, 0u}; }
 	static __device__ __forceinline__ Site load(const Cols& c, uint64_t i) { return Site{(int)__ldg(c.g + i)}; }
 	static __device__ __forceinline__ Site load_tile(const char* const* cp, uint32_t i) { return Site{(int)((const int8_t*)cp[0])[i]}; }
-	static __device__ __forceinline__ void fold(Acc& acc, const Site& s, int) {
+	static __device__ __forceinline__ void fold(Acc& acc, const Site& s, int, double, uint64_t) {
 		acc.nonmissing += (s.g >= 0);
 		acc.nhet += (s.g == 1);
 	}
@@ -160,6 +166,7 @@ __device__ __forceinline__ double dxy_site_value(double f1, double f2, int n1, i
 	return (n1 >= minind && n2 >= minind) ? __dadd_rn(__dmul_rn(f1, __dsub_rn(1.0, f2)), __dmul_rn(f2, __dsub_rn(1.0, f1))) : -9.0;
 }
 struct DxyStat {
+	typedef pgt_windows Out;
 	struct Acc {
 		double dxy;
 		uint32_t neff, nskip;
@@ -175,7 +182,7 @@ struct DxyStat {
 	static __device__ __forceinline__ Site load_tile(const char* const* cp, uint32_t i) {
 		return Site{((const double*)cp[0])[i], ((const double*)cp[1])[i], ((const int32_t*)cp[2])[i], ((const int32_t*)cp[3])[i]};
 	}
-	static __device__ __forceinline__ void fold(Acc& acc, const Site& s, int minind) {
+	static __device__ __forceinline__ void fold(Acc& acc, const Site& s, int minind, double, uint64_t) {
 		const double v = dxy_site_value(s.f1, s.f2, s.n1, s.n2, minind);
 		if (v >= 0.0) {
 			acc.dxy = __dadd_rn(acc.dxy, v);
@@ -201,6 +208,7 @@ struct DxyStat {
 
 // --- fused fst + dxy + het over one site axis (BASELINE config 5): one pass, 41 B/site
 struct FusedStat {
+	typedef pgt_windows Out;
 	struct Acc {
 		FstStat::Acc fst;
 		DxyStat::Acc dxy;
@@ -217,10 +225,10 @@ struct FusedStat {
 	static __device__ __forceinline__ Site load_tile(const char* const* cp, uint32_t i) {
 		return Site{FstStat::load_tile(cp, i), DxyStat::load_tile(cp + 2, i), HetStat::load_tile(cp + 6, i)};
 	}
-	static __device__ __forceinline__ void fold(Acc& acc, const Site& s, int minind) {
-		FstStat::fold(acc.fst, s.fst, minind);
-		DxyStat::fold(acc.dxy, s.dxy, minind);
-		HetStat::fold(acc.het, s.het, minind);
+	static __device__ __forceinline__ void fold(Acc& acc, const Site& s, int minind, double, uint64_t) {
+		FstStat::fold(acc.fst, s.fst, minind, 0.0, 0);
+		DxyStat::fold(acc.dxy, s.dxy, minind, 0.0, 0);
+		HetStat::fold(acc.het, s.het, minind, 0.0, 0);
 	}
 	static __device__ __forceinline__ void add(Acc& acc, const Acc& o) {
 		FstStat::add(acc.fst, o.fst);
@@ -240,6 +248,7 @@ struct FusedStat {
 // --- fst + het together: what one of the two crews of the fused sliding tile computes (pgt_slide.cuh); every
 // component is folded, combined and emitted exactly as by FstStat / HetStat alone.  Staged columns as FusedStat.
 struct FstHetStat {
+	typedef pgt_windows Out;
 	struct Acc {
 		FstStat::Acc fst;
 		HetStat::Acc het;
@@ -252,9 +261,9 @@ struct FstHetStat {
 	static __device__ __forceinline__ Site load_tile(const char* const* cp, uint32_t i) {
 		return Site{FstStat::load_tile(cp, i), HetStat::load_tile(cp + 6, i)};
 	}
-	static __device__ __forceinline__ void fold(Acc& acc, const Site& s, int minind) {
-		FstStat::fold(acc.fst, s.fst, minind);
-		HetStat::fold(acc.het, s.het, minind);
+	static __device__ __forceinline__ void fold(Acc& acc, const Site& s, int minind, double, uint64_t) {
+		FstStat::fold(acc.fst, s.fst, minind, 0.0, 0);
+		HetStat::fold(acc.het, s.het, minind, 0.0, 0);
 	}
 	static __device__ __forceinline__ void add(Acc& acc, const Acc& o) {
 		FstStat::add(acc.fst, o.fst);
@@ -265,6 +274,86 @@ struct FstHetStat {
 		HetStat::emit(out, o, acc.het);
 	}
 };
+
+// --- most extreme score over a window plan (pgt_scan_plan_extreme, ihsWindow / xpehhWindow statistics): the first
+// site of largest key (|v|, v or -v; a NaN key is -inf), sites past the cutoff, sites.  The accumulator is a total
+// order on (key, -site) plus two counts, so every butterfly, tree, scan and shard order gives the same bits.
+enum { XMODE_ABS = 0, XMODE_MAX = 1, XMODE_MIN = 2 };
+
+// Rows of an extreme scan: the geometry columns of pgt_windows (same meanings), the pgt_xwindows columns
+// (xnsites = its nsites: score sites), and where ext_value / ext_pos are gathered from (score / pos[ext_site -
+// site_origin]).
+struct XRows {
+	uint32_t *label, *start_pos, *end_pos, *mid_pos, *nsites;
+	double* ext_value;
+	uint32_t* ext_pos;
+	uint64_t* ext_site;
+	uint32_t *nbig, *xnsites;
+	double* prop;
+	const double* score;
+	const uint32_t* pos;
+	uint64_t site_origin;
+};
+
+template <int MODE>
+struct XStat {
+	typedef XRows Out;
+	// The key of the extreme site rides in the partial, not its score: a lane's fold is then one compare and two
+	// selects on registers (the score is gathered once per window in the epilogue, as its position).
+	struct Acc {
+		double key;
+		uint64_t site;
+		uint32_t nbig, n;
+	};
+	struct Site {
+		double v;
+	};
+	static __device__ __forceinline__ double key(double v) {
+		const double k = MODE == XMODE_ABS ? fabs(v) : (MODE == XMODE_MAX ? v : -v);
+		return k != k ? -CUDART_INF : k;
+	}
+	// identity: key -inf ties with any real site's key at worst, and then the smaller index wins
+	static __device__ __forceinline__ Acc zero() { return Acc{-CUDART_INF, ~0ull, 0u, 0u}; }
+	static __device__ __forceinline__ Site load(const Cols& c, uint64_t i) { return Site{__ldg(c.score + i)}; }
+	static __device__ __forceinline__ Site load_tile(const char* const* cp, uint32_t i) { return Site{((const double*)cp[0])[i]}; }
+	// beyond the cutoff (strict; NaN never is)
+	static __device__ __forceinline__ bool big(double v, double cutoff) {
+		return MODE == XMODE_ABS ? fabs(v) > cutoff : (MODE == XMODE_MAX ? v > cutoff : v < cutoff);
+	}
+	static __device__ __forceinline__ void fold(Acc& acc, const Site& s, int, double cutoff, uint64_t site) {
+		const double k = key(s.v);
+		if (k > acc.key || (k == acc.key && site < acc.site)) {
+			acc.key = k;
+			acc.site = site;
+		}
+		acc.nbig += big(s.v, cutoff) ? 1u : 0u;
+		++acc.n;
+	}
+	static __device__ __forceinline__ void add(Acc& acc, const Acc& o) {
+		if (o.key > acc.key || (o.key == acc.key && o.site < acc.site)) {
+			acc.key = o.key;
+			acc.site = o.site;
+		}
+		acc.nbig += o.nbig;
+		acc.n += o.n;
+	}
+	static __device__ __forceinline__ Acc shfl_xor(const Acc& v, int m) {
+		return Acc{shfl_xor_f64(v.key, m), (uint64_t)__shfl_xor_sync(0xffffffffu, (unsigned long long)v.site, m), shfl_xor_u32(v.nbig, m),
+		           shfl_xor_u32(v.n, m)};
+	}
+	static __device__ __forceinline__ void emit(const XRows& out, uint64_t o, const Acc& acc) {
+		if (out.ext_value) out.ext_value[o] = acc.n ? __ldg(out.score + (acc.site - out.site_origin)) : CUDART_NAN;
+		if (out.ext_site) out.ext_site[o] = acc.site;
+		if (out.ext_pos) out.ext_pos[o] = acc.n ? __ldg(out.pos + (acc.site - out.site_origin)) : 0u;
+		if (out.nbig) out.nbig[o] = acc.nbig;
+		if (out.xnsites) out.xnsites[o] = acc.n;
+		if (out.prop) out.prop[o] = acc.n ? __ddiv_rn((double)acc.nbig, (double)acc.n) : CUDART_NAN;
+	}
+};
+template <class Stat>
+struct IsXStat : std::false_type {};
+template <int MODE>
+struct IsXStat<XStat<MODE>> : std::true_type {};
 
 template <class Stat>
 __device__ __forceinline__ typename Stat::Acc warp_butterfly(typename Stat::Acc acc) {

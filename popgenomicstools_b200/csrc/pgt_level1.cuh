@@ -44,9 +44,10 @@ __global__ void __launch_bounds__(256) k_units(DevPlan P, Cols cols, typename St
 				if (lane + 32u * t < len) v[t] = Stat::load(cols, i0 + 32u * t);
 #pragma unroll
 			for (int t = 0; t < UPL; ++t)
-				if (lane + 32u * t < len) Stat::fold(acc, v[t], cols.minind);
+				if (lane + 32u * t < len) Stat::fold(acc, v[t], cols.minind, cols.cutoff, P.site_origin + i0 + 32u * t);
 		} else {
-			for (uint32_t x = lane; x < len; x += 32u) Stat::fold(acc, Stat::load(cols, i0 + (x - lane)), cols.minind);
+			for (uint32_t x = lane; x < len; x += 32u)
+				Stat::fold(acc, Stat::load(cols, i0 + (x - lane)), cols.minind, cols.cutoff, P.site_origin + i0 + (x - lane));
 		}
 		acc = warp_butterfly<Stat>(acc);
 		if (lane == 0) units[j - P.unit_lo] = acc;
@@ -109,6 +110,7 @@ struct TileCfg {
 	uint32_t stage_bytes;
 	uint32_t nstages;      // 2..kTileMaxStages
 	int minind;
+	double cutoff;         // XStat
 	uint64_t valid_elems;  // elements every column holds from element 0 (bounds the aligned superset copies)
 };
 
@@ -413,7 +415,8 @@ __global__ void __launch_bounds__(kTileThreads, 1)
 				if constexpr (std::is_same<Stat, HetStat>::value && G == 32) {
 					het_unit_from_tile(acc, cp[0], rel, len, lane);
 				} else {
-					for (uint32_t x = gl; x < len; x += G) Stat::fold(acc, Stat::load_tile(cp, rel + x), tc.minind);
+					for (uint32_t x = gl; x < len; x += G)
+						Stat::fold(acc, Stat::load_tile(cp, rel + x), tc.minind, tc.cutoff, P.site_origin + s0 + rel + x);
 				}
 				acc = group_butterfly<Stat, G>(acc);
 				if (active && gl == 0) units[j - P.unit_lo] = acc;
@@ -559,6 +562,21 @@ __global__ void __launch_bounds__(256) k_bp_bounds(DevPlan P, const uint32_t* __
 	}
 }
 
+// bp mode: the first and last site this call holds of every chromosome must lie on the chromosome (1 <= pos <= length);
+// *bad receives the smallest global index of a site that does not (left as it is when all do).  Chromosomes t0, t0 + stride, ...
+__device__ __forceinline__ void bp_check_positions(const DevPlan& P, const uint32_t* __restrict__ pos, uint64_t ndata, uint64_t t0, uint64_t stride,
+                                                   unsigned long long* __restrict__ bad) {
+	for (uint64_t c = t0; c < P.ncontig; c += stride) {
+		uint64_t lo = P.site_off[c], hi = P.site_off[c + 1];
+		if (lo < P.site_origin) lo = P.site_origin;
+		if (hi > P.site_origin + ndata) hi = P.site_origin + ndata;
+		if (hi <= lo) continue;
+		const uint64_t len = P.off[c + 1] - P.off[c];
+		if (__ldg(pos + (lo - P.site_origin)) < 1u) atomicMin(bad, (unsigned long long)lo);
+		else if (__ldg(pos + (hi - 1 - P.site_origin)) > len) atomicMin(bad, (unsigned long long)(hi - 1));
+	}
+}
+
 // bp mode, pgt_scan_bp_sites: the number of sites on the entries of every window [win_lo, win_hi) -- the difference of
 // the lower bounds of its first entry and of the entry after its last, the same searches k_bp_bounds makes for the
 // units at the window's two edges.  Also the position check: the first and last site this call holds of every
@@ -592,15 +610,12 @@ __global__ void __launch_bounds__(256) k_bp_sites(DevPlan P, const uint32_t* __r
 		PGT_CHECK(s0 <= s1 && s1 <= ndata);
 		nsites[w - P.win_lo] = (uint32_t)(s1 - s0);
 	}
-	for (uint64_t c = t0; c < P.ncontig; c += stride) {
-		uint64_t lo = P.site_off[c], hi = P.site_off[c + 1];
-		if (lo < P.site_origin) lo = P.site_origin;
-		if (hi > P.site_origin + ndata) hi = P.site_origin + ndata;
-		if (hi <= lo) continue;
-		const uint64_t len = P.off[c + 1] - P.off[c];
-		if (__ldg(pos + (lo - P.site_origin)) < 1u) atomicMin(bad, (unsigned long long)lo);
-		else if (__ldg(pos + (hi - 1 - P.site_origin)) > len) atomicMin(bad, (unsigned long long)(hi - 1));
-	}
+	bp_check_positions(P, pos, ndata, t0, stride, bad);
+}
+
+// bp mode, the position check alone (pgt_scan_plan_extreme)
+__global__ void __launch_bounds__(256) k_bp_pos_check(DevPlan P, const uint32_t* __restrict__ pos, uint64_t ndata, unsigned long long* __restrict__ bad) {
+	bp_check_positions(P, pos, ndata, (uint64_t)blockIdx.x * blockDim.x + threadIdx.x, (uint64_t)gridDim.x * blockDim.x, bad);
 }
 
 #endif  // PGT_LEVEL1_CUH

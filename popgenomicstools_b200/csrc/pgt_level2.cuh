@@ -8,14 +8,84 @@
 
 template <class Stat>
 __device__ __forceinline__ void emit_window(const DevPlan& P, const pgt_seg& sg, uint64_t w, uint64_t k, const typename Stat::Acc& acc,
-                                            const uint32_t* __restrict__ pos, const pgt_windows& out, uint64_t o, bool have_edges = false,
+                                            const uint32_t* __restrict__ pos, const typename Stat::Out& out, uint64_t o, bool have_edges = false,
                                             uint32_t edge_start = 0, uint32_t edge_end = 0);
 
 // two batches of 32 rows of every output column, staged in shared memory so that a block writes its rows with
-// full-width stores (double-buffered: one barrier per batch)
-struct RowStage {
+// full-width stores (double-buffered: one barrier per batch).  staged(): rows of the same columns as `out`, pointing into
+// the stage; store(): rows [half, half + nrows) of the stage to rows [o - lane, ...) of `out`, column f by warp f % 8.
+template <class Out>
+struct RowStage;
+template <>
+struct RowStage<pgt_windows> {
 	uint32_t u[9][64];  // label, start_pos, end_pos, mid_pos, nsites, nhet, nonmissing, neffective, nskip
 	double d[5][64];    // sum_a, sum_b, fst, het, dxy
+	__device__ __forceinline__ pgt_windows staged(const pgt_windows& out) {
+		pgt_windows st;
+		st.label = out.label ? u[0] : nullptr;
+		st.start_pos = out.start_pos ? u[1] : nullptr;
+		st.end_pos = out.end_pos ? u[2] : nullptr;
+		st.mid_pos = out.mid_pos ? u[3] : nullptr;
+		st.nsites = out.nsites ? u[4] : nullptr;
+		st.nhet = out.nhet ? u[5] : nullptr;
+		st.nonmissing = out.nonmissing ? u[6] : nullptr;
+		st.neffective = out.neffective ? u[7] : nullptr;
+		st.nskip = out.nskip ? u[8] : nullptr;
+		st.sum_a = out.sum_a ? d[0] : nullptr;
+		st.sum_b = out.sum_b ? d[1] : nullptr;
+		st.fst = out.fst ? d[2] : nullptr;
+		st.het = out.het ? d[3] : nullptr;
+		st.dxy = out.dxy ? d[4] : nullptr;
+		st.dxy_global = nullptr;
+		return st;
+	}
+	__device__ __forceinline__ void store(const pgt_windows& out, uint32_t half, uint64_t o, uint32_t nrows, uint32_t wi, uint32_t lane) const {
+		uint32_t* const gu[9] = {out.label, out.start_pos, out.end_pos, out.mid_pos, out.nsites, out.nhet, out.nonmissing, out.neffective, out.nskip};
+		double* const gd[5] = {out.sum_a, out.sum_b, out.fst, out.het, out.dxy};
+#pragma unroll
+		for (int f = 0; f < 9; ++f)
+			if ((f & 7) == (int)wi && gu[f] && lane < nrows) gu[f][o] = u[f][half + lane];
+#pragma unroll
+		for (int f = 0; f < 5; ++f)
+			if (((f + 9) & 7) == (int)wi && gd[f] && lane < nrows) gd[f][o] = d[f][half + lane];
+	}
+};
+template <>
+struct RowStage<XRows> {
+	uint32_t u[8][64];  // label, start_pos, end_pos, mid_pos, nsites, ext_pos, nbig, xnsites
+	uint64_t s[64];     // ext_site
+	double d[2][64];    // ext_value, prop
+	__device__ __forceinline__ XRows staged(const XRows& out) {
+		XRows st;
+		st.label = out.label ? u[0] : nullptr;
+		st.start_pos = out.start_pos ? u[1] : nullptr;
+		st.end_pos = out.end_pos ? u[2] : nullptr;
+		st.mid_pos = out.mid_pos ? u[3] : nullptr;
+		st.nsites = out.nsites ? u[4] : nullptr;
+		st.ext_pos = out.ext_pos ? u[5] : nullptr;
+		st.nbig = out.nbig ? u[6] : nullptr;
+		st.xnsites = out.xnsites ? u[7] : nullptr;
+		st.ext_site = out.ext_site ? s : nullptr;
+		st.ext_value = out.ext_value ? d[0] : nullptr;
+		st.prop = out.prop ? d[1] : nullptr;
+		st.score = out.score;
+		st.pos = out.pos;
+		st.site_origin = out.site_origin;
+		return st;
+	}
+	__device__ __forceinline__ void store(const XRows& out, uint32_t half, uint64_t o, uint32_t nrows, uint32_t wi, uint32_t lane) const {
+		uint32_t* const gu[8] = {out.label, out.start_pos, out.end_pos, out.mid_pos, out.nsites, out.ext_pos, out.nbig, out.xnsites};
+		double* const gd[2] = {out.ext_value, out.prop};
+		if (lane < nrows) {
+#pragma unroll
+			for (int f = 0; f < 8; ++f)
+				if (f == (int)wi && gu[f]) gu[f][o] = u[f][half + lane];
+			if (wi == 0 && out.ext_site) out.ext_site[o] = s[half + lane];
+#pragma unroll
+			for (int f = 0; f < 2; ++f)
+				if (f + 1 == (int)wi && gd[f]) gd[f][o] = d[f][half + lane];
+		}
+	}
 };
 
 // One warp per window: lane l adds unit partials l, l+32, ... (from +0.0, so a window of
@@ -27,8 +97,8 @@ struct RowStage {
 // another GPU's HBM (one NVLink packet per store).
 template <class Stat>
 __global__ void __launch_bounds__(256) k_windows(DevPlan P, const typename Stat::Acc* __restrict__ units, uint64_t units_base,
-                                                  const uint32_t* __restrict__ pos, pgt_windows out) {
-	__shared__ RowStage rows;
+                                                  const uint32_t* __restrict__ pos, typename Stat::Out out) {
+	__shared__ RowStage<typename Stat::Out> rows;
 	const uint32_t lane = threadIdx.x & 31u, wi = threadIdx.x >> 5;
 	// The per-window work is a chain of dependent memory round trips; keep it short: the segment is
 	// cached (w only grows, so it changes a few dozen times per warp instead of costing a binary
@@ -45,22 +115,7 @@ __global__ void __launch_bounds__(256) k_windows(DevPlan P, const typename Stat:
 	const uint64_t per = (nwin_all + gridDim.x - 1) / gridDim.x;
 	const uint64_t w_begin = P.win_lo + (uint64_t)blockIdx.x * per;
 	const uint64_t w_end = w_begin + per < P.win_hi ? w_begin + per : P.win_hi;
-	pgt_windows staged;  // the same columns as `out`, 32 rows each, in shared memory
-	staged.label = out.label ? rows.u[0] : nullptr;
-	staged.start_pos = out.start_pos ? rows.u[1] : nullptr;
-	staged.end_pos = out.end_pos ? rows.u[2] : nullptr;
-	staged.mid_pos = out.mid_pos ? rows.u[3] : nullptr;
-	staged.nsites = out.nsites ? rows.u[4] : nullptr;
-	staged.nhet = out.nhet ? rows.u[5] : nullptr;
-	staged.nonmissing = out.nonmissing ? rows.u[6] : nullptr;
-	staged.neffective = out.neffective ? rows.u[7] : nullptr;
-	staged.nskip = out.nskip ? rows.u[8] : nullptr;
-	staged.sum_a = out.sum_a ? rows.d[0] : nullptr;
-	staged.sum_b = out.sum_b ? rows.d[1] : nullptr;
-	staged.fst = out.fst ? rows.d[2] : nullptr;
-	staged.het = out.het ? rows.d[3] : nullptr;
-	staged.dxy = out.dxy ? rows.d[4] : nullptr;
-	staged.dxy_global = nullptr;
+	const typename Stat::Out staged = rows.staged(out);  // the same columns as `out`, 32 rows each, in shared memory
 	uint32_t half = 0;  // which 32 rows of the stage this batch uses
 	for (uint64_t b0 = w_begin; b0 < w_end; b0 += 32u, half ^= 32u) {  // block-uniform
 		const uint32_t nrows = (uint32_t)(w_end - b0 < 32u ? w_end - b0 : 32u);
@@ -100,15 +155,7 @@ __global__ void __launch_bounds__(256) k_windows(DevPlan P, const typename Stat:
 			if (lane == 0) emit_window<Stat>(P, sg, w, k, acc, pos, staged, half + r, true, sp, ep);
 		}
 		__syncthreads();
-		const uint64_t o = b0 - P.win_lo + lane;
-		uint32_t* const gu[9] = {out.label, out.start_pos, out.end_pos, out.mid_pos, out.nsites, out.nhet, out.nonmissing, out.neffective, out.nskip};
-		double* const gd[5] = {out.sum_a, out.sum_b, out.fst, out.het, out.dxy};
-#pragma unroll
-		for (int f = 0; f < 9; ++f)
-			if ((f & 7) == (int)wi && gu[f] && lane < nrows) gu[f][o] = rows.u[f][half + lane];
-#pragma unroll
-		for (int f = 0; f < 5; ++f)
-			if (((f + 9) & 7) == (int)wi && gd[f] && lane < nrows) gd[f][o] = rows.d[f][half + lane];
+		rows.store(out, half, b0 - P.win_lo + lane, nrows, wi, lane);
 		// no second barrier: the next batch fills the other half, and the barrier after it orders this store before the refill
 	}
 }
@@ -136,7 +183,7 @@ struct SmallTree<Stat, P2, P2> {
 
 template <class Stat>
 __device__ __forceinline__ void emit_window(const DevPlan& P, const pgt_seg& sg, uint64_t w, uint64_t k, const typename Stat::Acc& acc,
-                                            const uint32_t* __restrict__ pos, const pgt_windows& out, uint64_t o, bool have_edges,
+                                            const uint32_t* __restrict__ pos, const typename Stat::Out& out, uint64_t o, bool have_edges,
                                             uint32_t edge_start, uint32_t edge_end) {
 	uint64_t fs;
 	const uint32_t nsites = pgt_window_sites(P.g, sg, k, &fs);
@@ -168,7 +215,7 @@ __device__ __forceinline__ void emit_window(const DevPlan& P, const pgt_seg& sg,
 
 template <class Stat, int P2>
 __global__ void __launch_bounds__(256) k_windows_small(DevPlan P, const typename Stat::Acc* __restrict__ units, uint64_t units_base,
-                                                        const uint32_t* __restrict__ pos, pgt_windows out) {
+                                                        const uint32_t* __restrict__ pos, typename Stat::Out out) {
 	const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
 	uint32_t si = 0xffffffffu;
 	pgt_seg sg;
@@ -260,7 +307,7 @@ struct GlobalTerm<FusedStat> {
 // their column loads together before the first row is stored; the label comes from a cached contig range
 // instead of a binary search per window.
 template <class Stat>
-__global__ void __launch_bounds__(256) k_windows_persite(DevPlan P, Cols cols, pgt_windows out, double* __restrict__ gpart) {
+__global__ void __launch_bounds__(256) k_windows_persite(DevPlan P, Cols cols, typename Stat::Out out, double* __restrict__ gpart) {
 	constexpr int U = 4;
 	double gd = 0.0;  // this thread's share of the global line (gpart != NULL: one partial triple per block)
 	unsigned long long gne = 0, gnk = 0;
@@ -303,7 +350,7 @@ __global__ void __launch_bounds__(256) k_windows_persite(DevPlan P, Cols cols, p
 				lc_hi = P.off[lc + 1];
 			}
 			typename Stat::Acc acc = Stat::zero();
-			Stat::fold(acc, v[q], cols.minind);
+			Stat::fold(acc, v[q], cols.minind, cols.cutoff, site[q]);
 			if (GlobalTerm<Stat>::has && gpart) GlobalTerm<Stat>::add(acc, gd, gne, gnk);
 			if (out.label) out.label[o] = lc;
 			if (out.nsites) out.nsites[o] = 1u;
@@ -494,7 +541,7 @@ __global__ void __launch_bounds__(256) k_windows_persite4(DevPlan P, Cols cols, 
 #pragma unroll
 			for (int q = 0; q < 4; ++q) {
 				acc[q] = Stat::zero();
-				Stat::fold(acc[q], v[q], cols.minind);
+				Stat::fold(acc[q], v[q], cols.minind, cols.cutoff, gs + q);
 				if (GlobalTerm<Stat>::has && gpart) GlobalTerm<Stat>::add(acc[q], gd, gne, gnk);
 			}
 			st4(out.label ? out.label + o : nullptr, lab[0], lab[1], lab[2], lab[3]);
@@ -517,7 +564,7 @@ __global__ void __launch_bounds__(256) k_windows_persite4(DevPlan P, Cols cols, 
 			for (uint64_t q = 0; o + q < nwin; ++q) {  // the last one to three windows of the scan
 				PGT_CHECK(i + q < P.col_elems);
 				typename Stat::Acc acc = Stat::zero();
-				Stat::fold(acc, Stat::load(cols, i + q), cols.minind);
+				Stat::fold(acc, Stat::load(cols, i + q), cols.minind, cols.cutoff, gs + q);
 				if (GlobalTerm<Stat>::has && gpart) GlobalTerm<Stat>::add(acc, gd, gne, gnk);
 				const uint32_t ps = cols.pos ? __ldg(cols.pos + i + q) : 0u;
 				lc = find_contig(P.off, 0, P.ncontig, gs + q);
@@ -617,7 +664,7 @@ __global__ void __launch_bounds__(256) k_block_scan(DevPlan P, typename Stat::Ac
 
 template <class Stat>
 __global__ void __launch_bounds__(256) k_windows_hgw(DevPlan P, const typename Stat::Acc* __restrict__ suf, const typename Stat::Acc* __restrict__ pre,
-                                                      uint64_t units_base, const uint32_t* __restrict__ pos, pgt_windows out) {
+                                                      uint64_t units_base, const uint32_t* __restrict__ pos, typename Stat::Out out) {
 	const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
 	const uint64_t B = P.g.wunits;
 	uint32_t si = 0xffffffffu;

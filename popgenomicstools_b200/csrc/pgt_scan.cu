@@ -25,6 +25,7 @@
 // the caller-owned workspace, kernel selection and launches, host-memory mode, the C ABI entry points.
 // There is no CPU fallback: every entry point fails with PGT_ERR_CUDA when no device is usable.
 #include <cuda_runtime.h>
+#include <math_constants.h>
 
 #include <algorithm>
 #include <atomic>
@@ -205,7 +206,11 @@ struct ColDesc {
 	uint32_t elem;
 };
 
-// The columns a statistic reads, in staging order -- pos first in bp mode, then a b f1 f2 n1 n2 g.  The tiled and
+// The extreme-score statistic (XStat) inside the host code: not a pgt_stat of the ABI (pgt_scan rejects it), only a
+// key of the per-statistic tables below.
+static constexpr pgt_stat kStatExtreme = (pgt_stat)16;
+
+// The columns a statistic reads, in staging order -- pos first in bp mode, then a b f1 f2 n1 n2 g score.  The tiled and
 // sliding-tile kernels read their staged columns in this order.
 static int stat_columns(pgt_stat stat, pgt_mode mode, ColDesc* d) {
 	int n = 0;
@@ -221,6 +226,7 @@ static int stat_columns(pgt_stat stat, pgt_mode mode, ColDesc* d) {
 		d[n++] = {offsetof(Cols, n2), 4};
 	}
 	if (stat == PGT_STAT_HET || stat == PGT_STAT_FUSED) d[n++] = {offsetof(Cols, g), 1};
+	if (stat == kStatExtreme) d[n++] = {offsetof(Cols, score), 8};
 	return n;
 }
 static const void* col_ptr(const Cols& c, const ColDesc& d) {
@@ -230,15 +236,17 @@ static const void* col_ptr(const Cols& c, const ColDesc& d) {
 }
 static void set_col_ptr(Cols* c, const ColDesc& d, const void* p) { memcpy((char*)c + d.member, &p, sizeof(p)); }
 
-static Cols cols_from(const pgt_columns& c, int minind) { return Cols{c.pos, c.a, c.b, c.geno, c.f1, c.f2, c.n1, c.n2, minind}; }
+static Cols cols_from(const pgt_columns& c, int minind) { return Cols{c.pos, c.a, c.b, c.geno, c.f1, c.f2, c.n1, c.n2, nullptr, minind, 0.0}; }
 
 template <class Stat>
-static constexpr pgt_stat kStatOf = std::is_same<Stat, FstStat>::value   ? PGT_STAT_FST
+static constexpr pgt_stat kStatOf = IsXStat<Stat>::value                 ? kStatExtreme
+                                    : std::is_same<Stat, FstStat>::value ? PGT_STAT_FST
                                     : std::is_same<Stat, HetStat>::value ? PGT_STAT_HET
                                     : std::is_same<Stat, DxyStat>::value ? PGT_STAT_DXY
                                                                          : PGT_STAT_FUSED;
 
 static size_t acc_bytes(pgt_stat stat) {
+	if (stat == kStatExtreme) return sizeof(XStat<XMODE_ABS>::Acc);
 	switch (stat) {
 		case PGT_STAT_FST: return sizeof(FstStat::Acc);
 		case PGT_STAT_HET: return sizeof(HetStat::Acc);
@@ -314,14 +322,14 @@ static bool slide_shape(const pgt_geom& g, pgt_mode mode, pgt_stat stat, SlideSh
 // the summation order, so it is a function of (W, S, unit, statistic) and the tuning knobs only -- never of the input
 // size, the window range or the shard.
 static int scan_path(const pgt_plan* plan, pgt_stat stat, SlideShape* sh) {
-	if (slide_shape(plan->g, plan->mode, stat, sh)) return PGT_PATH_SLIDE;
+	if (stat != kStatExtreme && slide_shape(plan->g, plan->mode, stat, sh)) return PGT_PATH_SLIDE;
 	if (plan->mode == PGT_MODE_SITES && plan->g.W == 1 && plan->g.S == 1 && g_tune_level2 != 1) return PGT_PATH_PERSITE;
 	return PGT_PATH_UNITS;
 }
 
 struct Layout {
 	uint64_t w_lo, w_hi, u_lo, u_hi, g_hi, origin;
-	size_t segs_off, off_off, siteoff_off, gpart_off, units_off, pre_off, bounds_off, stage_off, outs_off, tileseg_off, total;
+	size_t segs_off, off_off, siteoff_off, gpart_off, units_off, pre_off, bounds_off, stage_off, outs_off, tileseg_off, flag_off, total;
 	uint64_t tileseg_cap;  // entries of the tile -> segment table (0 = not used: few segments)
 	bool hgw;              // level 2 in scan mode
 	bool unit_table;       // very many segments: level 1 reads unit starts from a table (k_unit_starts) instead of the segment records
@@ -340,7 +348,7 @@ struct Layout {
 
 static int make_layout(const pgt_plan* plan, const pgt_range* range, pgt_stat stat, pgt_mem mem, Layout* L) {
 	if (!plan) return pgt_set_error(PGT_ERR_ARGS, "plan is NULL");
-	if ((int)stat < 0 || (int)stat > (int)PGT_STAT_FUSED) return pgt_set_error(PGT_ERR_ARGS, "unknown statistic");
+	if (stat != kStatExtreme && ((int)stat < 0 || (int)stat > (int)PGT_STAT_FUSED)) return pgt_set_error(PGT_ERR_ARGS, "unknown statistic");
 	uint64_t lo = 0, hi = plan->nwin, org = plan->off[0];
 	if (range) {
 		if (range->w_hi != 0 || range->w_lo != 0) {
@@ -442,6 +450,9 @@ static int make_layout(const pgt_plan* plan, const pgt_range* range, pgt_stat st
 	L->tileseg_off = o;
 	L->tileseg_cap = plan->segs.size() > kTileSegTableMin ? nunits / 8 + 1024 : 0;
 	o += align_up((size_t)L->tileseg_cap * sizeof(uint32_t), 256);
+	// extreme scan of a bp plan in device memory: the position check's flag
+	L->flag_off = o;
+	if (stat == kStatExtreme && plan->mode == PGT_MODE_BP && mem == PGT_MEM_DEVICE) o += 256;
 	L->total = o + 256;
 	return PGT_OK;
 }
@@ -470,6 +481,7 @@ extern "C" int pgt_plan_bind_device(pgt_plan* plan, void* buffer, size_t bytes, 
 }
 
 extern "C" size_t pgt_scan_workspace_bytes(const pgt_plan* plan, const pgt_range* range, pgt_stat stat, pgt_mem mem) {
+	if ((int)stat < 0 || (int)stat > (int)PGT_STAT_FUSED) return 0;
 	Layout L;
 	if (make_layout(plan, range, stat, mem, &L) != PGT_OK) return 0;
 	return L.total;
@@ -522,7 +534,7 @@ static TileBudget tile_budget(const StatCols& sc) {
 }
 
 template <class Stat, bool INDIRECT>
-static int launch_units_tiled(const DevPlan& P, const StatCols& sc, const TileBudget& tb, int minind, typename Stat::Acc* units,
+static int launch_units_tiled(const DevPlan& P, const StatCols& sc, const TileBudget& tb, const Cols& cols, typename Stat::Acc* units,
                               const uint64_t* bounds, uint64_t valid_elems, uint32_t* tileseg, uint64_t tileseg_cap, cudaStream_t st) {
 	const uint64_t nunits = P.unit_hi - P.unit_lo;
 	const int nsm = num_sms();
@@ -561,7 +573,8 @@ static int launch_units_tiled(const DevPlan& P, const StatCols& sc, const TileBu
 	tc.ncol = sc.n;
 	tc.m = m;
 	tc.nstages = tb.nstages;
-	tc.minind = minind;
+	tc.minind = cols.minind;
+	tc.cutoff = cols.cutoff;
 	tc.valid_elems = valid_elems;
 	uint32_t o = 0;
 	for (uint32_t c = 0; c < sc.n; ++c) {
@@ -617,15 +630,17 @@ static int launch_units(const DevPlan& P, const Cols& cols, typename Stat::Acc* 
 	// (hetWindow's 1-byte column stays on the vectorised direct kernel: measured at 3e9 sites, 4096-site units,
 	// 6.14 TB/s direct against 5.44 TB/s through the ring -- both were issue-bound on the byte counting, 4.5 and
 	// 4.3 TB/s, until it went from POPC to dp4a; the ring's het consumer remains for forced / short-unit runs)
-	bool tiled = P.g.gw != 32 || (tb.bps > 1 && approx_bytes >= (256ull << 20));
+	// (the extreme score too: at 1e9 sites, 50000/10000 the direct kernel took 2.01 ms against 2.30 ms through the ring,
+	// dense bp 100000/10000 1.79 against 1.93 ms; profiles/r05b_plan_extreme_probe.jsonl)
+	bool tiled = P.g.gw != 32 || (tb.bps > 1 && !IsXStat<Stat>::value && approx_bytes >= (256ull << 20));
 	if (g_tune_level1 == 2) tiled = true;
 	if (g_tune_level1 == 1 && P.g.gw == 32) tiled = false;
 	// a tile holds whole units: very long units (unit_sites up to 4096) may not fit a stage;
 	// they always have gw == 32, so the direct kernel applies
 	if ((uint64_t)P.g.ueff * tb.bps + 64ull * kMaxTileCols > tb.stage_bytes) tiled = false;
 	if (tiled)
-		return bounds ? launch_units_tiled<Stat, true>(P, sc, tb, cols.minind, units, bounds, valid_elems, nullptr, 0, st)
-		              : launch_units_tiled<Stat, false>(P, sc, tb, cols.minind, units, bounds, valid_elems, tileseg, tileseg_cap, st);
+		return bounds ? launch_units_tiled<Stat, true>(P, sc, tb, cols, units, bounds, valid_elems, nullptr, 0, st)
+		              : launch_units_tiled<Stat, false>(P, sc, tb, cols, units, bounds, valid_elems, tileseg, tileseg_cap, st);
 	const int threads = 256;
 	const uint64_t want = (nunits + 7) / 8;  // one warp per unit, 8 warps per block
 	if constexpr (std::is_same<Stat, HetStat>::value) {  // hetWindow: the vectorised byte kernel replaces the generic direct kernel
@@ -666,7 +681,7 @@ static int launch_bounds_kernel(const DevPlan& P, const uint32_t* pos, uint64_t 
 
 // scan mode (L.hgw): `units` is scanned in place into SUF, `pre` receives PRE; see k_block_scan
 template <class Stat>
-static int launch_windows(const DevPlan& P, typename Stat::Acc* units, uint64_t units_base, const uint32_t* pos, const pgt_windows& out,
+static int launch_windows(const DevPlan& P, typename Stat::Acc* units, uint64_t units_base, const uint32_t* pos, const typename Stat::Out& out,
                           bool hgw, typename Stat::Acc* pre, uint64_t blk_lo, uint64_t blk_hi, cudaStream_t st) {
 	const uint64_t nwin = P.win_hi - P.win_lo;
 	if (nwin == 0) return PGT_OK;
@@ -677,7 +692,7 @@ static int launch_windows(const DevPlan& P, typename Stat::Acc* units, uint64_t 
 		k_windows_hgw<Stat><<<capped_grid((nwin + 255) / 256), 256, 0, st>>>(P, units, pre, units_base, pos, out);
 	} else if (P.g.wunits <= 32 && g_tune_level2 != 1) {
 		// fine windows: a thread per window
-		void (*kern)(DevPlan, const typename Stat::Acc*, uint64_t, const uint32_t*, pgt_windows);
+		void (*kern)(DevPlan, const typename Stat::Acc*, uint64_t, const uint32_t*, typename Stat::Out);
 		const uint32_t wu = P.g.wunits;
 		if (wu <= 1) kern = k_windows_small<Stat, 1>;
 		else if (wu <= 2) kern = k_windows_small<Stat, 2>;
@@ -817,28 +832,34 @@ static bool slide_runs_cover_owned_sites(const pgt_plan* plan, const Layout& L) 
 }
 
 // W = S = 1: the vectorised kernel when its preconditions hold (one segment; every used column and output pointer
-// 16-byte aligned at the scan's first window -- 4-byte aligned for the genotype column), else the scalar one.
+// 16-byte aligned at the scan's first window -- 4-byte aligned for the genotype column), else the scalar one.  (The
+// extreme scan has the scalar kernel only.)
 template <class Stat>
-static int launch_persite(const pgt_plan* plan, const DevPlan& P, const Cols& C, const pgt_windows& out, double* gpart, double* g3,
+static int launch_persite(const pgt_plan* plan, const DevPlan& P, const Cols& C, const typename Stat::Out& out, double* gpart, double* g3,
                           cudaStream_t st) {
 	const uint64_t nwin = P.win_hi - P.win_lo;
 	if (nwin == 0) return PGT_OK;
-	bool vec = g_tune_persite != 1 && plan->segs.size() == 1 && nwin >= 4;
+	bool vec = false;
 	uint64_t site0 = 0;
-	if (vec) {
-		site0 = plan->segs[0].site_base + (P.win_lo - plan->segs[0].win_base) - P.site_origin;
-		auto ok = [&](const void* p, size_t elem, size_t align) { return !p || (((uintptr_t)p + site0 * elem) & (align - 1)) == 0; };
-		ColDesc d[8];
-		const int nc = stat_columns(kStatOf<Stat>, PGT_MODE_SITES, d);
-		for (int i = 0; i < nc; ++i) vec = vec && col_ptr(C, d[i]) && ok(col_ptr(C, d[i]), d[i].elem, d[i].elem == 1 ? 4 : 16);
-		vec = vec && ok(C.pos, 4, 16);
-		for_each_field([&](const void* p) { vec = vec && (((uintptr_t)p) & 15) == 0; }, out);
+	if constexpr (!IsXStat<Stat>::value) {
+		vec = g_tune_persite != 1 && plan->segs.size() == 1 && nwin >= 4;
+		if (vec) {
+			site0 = plan->segs[0].site_base + (P.win_lo - plan->segs[0].win_base) - P.site_origin;
+			auto ok = [&](const void* p, size_t elem, size_t align) { return !p || (((uintptr_t)p + site0 * elem) & (align - 1)) == 0; };
+			ColDesc d[8];
+			const int nc = stat_columns(kStatOf<Stat>, PGT_MODE_SITES, d);
+			for (int i = 0; i < nc; ++i) vec = vec && col_ptr(C, d[i]) && ok(col_ptr(C, d[i]), d[i].elem, d[i].elem == 1 ? 4 : 16);
+			vec = vec && ok(C.pos, 4, 16);
+			for_each_field([&](const void* p) { vec = vec && (((uintptr_t)p) & 15) == 0; }, out);
+		}
 	}
 	ProfScope prof(1, st);
-	unsigned grid;
+	unsigned grid = 0;
 	if (vec) {
-		grid = std::min<unsigned>(one_wave_grid(k_windows_persite4<Stat>, 256, (nwin + 1023) / 1024), kGlobalMaxPartials);
-		k_windows_persite4<Stat><<<grid, 256, 0, st>>>(P, C, out, site0, gpart);
+		if constexpr (!IsXStat<Stat>::value) {
+			grid = std::min<unsigned>(one_wave_grid(k_windows_persite4<Stat>, 256, (nwin + 1023) / 1024), kGlobalMaxPartials);
+			k_windows_persite4<Stat><<<grid, 256, 0, st>>>(P, C, out, site0, gpart);
+		}
 	} else {
 		grid = std::min<unsigned>(one_wave_grid(k_windows_persite<Stat>, 256, (nwin + 1023) / 1024), kGlobalMaxPartials);  // four windows per thread and turn
 		k_windows_persite<Stat><<<grid, 256, 0, st>>>(P, C, out, gpart);
@@ -888,7 +909,8 @@ struct Scan {
 	DevPlan P;
 	Cols C;  // the caller's columns (device or host pointers)
 	const uint64_t* site_offsets;
-	const pgt_windows* out;
+	const pgt_windows* out;  // the extreme scan: its geometry rows (all NULL when none are wanted)
+	XRows x;                 // the extreme scan's rows (the caller's arrays; site_origin = the scan's)
 	char* ws;
 	uint64_t* bounds;  // bp mode / unit table: unit bounds in the workspace
 	uint64_t ndata;    // bp mode: sites the columns hold
@@ -896,6 +918,30 @@ struct Scan {
 	bool bp, want_global;
 	cudaStream_t st;
 };
+
+// the rows a scan of Stat writes
+template <class Stat>
+static typename Stat::Out rows_of(const Scan& s) {
+	if constexpr (IsXStat<Stat>::value) return s.x;
+	else return *s.out;
+}
+
+// bp mode: the first and last site this call holds of every chromosome must lie on the chromosome (1 <= pos <= length);
+// *bad receives the smallest global index of a site that does not (left as it is when all do)
+static void bp_check_positions_host(const pgt_plan* plan, const uint64_t* site_off, const uint32_t* pos, uint64_t origin, uint64_t ndata,
+                                    uint64_t* bad) {
+	const uint32_t nc = (uint32_t)plan->off.size() - 1;
+	for (uint32_t c = 0; c < nc; ++c) {
+		const uint64_t lo = std::max(site_off[c], origin), hi = std::min(site_off[c + 1], origin + ndata);
+		if (hi <= lo) continue;
+		const uint64_t len = plan->off[c + 1] - plan->off[c];
+		if (pos[lo - origin] < 1u) *bad = std::min(*bad, lo);
+		else if (pos[hi - 1 - origin] > len) *bad = std::min(*bad, hi - 1);
+	}
+}
+static int bp_position_error(uint64_t bad) {
+	return pgt_set_error(PGT_ERR_INPUT, "site " + std::to_string(bad) + " lies outside its chromosome (bp positions run from 1 to the chromosome length)");
+}
 
 // ---- PGT_MEM_DEVICE: the columns are read in place
 template <class Stat>
@@ -919,8 +965,8 @@ static int scan_device(const Scan& s) {
 				// the windows ARE the sites: when the owned range of the global line is exactly their span (always, unless the
 				// scan owns sites outside any window) the kernel adds its sites up on the way and the dxy columns are read once
 				global_done = s.want_global && GlobalTerm<Stat>::has && L.gsite_lo == first_site && L.gsite_hi == last_site + 1;
-				PGT_TRY(launch_persite<Stat>(plan, P, s.C, *s.out, global_done ? gpart : nullptr, s.out->dxy_global, s.st));
-			} else {
+				PGT_TRY(launch_persite<Stat>(plan, P, s.C, rows_of<Stat>(s), global_done ? gpart : nullptr, s.out->dxy_global, s.st));
+			} else if constexpr (!IsXStat<Stat>::value) {
 				global_done = s.want_global && GlobalTerm<Stat>::has && g_tune_slideglobal != 1 && slide_runs_cover_owned_sites(plan, L);
 				PGT_TRY(launch_slide<Stat>(plan, L.slide, P, s.C, last_site + 1 - L.origin, s.C.pos, *s.out, global_done ? gpart : nullptr,
 				                           s.out->dxy_global, s.st));
@@ -931,6 +977,16 @@ static int scan_device(const Scan& s) {
 			PGT_TRY(launch_global_sites(s.C, L.gsite_lo - L.origin, L.gsite_hi - L.origin, gpart, s.out->dxy_global, s.st));
 		}
 		return PGT_OK;
+	}
+	unsigned long long* bad = nullptr;  // the extreme scan of a bp plan checks the positions (read back at the end)
+	if (IsXStat<Stat>::value && s.bp) {
+		bad = (unsigned long long*)(s.ws + L.flag_off);
+		PGT_CUDA(cudaMemsetAsync(bad, 0xff, sizeof(*bad), s.st));
+		DevPlan Pc = P;
+		Pc.col_elems = s.ndata;
+		k_bp_pos_check<<<capped_grid((P.ncontig + 255) / 256), 256, 0, s.st>>>(Pc, s.C.pos, s.ndata, bad);
+		g_launches++;
+		PGT_CUDA(cudaGetLastError());
 	}
 	if (s.bp && nunits) PGT_TRY(launch_bounds_kernel(P, s.C.pos, s.ndata, s.bounds, s.st));
 	if (L.unit_table) {  // very many segments: unit starts once, then the INDIRECT level-1 kernels
@@ -945,7 +1001,14 @@ static int scan_device(const Scan& s) {
 	                           L.tileseg_cap, s.st));
 	// the global line reads the raw unit partials: before level 2, which may scan them in place
 	if (s.want_global) PGT_TRY(launch_global<Stat>(units, s.nglobal, gpart, s.out->dxy_global, s.st));
-	return launch_windows<Stat>(P, units, L.u_lo, s.C.pos, *s.out, L.hgw, (typename Stat::Acc*)(s.ws + L.pre_off), L.blk_lo, L.blk_hi, s.st);
+	PGT_TRY(launch_windows<Stat>(P, units, L.u_lo, s.C.pos, rows_of<Stat>(s), L.hgw, (typename Stat::Acc*)(s.ws + L.pre_off), L.blk_lo, L.blk_hi, s.st));
+	if (bad) {
+		unsigned long long h = 0;
+		PGT_CUDA(cudaMemcpyAsync(&h, bad, sizeof(h), cudaMemcpyDeviceToHost, s.st));
+		PGT_CUDA(cudaStreamSynchronize(s.st));
+		if (h != ~0ull) return bp_position_error(h);
+	}
+	return PGT_OK;
 }
 
 // ---- PGT_MEM_HOST: slabs of the axis are staged H2D on a copy stream (double-buffered) while the previous slab is
@@ -972,6 +1035,7 @@ struct HostStaging {
 		if (used[slot]) PGT_CUDA(cudaStreamWaitEvent(copy, freed[slot], 0));
 		*C = Cols{};
 		C->minind = s.C.minind;
+		C->cutoff = s.C.cutoff;
 		for (int i = 0; i < ncol; ++i) {
 			const char* src = (const char*)col_ptr(s.C, cd[i]) + (s0 - s.L.origin) * cd[i].elem;
 			if (ns) PGT_CUDA(cudaMemcpyAsync(buf[slot][i], src, ns * cd[i].elem, cudaMemcpyHostToDevice, copy));
@@ -1044,31 +1108,46 @@ static void start_bookkeeping(const Scan& s, Bookkeeper* book) {
 	}
 }
 
+// the values of extreme-score rows the window kernels write on the device (ext_value, ext_pos: gathered on the host from
+// ext_site), member by member
+template <class F, class... T>
+static void for_each_xrow_value(F&& fn, T&... t) {
+	fn(t.ext_site...), fn(t.prop...), fn(t.nbig...), fn(t.xnsites...);
+}
+
 // Per-window values are produced into device tables, then copied back: one table for the whole scan, or -- when the
 // windows come straight from the sites, slab by slab -- two slab-sized tables used in turn.  A table has 12 slots:
-// the nine values in slots 0-8, the global triple in slot 11.
-static pgt_windows device_table(const Scan& s, int which) {
+// the nine values in slots 0-8 (the extreme scan: for_each_xrow_value), the global triple in slot 11.  `host` are the
+// caller's rows the table is copied back to (the extreme scan: ext_site also when only ext_value / ext_pos are wanted).
+template <class Out>
+static Out device_table(const Scan& s, const Out& host, int which) {
 	const uint64_t rows = s.L.path == PGT_PATH_UNITS ? s.L.w_hi - s.L.w_lo : s.L.out_slab_rows;
 	const size_t ob = align_up((size_t)rows * 8 + 8, 256);
 	char* t = s.ws + s.L.outs_off + (size_t)which * 12 * ob;
-	pgt_windows d;
+	Out d;
 	memset(&d, 0, sizeof(d));
 	int k = 0;
 	auto slot = [&](auto*& dp, auto* want) {
 		if (want) dp = (decltype(want))(t + ob * k);
 		++k;
 	};
-	for_each_value(slot, d, *s.out);
-	d.dxy_global = s.want_global ? (double*)(t + ob * 11) : nullptr;
+	if constexpr (std::is_same<Out, XRows>::value) {
+		for_each_xrow_value(slot, d, host);
+	} else {
+		for_each_value(slot, d, host);
+		d.dxy_global = s.want_global ? (double*)(t + ob * 11) : nullptr;
+	}
 	return d;
 }
 // rows [row0, row0 + n) of the caller's arrays <- rows [0, n) of a device table, on `st`
-static int copy_back(const Scan& s, const pgt_windows& d, uint64_t row0, uint64_t n) {
+template <class Out>
+static int copy_back(const Scan& s, const Out& host, const Out& d, uint64_t row0, uint64_t n) {
 	cudaError_t e = cudaSuccess;
 	auto back = [&](auto* h, auto* dp) {
 		if (e == cudaSuccess && h && dp && n) e = cudaMemcpyAsync(h + row0, dp, n * sizeof(*h), cudaMemcpyDeviceToHost, s.st);
 	};
-	for_each_value(back, *s.out, d);
+	if constexpr (std::is_same<Out, XRows>::value) for_each_xrow_value(back, host, d);
+	else for_each_value(back, host, d);
 	if (e != cudaSuccess) return cuda_fail(e, "cudaMemcpyAsync(window table -> host)");
 	return PGT_OK;
 }
@@ -1078,7 +1157,7 @@ static int copy_back(const Scan& s, const pgt_windows& d, uint64_t row0, uint64_
 // every slab folds the part of the owned range [gsite_lo, gsite_hi) that no earlier slab has folded, one partial
 // triple per slab, added in slab order on the host.
 template <class Stat>
-static int host_window_slabs(const Scan& s, HostStaging& hs) {
+static int host_window_slabs(const Scan& s, HostStaging& hs, const typename Stat::Out& host) {
 	const pgt_plan* plan = s.plan;
 	const Layout& L = s.L;
 	const uint64_t slab_target = L.slab_sites - kSlabSlack;
@@ -1110,12 +1189,12 @@ static int host_window_slabs(const Scan& s, HostStaging& hs) {
 		Ps.win_hi = wb;
 		Ps.site_origin = s0;
 		Ps.col_elems = ns;
-		const pgt_windows o = device_table(s, hs.slot);  // rewritten two slabs later, after this slab's copy-back (order of `st`)
+		const typename Stat::Out o = device_table(s, host, hs.slot);  // rewritten two slabs later, after this slab's copy-back (order of `st`)
 		// (global line: fold_global below)
 		if (L.path == PGT_PATH_PERSITE) PGT_TRY(launch_persite<Stat>(plan, Ps, C, o, nullptr, nullptr, s.st));
-		else PGT_TRY(launch_slide<Stat>(plan, L.slide, Ps, C, ns, nullptr, o, nullptr, nullptr, s.st));
+		else if constexpr (!IsXStat<Stat>::value) PGT_TRY(launch_slide<Stat>(plan, L.slide, Ps, C, ns, nullptr, o, nullptr, nullptr, s.st));
 		PGT_TRY(fold_global(C, s0, s0 + ns));
-		PGT_TRY(copy_back(s, o, w - L.w_lo, wb - w));
+		PGT_TRY(copy_back(s, host, o, w - L.w_lo, wb - w));
 		PGT_TRY(hs.release(s.st));
 		w = wb;
 	}
@@ -1194,6 +1273,20 @@ static int scan_host(const Scan& s) {
 	// the copy stream must not start before the caller's stream reaches this point
 	PGT_CUDA(cudaEventRecord(hs.freed[0], s.st));
 	PGT_CUDA(cudaStreamWaitEvent(hs.copy, hs.freed[0], 0));
+	// the rows copied back; the extreme scan gathers ext_value and ext_pos on the host from ext_site (kept here if not wanted)
+	typename Stat::Out host = rows_of<Stat>(s);
+	std::vector<uint64_t> site_tmp;
+	if constexpr (IsXStat<Stat>::value) {
+		if (s.bp) {
+			uint64_t bad = ~0ull;
+			bp_check_positions_host(s.plan, s.site_offsets, s.C.pos, L.origin, s.ndata, &bad);
+			if (bad != ~0ull) return bp_position_error(bad);
+		}
+		if ((host.ext_value || host.ext_pos) && !host.ext_site) {
+			site_tmp.resize(L.w_hi - L.w_lo);
+			host.ext_site = site_tmp.data();
+		}
+	}
 	Bookkeeper book;
 	start_bookkeeping(s, &book);
 	hs.ncol = stat_columns(s.stat, s.plan->mode, hs.cd);
@@ -1204,19 +1297,44 @@ static int scan_host(const Scan& s) {
 			o += L.stage_col_bytes[i];
 		}
 	if (L.path != PGT_PATH_UNITS) {
-		PGT_TRY(host_window_slabs<Stat>(s, hs));
+		PGT_TRY(host_window_slabs<Stat>(s, hs, host));
 	} else {
 		typename Stat::Acc* units = (typename Stat::Acc*)(s.ws + L.units_off);
 		PGT_TRY(host_unit_slabs<Stat>(s, hs, units));
-		const pgt_windows dev = device_table(s, 0);
-		if (s.want_global) PGT_TRY(launch_global<Stat>(units, s.nglobal, (double*)(s.ws + L.gpart_off), dev.dxy_global, s.st));
+		const typename Stat::Out dev = device_table(s, host, 0);
+		if constexpr (!IsXStat<Stat>::value)
+			if (s.want_global) PGT_TRY(launch_global<Stat>(units, s.nglobal, (double*)(s.ws + L.gpart_off), dev.dxy_global, s.st));
 		PGT_TRY(launch_windows<Stat>(s.P, units, L.u_lo, nullptr, dev, L.hgw, (typename Stat::Acc*)(s.ws + L.pre_off), L.blk_lo, L.blk_hi, s.st));
-		PGT_TRY(copy_back(s, dev, 0, L.w_hi - L.w_lo));
-		if (s.want_global) PGT_CUDA(cudaMemcpyAsync(s.out->dxy_global, dev.dxy_global, 3 * sizeof(double), cudaMemcpyDeviceToHost, s.st));
+		PGT_TRY(copy_back(s, host, dev, 0, L.w_hi - L.w_lo));
+		if constexpr (!IsXStat<Stat>::value)
+			if (s.want_global) PGT_CUDA(cudaMemcpyAsync(s.out->dxy_global, dev.dxy_global, 3 * sizeof(double), cudaMemcpyDeviceToHost, s.st));
 	}
 	book.join();
 	PGT_CUDA(cudaStreamSynchronize(s.st));
 	PGT_CUDA(cudaStreamSynchronize(hs.copy));
+	if constexpr (IsXStat<Stat>::value) {
+		const uint64_t nan_bits = 0xfff8000000000000ull;  // CUDART_NAN, the empty row's value on the device
+		double empty_nan;
+		memcpy(&empty_nan, &nan_bits, sizeof(empty_nan));
+		// one random read per row and value: split over host threads as the bookkeeping (1e8 rows at W = S = 1)
+		const uint64_t nwin = L.w_hi - L.w_lo;
+		auto gather = [&host, &s, &L, empty_nan](uint64_t wa, uint64_t wb) {
+			for (uint64_t w = wa; w < wb; ++w) {
+				const bool empty = host.ext_site[w] == ~0ull;
+				if (host.ext_value) host.ext_value[w] = empty ? empty_nan : s.C.score[host.ext_site[w] - L.origin];
+				if (host.ext_pos) host.ext_pos[w] = empty ? 0u : s.C.pos[host.ext_site[w] - L.origin];
+			}
+		};
+		if (host.ext_site && (host.ext_value || host.ext_pos)) {
+			const unsigned nt = nwin < (1u << 16) ? 1u : std::min<unsigned>(8u, std::max(1u, std::thread::hardware_concurrency()));
+			const uint64_t per = (nwin + nt - 1) / nt;
+			std::vector<std::thread> th;
+			for (unsigned t = 1; t < nt; ++t)
+				if (per * t < nwin) th.emplace_back(gather, per * t, std::min<uint64_t>(nwin, per * (t + 1)));
+			gather(0, std::min<uint64_t>(nwin, per));
+			for (auto& t : th) t.join();
+		}
+	}
 	return PGT_OK;
 }
 
@@ -1238,10 +1356,10 @@ static DevPlan dev_plan(const pgt_plan* plan, const char* segs, const char* off,
 	return P;
 }
 
+// xrows: the extreme scan's rows (then `out` holds its geometry rows), else NULL
 template <class Stat>
-static int run_scan(const pgt_plan* plan, const pgt_range* range, pgt_stat stat, const pgt_columns* cols, int minind,
-                    const uint64_t* site_offsets, const pgt_windows* out, void* workspace, size_t workspace_bytes, pgt_mem mem,
-                    cudaStream_t st) {
+static int run_scan(const pgt_plan* plan, const pgt_range* range, pgt_stat stat, const Cols& C, const uint64_t* site_offsets,
+                    const pgt_windows* out, const XRows* xrows, void* workspace, size_t workspace_bytes, pgt_mem mem, cudaStream_t st) {
 	int ndev = 0;
 	if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0)
 		return pgt_set_error(PGT_ERR_CUDA, "no usable CUDA device (libpgtscan has no CPU fallback)");
@@ -1251,10 +1369,9 @@ static int run_scan(const pgt_plan* plan, const pgt_range* range, pgt_stat stat,
 	if (!workspace) return pgt_set_error(PGT_ERR_ARGS, "workspace is NULL");
 	if (workspace_bytes < L.total) return pgt_set_error(PGT_ERR_NOMEM, "workspace too small, see pgt_scan_workspace_bytes");
 	const bool bp = plan->mode == PGT_MODE_BP;
-	if (bp && (!site_offsets || !cols->pos)) return pgt_set_error(PGT_ERR_ARGS, "bp mode needs site_offsets and pos");
+	if (bp && (!site_offsets || !C.pos)) return pgt_set_error(PGT_ERR_ARGS, "bp mode needs site_offsets and pos");
 	const uint64_t nunits = L.u_hi - L.u_lo;
 	if (nunits == 0 && L.w_hi == L.w_lo) return PGT_OK;  // empty input / empty shard: nothing to read or write
-	const Cols C = cols_from(*cols, minind);
 	ColDesc cd[8];
 	const int ncol = stat_columns(stat, plan->mode, cd);
 	for (int i = 0; i < ncol; ++i)
@@ -1290,6 +1407,11 @@ static int run_scan(const pgt_plan* plan, const pgt_range* range, pgt_stat stat,
 	s.C = C;
 	s.site_offsets = site_offsets;
 	s.out = out;
+	memset(&s.x, 0, sizeof(s.x));
+	if (xrows) {
+		s.x = *xrows;
+		s.x.site_origin = L.origin;
+	}
 	s.ws = ws;
 	s.bounds = (bp || L.unit_table) ? (uint64_t*)(ws + L.bounds_off) : nullptr;
 	s.nglobal = L.g_hi > L.u_lo ? L.g_hi - L.u_lo : 0;
@@ -1306,14 +1428,14 @@ extern "C" int pgt_scan(const pgt_plan* plan, const pgt_range* range, pgt_stat s
 	if (mem != PGT_MEM_DEVICE && mem != PGT_MEM_HOST) return pgt_set_error(PGT_ERR_ARGS, "pgt_scan: unknown memory space");
 	cudaStream_t st = (cudaStream_t)stream;
 	switch (stat) {
-		case PGT_STAT_FST: return run_scan<FstStat>(plan, range, stat, cols, minind, site_offsets, out, workspace, workspace_bytes, mem, st);
-		case PGT_STAT_HET: return run_scan<HetStat>(plan, range, stat, cols, minind, site_offsets, out, workspace, workspace_bytes, mem, st);
+		case PGT_STAT_FST: return run_scan<FstStat>(plan, range, stat, cols_from(*cols, minind), site_offsets, out, nullptr, workspace, workspace_bytes, mem, st);
+		case PGT_STAT_HET: return run_scan<HetStat>(plan, range, stat, cols_from(*cols, minind), site_offsets, out, nullptr, workspace, workspace_bytes, mem, st);
 		case PGT_STAT_DXY:
 			if (minind < 1) return pgt_set_error(PGT_ERR_ARGS, "-minind must be at least 1");
-			return run_scan<DxyStat>(plan, range, stat, cols, minind, site_offsets, out, workspace, workspace_bytes, mem, st);
+			return run_scan<DxyStat>(plan, range, stat, cols_from(*cols, minind), site_offsets, out, nullptr, workspace, workspace_bytes, mem, st);
 		case PGT_STAT_FUSED:
 			if (minind < 1) return pgt_set_error(PGT_ERR_ARGS, "-minind must be at least 1");
-			return run_scan<FusedStat>(plan, range, stat, cols, minind, site_offsets, out, workspace, workspace_bytes, mem, st);
+			return run_scan<FusedStat>(plan, range, stat, cols_from(*cols, minind), site_offsets, out, nullptr, workspace, workspace_bytes, mem, st);
 	}
 	return pgt_set_error(PGT_ERR_ARGS, "pgt_scan: unknown statistic");
 }
@@ -1443,4 +1565,42 @@ extern "C" int pgt_scan_bp_sites(const pgt_plan* plan, const pgt_range* range, c
 	if (bad != ~0ull)
 		return pgt_set_error(PGT_ERR_INPUT, "site " + std::to_string(bad) + " lies outside its chromosome (bp positions run from 1 to the chromosome length)");
 	return PGT_OK;
+}
+
+// ---- the extreme score over a window plan (pgt_scan_plan_extreme): the scan of pgt_scan with the statistic XStat
+extern "C" size_t pgt_scan_plan_extreme_workspace_bytes(const pgt_plan* plan, const pgt_range* range, pgt_mem mem) {
+	Layout L;
+	if (make_layout(plan, range, kStatExtreme, mem, &L) != PGT_OK) return 0;
+	return L.total;
+}
+
+extern "C" int pgt_scan_plan_extreme(const pgt_plan* plan, const pgt_range* range, pgt_xstat stat, double cutoff, const uint32_t* pos,
+                                     const double* score, const uint64_t* site_offsets, const pgt_windows* rows, const pgt_xwindows* out,
+                                     void* workspace, size_t workspace_bytes, pgt_mem mem, void* stream) {
+	if (!plan || !out) return pgt_set_error(PGT_ERR_ARGS, "pgt_scan_plan_extreme: plan and out must not be NULL");
+	if (stat != PGT_XSTAT_IHS && stat != PGT_XSTAT_XPEHH) return pgt_set_error(PGT_ERR_ARGS, "pgt_scan_plan_extreme: unknown statistic");
+	if (mem != PGT_MEM_DEVICE && mem != PGT_MEM_HOST) return pgt_set_error(PGT_ERR_ARGS, "pgt_scan_plan_extreme: unknown memory space");
+	if (!score) return pgt_set_error(PGT_ERR_ARGS, "pgt_scan_plan_extreme: score column is NULL");
+	pgt_windows geo;
+	memset(&geo, 0, sizeof(geo));
+	if (rows) {
+		bool other = rows->dxy_global != nullptr;
+		for_each_value([&](const void* p) { other = other || p; }, *rows);
+		if (other) return pgt_set_error(PGT_ERR_ARGS, "pgt_scan_plan_extreme: rows may only ask for label, start_pos, end_pos, mid_pos and nsites");
+		geo = *rows;
+	}
+	if (!pos && (plan->mode == PGT_MODE_BP || out->ext_pos || geo.start_pos || geo.end_pos || geo.mid_pos))
+		return pgt_set_error(PGT_ERR_ARGS, "pgt_scan_plan_extreme: pos is required in bp mode and for ext_pos, start_pos, end_pos and mid_pos");
+	Cols C;
+	memset(&C, 0, sizeof(C));
+	C.pos = pos;
+	C.score = score;
+	C.minind = 1;
+	C.cutoff = cutoff;
+	XRows x{geo.label, geo.start_pos, geo.end_pos, geo.mid_pos, geo.nsites, out->ext_value, out->ext_pos, out->ext_site, out->nbig, out->nsites,
+	        out->prop, score, pos, 0};
+	cudaStream_t st = (cudaStream_t)stream;
+	if (stat == PGT_XSTAT_IHS) return run_scan<XStat<XMODE_ABS>>(plan, range, kStatExtreme, C, site_offsets, &geo, &x, workspace, workspace_bytes, mem, st);
+	if (cutoff < 0) return run_scan<XStat<XMODE_MIN>>(plan, range, kStatExtreme, C, site_offsets, &geo, &x, workspace, workspace_bytes, mem, st);
+	return run_scan<XStat<XMODE_MAX>>(plan, range, kStatExtreme, C, site_offsets, &geo, &x, workspace, workspace_bytes, mem, st);
 }

@@ -160,3 +160,35 @@ extern "C" int pgt_scan_extreme_sharded(const pgt_xplan* plan, pgt_xstat stat, d
 	std::vector<Shard> shards;
 	return run_shards("pgt_scan_extreme_sharded", devices, ndev, shards, describe, scan);
 }
+
+// ---- the extreme score over a window plan, same scheme as pgt_scan_sharded: windows cut by pgt_plan_shard, every shard
+// the ordinary host-memory scan over the whole columns (element 0 = site 0); the reduction is exact, so any cut gives
+// the same rows.
+extern "C" int pgt_scan_plan_extreme_sharded(const pgt_plan* plan, pgt_xstat stat, double cutoff, const uint32_t* pos, const double* score,
+                                             const uint64_t* site_offsets, const pgt_windows* rows, const pgt_xwindows* out, const int* devices,
+                                             uint32_t ndev) {
+	if (!plan || !score || !out) return pgt_set_error(PGT_ERR_ARGS, "pgt_scan_plan_extreme_sharded: plan, score and out must not be NULL");
+	if (stat != PGT_XSTAT_IHS && stat != PGT_XSTAT_XPEHH) return pgt_set_error(PGT_ERR_ARGS, "pgt_scan_plan_extreme_sharded: unknown statistic");
+	if (plan->d_tables)
+		return pgt_set_error(PGT_ERR_ARGS, "pgt_scan_plan_extreme_sharded: the plan is bound to one device (pgt_plan_bind_device); unbind it first");
+	auto describe = [&](uint32_t i, Shard& s) -> int {
+		PGT_TRY(pgt_plan_shard(plan, i, ndev, &s.range.w_lo, &s.range.w_hi, nullptr, nullptr));
+		s.idle = s.range.w_lo == s.range.w_hi;  // ({0, 0} would mean "all windows")
+		if (!s.idle) s.ws_bytes = pgt_scan_plan_extreme_workspace_bytes(plan, &s.range, PGT_MEM_HOST);
+		return PGT_OK;
+	};
+	auto scan = [&](Shard& s, cudaStream_t st) {
+		auto shift = [d = s.range.w_lo](auto*& p) { p = p ? p + d : p; };
+		pgt_windows r;
+		if (rows) {
+			r = *rows;
+			for_each_field(shift, r);
+		}
+		pgt_xwindows x = *out;
+		for_each_xfield(shift, x);
+		return pgt_scan_plan_extreme(plan, &s.range, stat, cutoff, pos, score, site_offsets, rows ? &r : nullptr, &x, s.ws, s.ws_bytes,
+		                             PGT_MEM_HOST, st);
+	};
+	std::vector<Shard> shards;
+	return run_shards("pgt_scan_plan_extreme_sharded", devices, ndev, shards, describe, scan);
+}

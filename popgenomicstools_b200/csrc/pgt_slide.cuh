@@ -208,7 +208,7 @@ __device__ __forceinline__ void slide_consume(const DevPlan& P, const TileCfg& t
 						const uint32_t i = base + (uint32_t)e;
 						if (member && (uint32_t)e < sc.E && e0 + (uint32_t)e < Wu && i >= s_lo && i < s_hi) {
 							PGT_CHECK(i - s_lo < ctl->ns[stg]);
-							Stat::fold(leaf[e], Stat::load_tile(cp, i - s_lo), tc.minind);
+							Stat::fold(leaf[e], Stat::load_tile(cp, i - s_lo), tc.minind, 0.0, 0);  // (no statistic of this path reads the site index)
 							if (has_pos) pv[e] = pstage[i - s_lo];
 							if (GlobalTerm<Stat>::has && i < g_hi) GlobalTerm<Stat>::add(leaf[e], gd, gne, gnk);
 						}
@@ -521,7 +521,7 @@ __global__ void __launch_bounds__(1024) k_global_sites(Cols cols, uint64_t i0, u
 		for (int q = 0; q < U; ++q) {
 			if (i + q * stride >= i1) break;
 			DxyStat::Acc a = DxyStat::zero();
-			DxyStat::fold(a, v[q], cols.minind);
+			DxyStat::fold(a, v[q], cols.minind, 0.0, 0);
 			d = __dadd_rn(d, a.dxy);
 			ne += a.neff;
 			nk += a.nskip;

@@ -135,7 +135,13 @@ class WindowPlan(_Plan):
         r = _range(self, window_range, site_origin, site_count)
         return int(self._lib.pgt_scan_workspace_bytes(self._h, C.byref(r), stat, mem))
 
-    _workspace_bytes = workspace_bytes
+    def extreme_workspace_bytes(self, mem, window_range=None, site_origin=0, site_count=0):
+        """Device scratch of pgt_scan_plan_extreme (scan_extreme over this plan)."""
+        r = _range(self, window_range, site_origin, site_count)
+        return int(self._lib.pgt_scan_plan_extreme_workspace_bytes(self._h, C.byref(r), mem))
+
+    def _workspace_bytes(self, stat, *key):
+        return self.extreme_workspace_bytes(*key) if stat == "extreme" else self.workspace_bytes(stat, *key)
 
     def workspace(self, device, stat, mem, window_range=None, site_origin=0, site_count=0):
         """Device scratch for a scan, cached per (device, stat, mem, range)."""
